@@ -2,7 +2,7 @@
 """bench.py -- decoded images/s of the SDNet decoding path on 1..8 B200s.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--mode both|noise|blobs]
-                    [--workload cfg5|cfg2|cfg3|cfg4] [--dtype f32|f16|bf16]
+                    [--workload cfg5|cfg2|cfg3|cfg4] [--dtype f32|f16|bf16] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -18,6 +18,11 @@ Both synthetic modes of SURVEY 8(d) are timed (``modes``); the headline ``value`
 Outside the timed region the very plan that was timed is checked, bit for bit, against the reference's
 own op sequence on the device (``parity_checked``) and, for N > 1, every rank checks the gathered result
 against a single-GPU decode of the whole batch (``gather_bit_exact``).
+
+``--dump-outputs DIR`` writes what the last timed step of each mode returned (the packed detections of the whole
+global batch, as rank 0 holds them after the gather) as ``DIR/<mode>_<field>.npy``, so that two builds can be
+compared output for output on identical inputs.  Past 64 MB a fixed sample of images is written instead, and
+``DIR/<mode>_images.npy`` lists which.
 
 Prints ONE JSON line.  ``--impl reference`` times the reference decoder on the host CPU instead: the
 UNMODIFIED reference ``Decoder`` from ``oracle/_ref`` when that archive exists (``kind: "reference"``),
@@ -40,6 +45,7 @@ sys.path.insert(0, str(ROOT))
 UNIQUE_IMAGES = 32  # distinct synthetic images generated on the CPU; tiled to fill a cfg5 shard
 CPU_BATCH = 16  # images per CPU-baseline step (the reference's cfg3 batch)
 L2_BYTES = 126 * 1024 * 1024
+DUMP_BYTES = 63 << 20  # --dump-outputs array data over all modes; the rest of 64 MB is left for the .npy headers
 
 
 def parse_args():
@@ -68,7 +74,16 @@ def parse_args():
                          "written again (two runs later) and at the end of the timed region")
     ap.add_argument("--gather", choices=("fused", "nccl"), default="fused",
                     help="N > 1: tail kernel stores into every peer (symmetric memory) + barrier, or ncclAllGather")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the packed detections of the last timed step of each mode as "
+                         "DIR/<mode>_<field>.npy (float32, or float64 for integer fields; a fixed sample of images "
+                         "when they exceed 64 MB)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's results: not available with --impl reference")
+    return args
 
 
 # ----------------------------------------------------------------------------- clocks
@@ -276,6 +291,29 @@ def fields_equal(got, want, got_rows=None):
     return bad
 
 
+def dump_outputs(directory, per_mode: dict):
+    """Write ``{mode: {field: host tensor}}`` as ``directory/<mode>_<field>.npy``: float fields as float32, integer
+    fields as float64 (exact for every index and count here).  Every field is indexed by image first; when a mode's
+    arrays exceed its share of ``DUMP_BYTES`` they are cut to a fixed, seeded sample of images, whose indices are
+    written as ``<mode>_images.npy``."""
+    import numpy as np
+
+    out = Path(directory)
+    out.mkdir(parents=True, exist_ok=True)
+    budget = DUMP_BYTES // len(per_mode)
+    for mode, fields in per_mode.items():
+        arrays = {k: v.numpy().astype(np.float32 if v.dtype.is_floating_point else np.float64) for k, v in fields.items()}
+        images = next(iter(arrays.values())).shape[0]
+        per_image = sum(a.nbytes for a in arrays.values()) // images
+        if per_image * images > budget:
+            rows = np.random.default_rng(0).choice(images, budget // (per_image + 8), replace=False)
+            rows.sort()
+            arrays = {k: a[rows] for k, a in arrays.items()}
+            arrays["images"] = rows.astype(np.float64)
+        for k, a in arrays.items():
+            np.save(out / f"{mode}_{k}.npy", a)
+
+
 def main():
     global _REAL_STDOUT
     args = parse_args()
@@ -383,15 +421,15 @@ def main():
             depth = 1  # the ncclAllGather baseline stays serial
 
     def step(o):
+        """Enqueue one decode of the batch; returns the PackedDetections it writes."""
         if pipe is not None:
-            pipe.submit(o["anchor_hm"], o["part_hm"], o["offsets"], o["embeddings"], conf32, dist32)
-            return
+            return pipe.submit(o["anchor_hm"], o["part_hm"], o["offsets"], o["embeddings"], conf32, dist32)[0]
         if fused is not None:
-            fused.run(o["anchor_hm"], o["part_hm"], o["offsets"], o["embeddings"], conf32, dist32)
-            return
-        plan.run(o["anchor_hm"], o["part_hm"], o["offsets"], o["embeddings"], conf32, dist32)
+            return fused.run(o["anchor_hm"], o["part_hm"], o["offsets"], o["embeddings"], conf32, dist32)
+        res = plan.run(o["anchor_hm"], o["part_hm"], o["offsets"], o["embeddings"], conf32, dist32)
         if world > 1:
             dist.all_gather_into_tensor(gathered, plan.out.blob)
+        return res
 
     def fence():
         torch.cuda.synchronize(device)
@@ -406,7 +444,7 @@ def main():
         peak_gbs, peak_src = 6650.0, "fallback (B200_PROFILING.md 6.65 TB/s)"
     peaks_bytes = shard * (M + N) * H * W * esize  # algorithmic bytes of the dominant kernel: heat maps read once
 
-    per_mode = {}
+    per_mode, dumped = {}, {}
     align = torch.zeros(1, device=device)
     for mode in modes:
         rot = outs_of[mode]
@@ -424,13 +462,20 @@ def main():
                 dist.all_reduce(align)
             ev0.record()
             for i in range(args.steps):
-                step(rot[i % len(rot)])
+                last = step(rot[i % len(rot)])
             if pipe is not None:
                 pipe.drain()  # fused gather in lazy mode: includes the wait for every rank's rows of each plan's last run
             elif fused is not None:
                 fused.wait_arrival()
             ev1.record()
             fence()
+        if args.dump_outputs and rank == 0:  # copied now: the untimed runs below reuse the timed plans' outputs
+            if gathered is not None:  # ncclAllGather: the caller's result is every rank's blob, merged
+                from structuredetector_b200.parallel import merge_packed
+
+                last = merge_packed([gathered[r * blob_bytes:(r + 1) * blob_bytes] for r in range(world)], [shard] * world,
+                                    K, P, M + N)
+            dumped[mode] = {k: getattr(last, k).cpu() for k in FIELDS}
         ms_total = ev0.elapsed_time(ev1)
         by_rank = None
         if world > 1:
@@ -503,6 +548,8 @@ def main():
                            "planes_via_exact_select": diag_overflow, "candidates_per_plane_mean": cand_mean},
         }
 
+    if dumped:
+        dump_outputs(args.dump_outputs, dumped)
     head = min(per_mode, key=lambda m: per_mode[m]["value"])  # the slower mode is the headline
     hm = per_mode[head]
     ms_per_step, value, kernel_ms = hm["ms_per_step"], hm["value"], hm["kernel_ms"]

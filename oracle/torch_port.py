@@ -8,8 +8,8 @@ composed by our own code, runnable on ``cpu`` (the CPU baseline / ``--impl refer
 arm of bench.py) or on ``cuda`` (the on-device checker used by ``-m gpu`` tests).
 
 Only ``tests/``, ``__graft_entry__.smoke()`` and ``bench.py``'s CPU-baseline legs may
-import it.  It is validated against the live reference in ``tests/test_oracle.py`` when
-``/root/reference`` is present and against ``tests/golden/`` otherwise.
+import it.  ``tests/test_oracle.py`` validates it against the reference's stored outputs in
+``tests/golden/`` and against the oracle on other shapes.
 
 Differences from the reference that are deliberate:
   * returns packed tensors (same layout as the C-ABI outputs) and builds Python objects

@@ -1,5 +1,5 @@
 """Build glue: `pip install -e .` / `python setup.py build_ext --inplace` compile the sm_100a
-library in-tree with nvcc (same command as `python -m structuredetector_b200.build`)."""
+library in-tree with nvcc (same command as `python structuredetector_b200/build.py`)."""
 from setuptools import setup
 from setuptools.command.build_py import build_py
 

@@ -2,7 +2,7 @@
 
 There is deliberately no fallback: if the shared library is missing or does not export
 the expected ABI, importing the decode ops raises.  Build it with
-``python -m structuredetector_b200.build`` (or ``__graft_entry__.build()``).
+``python structuredetector_b200/build.py`` (or ``__graft_entry__.build()``).
 """
 from __future__ import annotations
 
@@ -153,7 +153,7 @@ def load_from(path) -> ctypes.CDLL:
     if not path.exists():
         raise NativeLibraryError(
             f"{path} is missing: build the CUDA extension first "
-            "(python -m structuredetector_b200.build). There is no CPU fallback."
+            "(python structuredetector_b200/build.py). There is no CPU fallback."
         )
     lib = ctypes.CDLL(str(path))
     missing = [name for name in EXPORTS if not hasattr(lib, name)]

@@ -1,6 +1,8 @@
 """Build ``csrc/libsdnet_decode.so`` in-tree with nvcc for sm_100a.
 
-    python -m structuredetector_b200.build [--force]
+    python structuredetector_b200/build.py [--force]
+
+Run as a file, not with ``-m``: importing the package needs the extensions built here.
 """
 from __future__ import annotations
 

@@ -23,7 +23,7 @@ from .annotations import ImageAnnotation, Keypoint, Object
 try:
     from . import _fastobj  # C object assembly (csrc/fastobj.c), built by structuredetector_b200.build
 except ImportError as exc:  # no silent slow path: say how to get it
-    raise ImportError("structuredetector_b200._fastobj is missing: run `python -m structuredetector_b200.build` "
+    raise ImportError("structuredetector_b200._fastobj is missing: run `python structuredetector_b200/build.py` "
                       "(gcc, CPython headers) to build the object-assembly extension") from exc
 
 __all__ = ["Decoder", "CoreMLDecoder", "KeypointDecoder", "RawDecoder", "CoreMLModel"]

@@ -11,9 +11,9 @@ if str(ROOT) not in sys.path:
 def pytest_sessionstart(session):
     """The host-side C extension is a build artefact (git-ignored): make sure it exists before the
     package is imported.  gcc only, a no-op when it is up to date."""
-    from structuredetector_b200 import build
+    from __graft_entry__ import load_build_module
 
-    build.build_fastobj()
+    load_build_module().build_fastobj()
 
 
 def pytest_configure(config):

@@ -1,14 +1,12 @@
 """Shared test plumbing: plain-tuple views of decoder outputs, sigmoid adapters, arg namespaces."""
 from __future__ import annotations
 
-import sys
 from pathlib import Path
 from types import SimpleNamespace
 
 import numpy as np
 import torch
 
-REFERENCE_SRC = Path("/root/reference/src")
 GOLDEN_DIR = Path(__file__).resolve().parent / "golden"
 
 
@@ -47,20 +45,6 @@ def torch_sigmoid_fn(device="cpu"):
 
 def np_inputs(outputs):
     return [outputs[k].detach().cpu().numpy() for k in ("anchor_hm", "part_hm", "offsets", "embeddings")]
-
-
-def reference_available() -> bool:
-    return (REFERENCE_SRC / "sdnet" / "data" / "decoders.py").exists()
-
-
-def import_reference():
-    """Import the unmodified reference package read-only (never writes bytecode)."""
-    sys.dont_write_bytecode = True
-    if str(REFERENCE_SRC) not in sys.path:
-        sys.path.insert(0, str(REFERENCE_SRC))
-    import sdnet.data.decoders as ref_decoders  # noqa: WPS433
-
-    return ref_decoders
 
 
 def packed_np(packed):

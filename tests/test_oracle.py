@@ -1,6 +1,6 @@
 """CPU: the oracle against the golden vectors produced by running the reference itself
-(tests/golden/make_golden.py), and -- when /root/reference is present -- against the live
-reference.  This is what pins the oracle (SURVEY.md 8c: the reference has no tests of its own)."""
+(tests/golden/make_golden.py), and against the port of the reference's op sequence on shapes the vectors
+do not have.  This is what pins the oracle (SURVEY.md 8c: the reference has no tests of its own)."""
 import numpy as np
 import pytest
 import torch
@@ -8,8 +8,8 @@ import torch
 from oracle import sdnet_oracle as O
 from oracle import torch_port as TP
 from structuredetector_b200.synth import CONFIGS, DecodeConfig, make_raw, split_outputs
-from tests.helpers import (assert_objects_close, assert_topk_equal_up_to_ties, golden_args, golden_names, import_reference,
-                           listify, load_golden, np_inputs, plain, reference_available, torch_sigmoid_fn)
+from tests.helpers import (assert_objects_close, assert_topk_equal_up_to_ties, golden_args, golden_names, listify, load_golden,
+                           np_inputs, torch_sigmoid_fn)
 
 TIE_FREE = [n for n in golden_names() if not n.startswith(("ties", "half"))]
 
@@ -129,22 +129,24 @@ def test_oracle_helpers_semantics():
     assert not (np.float32(0.4) > np.float32(0.4))
 
 
-@pytest.mark.skipif(not reference_available(), reason="/root/reference not present (GPU box)")
 @pytest.mark.parametrize("mode", ["noise", "blobs", "ladder"])
-def test_oracle_matches_live_reference(mode):
-    ref = import_reference()
+def test_oracle_matches_torch_port_off_the_golden_shapes(mode):
+    """3 labels x 2 parts on 56x72 maps with K = 50, P = 60, a shape none of the stored vectors has: the oracle and the
+    port of the reference's op sequence (both pinned to the reference's stored outputs above) return the same objects."""
     cfg = DecodeConfig("live", 2, 3, 2, 56, 72, 50, 60, cfg_id=77)
     raw = make_raw(cfg, mode)
     outs = split_outputs(raw, cfg.labels, cfg.parts)
     from tests.helpers import make_args
 
     args = make_args(cfg)
-    anns = ref.Decoder(args)({k: v.clone() for k, v in outs.items()})
+    port = TP.decode({k: v.clone() for k, v in outs.items()}, args._r_labels, args._r_parts, args.anchor_name,
+                     args.down_ratio, cfg.max_objects, cfg.max_parts, cfg.conf_threshold, cfg.dist_thresh)
     pk = O.decode_packed(*np_inputs(outs), cfg.max_objects, cfg.max_parts, cfg.conf_threshold, cfg.dist_thresh,
                          sigmoid_fn=torch_sigmoid_fn("cpu"))
     objs = O.assemble(pk, args._r_labels, args._r_parts, args.anchor_name, cfg.conf_threshold,
                       (cfg.width, cfg.height), (4 * cfg.width, 4 * cfg.height))
-    assert plain(anns) == objs
+    assert sum(len(o) for o in objs) > 0
+    assert listify(port) == listify(objs)
 
 
 @pytest.mark.parametrize("name", ["half_f16", "half_bf16"])
