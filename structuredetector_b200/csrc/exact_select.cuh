@@ -31,9 +31,8 @@ struct ExactParams {
 template <int DT>
 __device__ __forceinline__ u32 exact_key(const void* plane, long long sh, int H, int W, int R, int y, int x, bool pre) {
   const float v = ld_in<DT>(plane, (long long)y * sh + x);
-  if (pre) {
-    const u32 bits = __float_as_uint(v);
-    return (bits & 0x80000000u) ? ~bits : (bits | 0x80000000u);
+  if (pre) {  // zeros are suppressed pixels, left to the tail's zero-fill like in the peaks kernels (shared_floor)
+    return v > 0.0f ? (__float_as_uint(v) | 0x80000000u) : 0u;
   }
   float h = v;
   for (int dy = -R; dy <= R; ++dy) {

@@ -132,11 +132,15 @@ __device__ __forceinline__ int floor_bin_fine(const u32* hist, int lane, int K) 
 // it counted has a lower index), a shared floor needs a strict score gap: a pixel is dropped
 // only if its logit is below edge(b) - kNear with edge(b) in [kLo, kHi] (Num<DT>), where
 // S(x - kNear) < S(x) is verified exhaustively (tests/test_gpu_parity.py).
+// Pre-activated maps never go below a floor of 0: their zeros are the pixels NMS suppressed, which the tail's zero-fill
+// supplies in torch.topk's order (class, then index).  Recording only some of them -- those a warp meets before its
+// floor rises -- would put those ahead of the zero-filled ones.
 template <int DT = SDNET_DTYPE_F32>
 __device__ __forceinline__ float shared_floor(int fbin, float xscale) {
-  if (fbin <= 0) return -CUDART_INF_F;
+  const bool pre = xscale != 1.0f;
+  if (fbin <= 0) return pre ? 0.0f : -CUDART_INF_F;
   const float edge = kBinLo + (float)fbin * (1.0f / kFineScale);
-  if (xscale != 1.0f) return edge / xscale;  // pre-activated: keys are strictly monotone in the value
+  if (pre) return fmaxf(edge / xscale, 0.0f);  // keys are strictly monotone in the value
   if (edge < Num<DT>::kLo || edge > Num<DT>::kHi2) return -CUDART_INF_F;
   return edge - (edge <= Num<DT>::kHi ? Num<DT>::kNear : Num<DT>::kNear2);
 }
