@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define SDNET_ABI_VERSION 8
+#define SDNET_ABI_VERSION 9
 
 /* element types of the four input tensors */
 #define SDNET_DTYPE_F32 0
@@ -47,7 +47,7 @@ extern "C" {
 /* argument errors */
 #define SDNET_E_NULL -1      /* a required pointer is NULL */
 #define SDNET_E_SHAPE -2     /* non-positive dimension, H*W >= 2^24, K or P > H*W (torch.topk: "k out of range"),
-                                K or P > SDNET_MAX_TOPK, M+N > SDNET_MAX_CHANNELS */
+                                K or P > SDNET_MAX_TOPK, M+N > SDNET_MAX_CHANNELS, T outside 1..SDNET_MAX_THRESHOLDS */
 #define SDNET_E_STRIDE -3    /* innermost (w) stride is not 1 */
 #define SDNET_E_DTYPE -4     /* unsupported dtype */
 #define SDNET_E_WORKSPACE -5 /* workspace missing, misaligned (256 B) or smaller than sdnet_decode_workspace_bytes */
@@ -252,6 +252,51 @@ typedef struct SdnetObjectMatchParams {
 } SdnetObjectMatchParams;
 
 int sdnet_match_objects_launch(const SdnetObjectMatchParams* params, void* stream);
+
+/* Threshold sweep of the evaluator: for each of T confidence thresholds, what sdnet_match_launch and (with
+ * SDNET_SWEEP_OBJECTS) sdnet_match_objects_launch compute on a decode at that threshold, from ONE decode.
+ * anchor_out / part_out do not depend on the decoder's conf; only the grouping does, so it is redone per
+ * threshold: anchors with score > conf_group[t] keep (x, y), the others sit at (+1e6, +1e6); parts with
+ * score > conf_group[t] keep their origin, the others sit at (-1e6, -1e6); every part goes to the first anchor
+ * at the smallest fp32 distance sqrt(dx*dx + dy*dy) (each step rounded, no FMA), if that distance is
+ * < dist_abs_f32 (decoders.py:80-100, the full P x K search).  The `assign` and `counts` the decode wrote are not
+ * read, so the decode's own conf does not matter; it must have grouped (part_out's origins are needed).
+ * Every output is indexed [image][threshold]. */
+#define SDNET_MAX_THRESHOLDS 256
+#define SDNET_SWEEP_OBJECTS 1u /* SdnetSweepParams.flags: also the object-level (CSI, classification) tables */
+typedef struct SdnetSweepParams {
+  uint32_t struct_size; /* sizeof(SdnetSweepParams) */
+  int32_t B, M, N, K, P;
+  int32_t T;            /* thresholds, 1 .. SDNET_MAX_THRESHOLDS */
+  int32_t max_gt_objects, max_gt_parts; /* row lengths of the ground-truth arrays, <= SDNET_MAX_GT */
+  uint32_t flags;       /* SDNET_SWEEP_* */
+  float dist_abs_f32;   /* the decoder's gate: (float)(dist_thresh * min(W, H)) (decoders.py:100) */
+  double sx, sy;        /* heat-map -> network-input scale, in/out (decoders.py:139) */
+  double csi_threshold; /* args.csi_threshold (evaluator.py:414); read with SDNET_SWEEP_OBJECTS */
+  const double* conf;          /* (T): the evaluator's thresholds (objects: score > conf; raw parts: not score < conf) */
+  const float* conf_group;     /* (T): the same thresholds rounded to the heat maps' dtype, for the grouping's score > conf */
+  const float* anchor_out;     /* (B, K, 4) as written by sdnet_decode_launch */
+  const float* part_out;       /* (B, P, 6) */
+  const double* image_scale;   /* (B, 4): as in SdnetMatchParams */
+  const double* gt_objects;    /* (B, max_gt_objects, 3): anchor x, y, class index; annotation order */
+  const int32_t* n_gt_objects; /* (B) */
+  const double* gt_parts;      /* (B, max_gt_parts, 3): x, y, kind index; grouped by object, object order */
+  const int32_t* gt_part_owner;/* (B, max_gt_parts): as in SdnetObjectMatchParams; read with SDNET_SWEEP_OBJECTS */
+  const int32_t* n_gt_parts;   /* (B) */
+  const int32_t* cls_group;    /* (M): as in SdnetObjectMatchParams; read with SDNET_SWEEP_OBJECTS */
+  int32_t* anchor_stats;       /* (B, T, M, 3): ndet, npos, tp */
+  int32_t* part_stats;         /* (B, T, N, 3) */
+  double* anchor_acc;          /* (B, T, K): as SdnetMatchParams.anchor_acc */
+  double* part_acc;            /* (B, T, P) */
+  int32_t* csi_stats;          /* (B, T, M, 3)   } SDNET_SWEEP_OBJECTS only: */
+  double* csi_acc;             /* (B, T, K)      } as the fields of the same name */
+  int32_t* classif_stats;      /* (B, T, 20, 3)  } in SdnetObjectMatchParams */
+  double* classif_acc;         /* (B, T, K)      } */
+  int32_t* pred_parts;         /* (B, T, K)      } */
+  int32_t* assign_out;         /* optional (B, T, P): the regrouped assignment (NULL to skip) */
+} SdnetSweepParams;
+
+int sdnet_sweep_launch(const SdnetSweepParams* params, void* stream);
 
 #ifdef __cplusplus
 }

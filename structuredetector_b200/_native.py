@@ -13,7 +13,7 @@ import os as _os
 
 # SDNET_DECODE_LIB: load another build of the same library (kernel experiments, tools/xbuild.sh)
 LIB_PATH = Path(_os.environ.get("SDNET_DECODE_LIB") or Path(__file__).resolve().parent / "csrc" / "libsdnet_decode.so").resolve()
-ABI_VERSION = 8
+ABI_VERSION = 9
 DEST_PEER_STORES, DEST_MULTICAST = 0, 1  # SdnetDecodeParams.dest_mode
 
 FLAG_PRE_ACTIVATED = 1
@@ -28,6 +28,8 @@ MAX_TOPK = 1024
 MAX_CHANNELS = 255
 MAX_DEST = 16
 MAX_GT = 1024  # SDNET_MAX_GT
+MAX_THRESHOLDS = 256  # SDNET_MAX_THRESHOLDS
+SWEEP_OBJECTS = 1  # SdnetSweepParams.flags
 
 EXPORTS = (
     "sdnet_abi_version",
@@ -40,6 +42,7 @@ EXPORTS = (
     "sdnet_match_launch",
     "sdnet_gather_wait_launch",
     "sdnet_match_objects_launch",
+    "sdnet_sweep_launch",
     "sdnet_activate_launch",
     "sdnet_suppress_launch",
     "sdnet_suppress_into_launch",
@@ -131,6 +134,26 @@ class SdnetObjectMatchParams(ctypes.Structure):
     ]
 
 
+class SdnetSweepParams(ctypes.Structure):
+    _fields_ = [
+        ("struct_size", ctypes.c_uint32),
+        ("B", ctypes.c_int32), ("M", ctypes.c_int32), ("N", ctypes.c_int32), ("K", ctypes.c_int32), ("P", ctypes.c_int32),
+        ("T", ctypes.c_int32), ("max_gt_objects", ctypes.c_int32), ("max_gt_parts", ctypes.c_int32),
+        ("flags", ctypes.c_uint32), ("dist_abs_f32", ctypes.c_float),
+        ("sx", ctypes.c_double), ("sy", ctypes.c_double), ("csi_threshold", ctypes.c_double),
+        ("conf", ctypes.c_void_p), ("conf_group", ctypes.c_void_p),
+        ("anchor_out", ctypes.c_void_p), ("part_out", ctypes.c_void_p), ("image_scale", ctypes.c_void_p),
+        ("gt_objects", ctypes.c_void_p), ("n_gt_objects", ctypes.c_void_p),
+        ("gt_parts", ctypes.c_void_p), ("gt_part_owner", ctypes.c_void_p), ("n_gt_parts", ctypes.c_void_p),
+        ("cls_group", ctypes.c_void_p),
+        ("anchor_stats", ctypes.c_void_p), ("part_stats", ctypes.c_void_p),
+        ("anchor_acc", ctypes.c_void_p), ("part_acc", ctypes.c_void_p),
+        ("csi_stats", ctypes.c_void_p), ("csi_acc", ctypes.c_void_p),
+        ("classif_stats", ctypes.c_void_p), ("classif_acc", ctypes.c_void_p), ("pred_parts", ctypes.c_void_p),
+        ("assign_out", ctypes.c_void_p),
+    ]
+
+
 class NativeLibraryError(RuntimeError):
     pass
 
@@ -172,6 +195,8 @@ def load_from(path) -> ctypes.CDLL:
     lib.sdnet_match_launch.argtypes = [ctypes.POINTER(SdnetMatchParams), ctypes.c_void_p]
     lib.sdnet_match_objects_launch.restype = ctypes.c_int
     lib.sdnet_match_objects_launch.argtypes = [ctypes.POINTER(SdnetObjectMatchParams), ctypes.c_void_p]
+    lib.sdnet_sweep_launch.restype = ctypes.c_int
+    lib.sdnet_sweep_launch.argtypes = [ctypes.POINTER(SdnetSweepParams), ctypes.c_void_p]
     lib.sdnet_decode_peaks_path.restype = ctypes.c_int
     lib.sdnet_decode_peaks_path.argtypes = [ctypes.POINTER(SdnetDecodeParams)]
     lib.sdnet_decode_schedule.restype = ctypes.c_int

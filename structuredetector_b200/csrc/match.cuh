@@ -119,9 +119,18 @@ __device__ __forceinline__ double csi_of_pair(const ObjScratch& s, int k, int j,
   return (double)tp / (double)(npos + ndet - tp);
 }
 
-__global__ void __launch_bounds__(kMatchThreads) sdnet_match_objects_kernel(const SdnetObjectMatchParams p) {
-  extern __shared__ __align__(16) unsigned char obj_smem[];
-  const int b = blockIdx.x, tid = threadIdx.x, nt = blockDim.x;
+// Dynamic shared memory match_objects needs (16-byte aligned base).
+inline size_t match_objects_smem_bytes(int max_gt_objects, int max_gt_parts, int K, int P, int M) {
+  const size_t Go = (size_t)max_gt_objects, Gp = (size_t)max_gt_parts, k = (size_t)K, q = (size_t)P;
+  const size_t n_stats = 3 * (size_t)(M > 20 ? M : 20);
+  return 8 * (2 * Go + 3 * k + 2 * q + 2 * Gp) + 4 * (3 * Go + 1 + 3 * k + 1 + 2 * q + Gp + n_stats) + 16;
+}
+
+// The object-level matching of image b with the part assignment `asg` (P entries; shared or global memory), its
+// results stored in output row `row` of p's outputs.  `obj_smem` holds match_objects_smem_bytes.
+__device__ __forceinline__ void match_objects(const SdnetObjectMatchParams& p, int b, size_t row, const int* asg,
+                                              unsigned char* obj_smem) {
+  const int tid = threadIdx.x, nt = blockDim.x;
   const int K = p.K, P = p.P, Go = p.max_gt_objects, Gp = p.max_gt_parts;
   ObjScratch s;
   {
@@ -137,7 +146,6 @@ __global__ void __launch_bounds__(kMatchThreads) sdnet_match_objects_kernel(cons
   const double rx = scale[0], ry = scale[1], thresh = scale[2], norm = scale[3];
   const float* A = p.anchor_out + (size_t)b * K * 4;
   const float* Q = p.part_out + (size_t)b * P * 6;
-  const int* asg = p.assign + (size_t)b * P;
   const int n_go = min(p.n_gt_objects[b], Go), n_gp = min(p.n_gt_parts[b], Gp);
   const double* G = p.gt_objects + (size_t)b * Go * 3;
   const double* Hh = p.gt_parts + (size_t)b * Gp * 3;
@@ -220,7 +228,7 @@ __global__ void __launch_bounds__(kMatchThreads) sdnet_match_objects_kernel(cons
       s.best[k] = best;
     }
     __syncthreads();
-    double* acc_out = (pass == 0 ? p.classif_acc : p.csi_acc) + (size_t)b * K;
+    double* acc_out = (pass == 0 ? p.classif_acc : p.csi_acc) + row * K;
     for (int k = tid; k < K; k += nt) {
       const int jb = s.jbest[k];
       const bool tp = jb >= 0 && s.win[jb] == k;
@@ -228,12 +236,18 @@ __global__ void __launch_bounds__(kMatchThreads) sdnet_match_objects_kernel(cons
       if (tp) atomicAdd(&s.stats[3 * key_of((int)A[4 * k + 3], s.npp[k]) + 2], 1);
     }
     __syncthreads();
-    int* stats_out = pass == 0 ? p.classif_stats + (size_t)b * 60 : p.csi_stats + (size_t)b * p.M * 3;
+    int* stats_out = pass == 0 ? p.classif_stats + row * 60 : p.csi_stats + row * p.M * 3;
     for (int i = tid; i < 3 * n_lab; i += nt) stats_out[i] = s.stats[i];
     if (pass == 0)
-      for (int k = tid; k < K; k += nt) p.pred_parts[(size_t)b * K + k] = (double)A[4 * k + 2] > p.conf ? s.npp[k] : -1;
+      for (int k = tid; k < K; k += nt) p.pred_parts[row * K + k] = (double)A[4 * k + 2] > p.conf ? s.npp[k] : -1;
     __syncthreads();
   }
+}
+
+__global__ void __launch_bounds__(kMatchThreads) sdnet_match_objects_kernel(const SdnetObjectMatchParams p) {
+  extern __shared__ __align__(16) unsigned char obj_smem[];
+  const int b = blockIdx.x;
+  match_objects(p, b, (size_t)b, p.assign + (size_t)b * p.P, obj_smem);
 }
 
 }  // namespace

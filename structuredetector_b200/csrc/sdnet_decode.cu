@@ -18,7 +18,8 @@
 //   3. tail kernel (tail.cuh) -- one CTA per image: radix-select + sort of the candidates under the
 //      total order (score desc, class asc, index asc), zero-fill, offset/embedding gather,
 //      coordinate assembly, masking, nearest-anchor grouping.
-// plus sdnet_activate_kernel (metadata maps) and sdnet_match_kernel (match.cuh, the evaluator's matching).
+// plus sdnet_activate_kernel (metadata maps), sdnet_match_kernel (match.cuh, the evaluator's matching) and
+// sdnet_sweep_kernel (sweep.cuh, the evaluator at many confidence thresholds).
 //
 // Numerics contract (SURVEY.md appendix A):
 //   * score  = min(max(1/(1+expf(-x)), 1e-6f), (float)(1-1e-6))   -- ATen's CUDA formula;
@@ -39,6 +40,7 @@
 #include "exact_select.cuh"
 #include "tail.cuh"
 #include "match.cuh"
+#include "sweep.cuh"
 #include "suppress.cuh"
 
 namespace {
@@ -526,12 +528,33 @@ int sdnet_match_objects_launch(const SdnetObjectMatchParams* p, void* stream) {
       p->M + p->N > SDNET_MAX_CHANNELS || p->max_gt_objects < 0 || p->max_gt_parts < 0 || p->max_gt_objects > SDNET_MAX_GT ||
       p->max_gt_parts > SDNET_MAX_GT)
     return SDNET_E_SHAPE;
-  const size_t Go = (size_t)p->max_gt_objects, Gp = (size_t)p->max_gt_parts, K = (size_t)p->K, P = (size_t)p->P;
-  const size_t n_stats = 3 * (size_t)(p->M > 20 ? p->M : 20);
-  const size_t smem = 8 * (2 * Go + 3 * K + 2 * P + 2 * Gp) + 4 * (3 * Go + 1 + 3 * K + 1 + 2 * P + Gp + n_stats) + 16;
+  const size_t smem = match_objects_smem_bytes(p->max_gt_objects, p->max_gt_parts, p->K, p->P, p->M);
   cudaError_t err = cudaFuncSetAttribute(sdnet_match_objects_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (err != cudaSuccess) return (int)err;
   sdnet_match_objects_kernel<<<dim3((unsigned)p->B), dim3(kMatchThreads), smem, static_cast<cudaStream_t>(stream)>>>(*p);
+  return (int)cudaGetLastError();
+}
+
+int sdnet_sweep_launch(const SdnetSweepParams* p, void* stream) {
+  if (!p) return SDNET_E_NULL;
+  if (p->struct_size != sizeof(SdnetSweepParams)) return SDNET_E_STRUCT;
+  const bool objects = (p->flags & SDNET_SWEEP_OBJECTS) != 0;
+  if (!p->conf || !p->conf_group || !p->anchor_out || !p->part_out || !p->image_scale || !p->n_gt_objects ||
+      !p->n_gt_parts || !p->anchor_stats || !p->part_stats || !p->anchor_acc || !p->part_acc ||
+      (p->max_gt_objects > 0 && !p->gt_objects) || (p->max_gt_parts > 0 && !p->gt_parts))
+    return SDNET_E_NULL;
+  if (objects && (!p->cls_group || !p->csi_stats || !p->csi_acc || !p->classif_stats || !p->classif_acc ||
+                  !p->pred_parts || (p->max_gt_parts > 0 && !p->gt_part_owner)))
+    return SDNET_E_NULL;
+  if (p->B <= 0 || p->M <= 0 || p->N <= 0 || p->K <= 0 || p->P <= 0 || p->K > SDNET_MAX_TOPK || p->P > SDNET_MAX_TOPK ||
+      p->M + p->N > SDNET_MAX_CHANNELS || p->T < 1 || p->T > SDNET_MAX_THRESHOLDS || p->max_gt_objects < 0 ||
+      p->max_gt_parts < 0 || p->max_gt_objects > SDNET_MAX_GT || p->max_gt_parts > SDNET_MAX_GT ||
+      (long long)p->B * p->T > 0x7fffffffll)
+    return SDNET_E_SHAPE;
+  const size_t smem = sweep_smem_bytes(*p);
+  cudaError_t err = cudaFuncSetAttribute(sdnet_sweep_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (err != cudaSuccess) return (int)err;
+  sdnet_sweep_kernel<<<dim3((unsigned)(p->B * p->T)), dim3(kMatchThreads), smem, static_cast<cudaStream_t>(stream)>>>(*p);
   return (int)cudaGetLastError();
 }
 

@@ -7,11 +7,13 @@ formulas, so tables and CSV code written against them keep working.  What moves 
 against their nearest ground truth -- through ``sdnet_match_launch``; ``eval_csi`` with ``compute_csi``
 (:380-420, 539-581) and ``eval_classif`` (:429-474) -- predicted objects (anchor + grouped parts) against
 ground-truth objects -- through ``sdnet_match_objects_launch``; both straight on the tensors
-``sdnet_decode_launch`` wrote: no Python object is built for a prediction.
+``sdnet_decode_launch`` wrote: no Python object is built for a prediction.  ``ThresholdSweep`` runs both at many
+confidence thresholds from one decode (``sdnet_sweep_launch``): the precision / recall / F1 curve over the threshold.
 """
 from __future__ import annotations
 
 import ctypes
+import math
 from functools import reduce
 from pathlib import Path
 
@@ -20,7 +22,7 @@ import torch
 
 from . import _native, ops
 
-__all__ = ["Evaluation", "Evaluations", "Evaluator"]
+__all__ = ["Evaluation", "Evaluations", "Evaluator", "ThresholdSweep"]
 
 
 class Evaluation:
@@ -305,8 +307,7 @@ class Evaluator:
         if not (eval_csi or eval_classif):
             return
         # ---- object-level metrics: eval_csi / compute_csi and eval_classif (evaluator.py:380-474, 539-581)
-        groups = torch.tensor([{"bean": 0, "maize": 1}.get(self._label_names.get(i), -1) for i in range(M)], dtype=torch.int32,
-                              device=device)
+        groups = self._classification_groups(device)
         c_stats = torch.empty(B, M, 3, dtype=torch.int32, device=device)
         k_stats = torch.empty(B, 20, 3, dtype=torch.int32, device=device)
         c_acc = torch.empty(B, K, dtype=torch.float64, device=device)
@@ -334,6 +335,11 @@ class Evaluator:
             key = np.where((n_parts >= 0) & (n_parts <= 9), group_np[np.clip(host[4], 0, M - 1)] * 10 + n_parts, -1)
             key = np.where(group_np[np.clip(host[4], 0, M - 1)] >= 0, key, -1)
             self._absorb(self.classification_eval, dict(enumerate(Evaluator.get_classification_labels())), k_stats, k_acc, key)
+
+    def _classification_groups(self, device):
+        """cls_group of the object matchers: 0 / 1 for the classes named "bean" / "maize", -1 for the others."""
+        return torch.tensor([{"bean": 0, "maize": 1}.get(self._label_names.get(i), -1) for i in range(len(self._label_index))],
+                            dtype=torch.int32, device=device)
 
     @staticmethod
     def _absorb(target: Evaluations, names, stats, acc, cls):
@@ -370,3 +376,157 @@ class Evaluator:
             for label, evaluation in sorted(evals.items(), key=lambda item: item[0]):
                 text += f"  {label}: {evaluation}\n"
         return text
+
+
+class ThresholdSweep:
+    """The evaluator at a grid of confidence thresholds, from one decode.
+
+    ``at(t)`` is a plain ``Evaluator`` holding exactly what ``Evaluator.accumulate_packed(decode at t, ...,
+    conf_thresh=t)`` would hold, for every decode and evaluation this sweep has accumulated: the detections a decoder
+    keeps do not depend on its threshold, only its grouping does, and ``sdnet_sweep_launch`` redoes the grouping at
+    every grid point (the full nearest-anchor search of the decoder, in the same fp32 arithmetic) before matching.
+    ``curve`` and ``best_threshold`` read the precision / recall / F1 curve off the grid.
+
+    ``thresholds``: finite, strictly increasing, at most 256.  ``dtype``: the dtype of the heat maps the detections
+    were decoded from -- the grouping compares ``score > t`` in that dtype, as the decoder does.  ``dist_thresh``: the
+    decoder's grouping distance (default ``args.decoder_dist_thresh``); ``args`` as for ``Evaluator``.
+    """
+
+    TABLES = {"anchor": "anchor_eval", "part": "part_eval", "kps": "kps_eval", "csi": "csi_eval",
+              "classification": "classification_eval"}
+
+    def __init__(self, args, thresholds, *, dtype: torch.dtype = torch.float32, dist_thresh=None):
+        values = [float(t) for t in thresholds]
+        if not values or len(values) > _native.MAX_THRESHOLDS:
+            raise ValueError(f"{len(values)} thresholds; a sweep takes 1 to {_native.MAX_THRESHOLDS}")
+        if not all(math.isfinite(v) for v in values):
+            raise ValueError("thresholds must be finite")
+        if any(b <= a for a, b in zip(values, values[1:])):
+            raise ValueError("thresholds must be strictly increasing")
+        if dtype not in ops._DTYPES:
+            raise ValueError(f"dtype {dtype} is not a heat-map dtype of the decoder (float32, float16, bfloat16)")
+        self.args = args
+        self.thresholds = np.array(values, dtype=np.float64)
+        self.dtype = dtype
+        self.dist_thresh = float(args.decoder_dist_thresh if dist_thresh is None else dist_thresh)
+        self._evaluators = [Evaluator(args) for _ in values]
+        self.lib = _native.load()
+        self.last_copy_bytes = 0  # device -> host bytes of the last accumulate_packed
+
+    def reset(self):
+        for ev in self._evaluators:
+            ev.reset()
+
+    def at(self, t) -> Evaluator:
+        """The ``Evaluator`` of grid point ``t`` (``KeyError`` if ``t`` is not on the grid)."""
+        hit = np.flatnonzero(self.thresholds == float(t))
+        if hit.size == 0:
+            raise KeyError(t)
+        return self._evaluators[int(hit[0])]
+
+    def accumulate_packed(self, packed: ops.PackedDetections, annotations, out_size, eval_csi=False, eval_classif=False):
+        """Add one decoded batch at every threshold of the grid.  Arguments as for ``Evaluator.accumulate_packed``, but
+        ``packed`` must come from a decode WITH grouping (``Decoder``, ``CoreMLDecoder``, ``ops.decode_packed(...,
+        group=True)``), because the part origins are regrouped; the threshold it was decoded at does not matter: its
+        ``assign`` and ``counts`` are not read."""
+        ev0 = self._evaluators[0]
+        B, K = packed.anchor_inds.shape
+        P = packed.part_inds.shape[1]
+        T = len(self.thresholds)
+        if len(annotations) != B:
+            raise ValueError(f"{len(annotations)} annotations for a batch of {B} images")
+        device = packed.anchor_out.device
+        M, N = len(ev0._label_index), len(ev0._part_index)
+        (gt_a, n_a, wa), (gt_p, n_p, wp), scale, owner = ev0._pack_ground_truth(annotations, device)
+        if device.type != "cuda":
+            raise RuntimeError(f"the packed detections live on {device}: the sweep runs on a CUDA device only")
+        objects = eval_csi or eval_classif
+        out_w, out_h = out_size
+        in_w, in_h = int(self.args.down_ratio * out_w), int(self.args.down_ratio * out_h)  # decoders.py:37-38
+        i32, f64 = {"dtype": torch.int32, "device": device}, {"dtype": torch.float64, "device": device}
+        conf = torch.tensor(self.thresholds, **f64)
+        conf_group = torch.tensor([ops._f32(t, self.dtype) for t in self.thresholds], dtype=torch.float32, device=device)
+        a_stats, p_stats = torch.empty(B, T, M, 3, **i32), torch.empty(B, T, N, 3, **i32)
+        a_acc, p_acc = torch.empty(B, T, K, **f64), torch.empty(B, T, P, **f64)
+        prm = _native.SdnetSweepParams()
+        prm.struct_size = ctypes.sizeof(_native.SdnetSweepParams)
+        prm.B, prm.M, prm.N, prm.K, prm.P, prm.T = B, M, N, K, P, T
+        prm.max_gt_objects, prm.max_gt_parts = wa, wp
+        prm.dist_abs_f32 = ops._f32(self.dist_thresh * min(out_w, out_h))  # as ops.decode_packed
+        prm.sx, prm.sy = in_w / out_w, in_h / out_h
+        prm.csi_threshold = float(getattr(self.args, "csi_threshold", 0.75))
+        prm.conf, prm.conf_group = conf.data_ptr(), conf_group.data_ptr()
+        prm.anchor_out, prm.part_out = packed.anchor_out.data_ptr(), packed.part_out.data_ptr()
+        prm.image_scale = scale.data_ptr()
+        prm.gt_objects, prm.n_gt_objects = gt_a.data_ptr(), n_a.data_ptr()
+        prm.gt_parts, prm.gt_part_owner, prm.n_gt_parts = gt_p.data_ptr(), owner.data_ptr(), n_p.data_ptr()
+        prm.anchor_stats, prm.part_stats = a_stats.data_ptr(), p_stats.data_ptr()
+        prm.anchor_acc, prm.part_acc = a_acc.data_ptr(), p_acc.data_ptr()
+        a_cls = packed.anchor_out[:, :, 3].to(torch.int32)
+        p_cls = packed.part_out[:, :, 3].to(torch.int32)
+        # (evaluations of each grid point, names, stats (B, T, C, 3), acc (B, T, slots), label of each acc (B, T, slots))
+        tables = [("anchor_eval", ev0._label_names, a_stats, a_acc, a_cls[:, None].expand(B, T, K)),
+                  ("part_eval", ev0._part_names, p_stats, p_acc, p_cls[:, None].expand(B, T, P))]
+        if objects:
+            groups = ev0._classification_groups(device)
+            c_stats, k_stats = torch.empty(B, T, M, 3, **i32), torch.empty(B, T, 20, 3, **i32)
+            c_acc, k_acc = torch.empty(B, T, K, **f64), torch.empty(B, T, K, **f64)
+            n_parts = torch.empty(B, T, K, **i32)
+            prm.flags = _native.SWEEP_OBJECTS
+            prm.cls_group = groups.data_ptr()
+            prm.csi_stats, prm.csi_acc = c_stats.data_ptr(), c_acc.data_ptr()
+            prm.classif_stats, prm.classif_acc, prm.pred_parts = k_stats.data_ptr(), k_acc.data_ptr(), n_parts.data_ptr()
+        stream = torch.cuda.current_stream(device).cuda_stream
+        _native.check(self.lib.sdnet_sweep_launch(ctypes.byref(prm), ctypes.c_void_p(stream)), "sdnet_sweep_launch")
+        if eval_csi:
+            tables.append(("csi_eval", ev0._label_names, c_stats, c_acc, a_cls[:, None].expand(B, T, K)))
+        if eval_classif:
+            g = groups[a_cls.clamp(0, M - 1).long()][:, None]  # as Evaluator.accumulate_packed's classification key
+            key = torch.where((n_parts >= 0) & (n_parts <= 9), g * 10 + n_parts, -1)
+            tables.append(("classification_eval", dict(enumerate(Evaluator.get_classification_labels())), k_stats, k_acc,
+                           torch.where(g >= 0, key, -1)))
+        # Only the true positives' values cross to the host: per table, the non-NaN accumulators in (threshold, image,
+        # slot) order with their labels, and the per-threshold totals.
+        stats, hits, vals, labs = [], [], [], []
+        for _, _, st, acc, cls in tables:
+            acc, cls = acc.transpose(0, 1), cls.transpose(0, 1)  # (T, B, slots)
+            hit = ~torch.isnan(acc)
+            stats.append(st.sum(dim=0, dtype=torch.int64).flatten())
+            hits.append(hit.sum(dim=(1, 2)))
+            vals.append(acc[hit])
+            labs.append(cls[hit].to(torch.int32))
+        host = [torch.cat(x).cpu().numpy() for x in (stats, hits, vals, labs)]
+        self.last_copy_bytes = sum(x.nbytes for x in host)
+        h_stats, h_hits, h_vals, h_labs = host
+        s_off = h_off = v_off = 0
+        for attr, names, st, _, _ in tables:
+            per_t = st.shape[2] * 3
+            for t, ev in enumerate(self._evaluators):
+                n = int(h_hits[h_off + t])
+                Evaluator._absorb(getattr(ev, attr), names, h_stats[s_off: s_off + per_t].reshape(1, -1, 3),
+                                  h_vals[v_off: v_off + n], h_labs[v_off: v_off + n])
+                s_off += per_t
+                v_off += n
+            h_off += T
+
+    def curve(self, table: str, label=None) -> dict:
+        """Per grid point: threshold, tp, npos, ndet, precision, recall, f1_score of ``table`` (anchor, part, kps, csi,
+        classification) for ``label``, or for all its labels together (``Evaluations.reduce``) when ``label`` is None."""
+        if table not in self.TABLES:
+            raise ValueError(f"unknown table {table!r}; one of {sorted(self.TABLES)}")
+        rows = []
+        for ev in self._evaluators:
+            evals = getattr(ev, self.TABLES[table])
+            e = evals.reduce() if label is None else evals[label]
+            rows.append((e.tp, e.npos, e.ndet, e.precision, e.recall, e.f1_score))
+        cols = list(zip(*rows))
+        out = {"threshold": self.thresholds.copy()}
+        for i, name in enumerate(("tp", "npos", "ndet")):
+            out[name] = np.array(cols[i], dtype=np.int64)
+        for i, name in enumerate(("precision", "recall", "f1_score"), start=3):
+            out[name] = np.array(cols[i], dtype=np.float64)
+        return out
+
+    def best_threshold(self, table: str, label=None) -> float:
+        """The grid threshold with the highest F1 score of ``table`` / ``label`` (the lowest one on a tie)."""
+        return float(self.thresholds[int(np.argmax(self.curve(table, label)["f1_score"]))])
