@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define SDNET_ABI_VERSION 9
+#define SDNET_ABI_VERSION 10
 
 /* element types of the four input tensors */
 #define SDNET_DTYPE_F32 0
@@ -47,7 +47,8 @@ extern "C" {
 /* argument errors */
 #define SDNET_E_NULL -1      /* a required pointer is NULL */
 #define SDNET_E_SHAPE -2     /* non-positive dimension, H*W >= 2^24, K or P > H*W (torch.topk: "k out of range"),
-                                K or P > SDNET_MAX_TOPK, M+N > SDNET_MAX_CHANNELS, T outside 1..SDNET_MAX_THRESHOLDS */
+                                K or P > SDNET_MAX_TOPK, M+N > SDNET_MAX_CHANNELS, T outside 1..SDNET_MAX_THRESHOLDS,
+                                G outside 0..SDNET_MAX_GATES */
 #define SDNET_E_STRIDE -3    /* innermost (w) stride is not 1 */
 #define SDNET_E_DTYPE -4     /* unsupported dtype */
 #define SDNET_E_WORKSPACE -5 /* workspace missing, misaligned (256 B) or smaller than sdnet_decode_workspace_bytes */
@@ -253,15 +254,20 @@ typedef struct SdnetObjectMatchParams {
 
 int sdnet_match_objects_launch(const SdnetObjectMatchParams* params, void* stream);
 
-/* Threshold sweep of the evaluator: for each of T confidence thresholds, what sdnet_match_launch and (with
- * SDNET_SWEEP_OBJECTS) sdnet_match_objects_launch compute on a decode at that threshold, from ONE decode.
- * anchor_out / part_out do not depend on the decoder's conf; only the grouping does, so it is redone per
- * threshold: anchors with score > conf_group[t] keep (x, y), the others sit at (+1e6, +1e6); parts with
- * score > conf_group[t] keep their origin, the others sit at (-1e6, -1e6); every part goes to the first anchor
- * at the smallest fp32 distance sqrt(dx*dx + dy*dy) (each step rounded, no FMA), if that distance is
- * < dist_abs_f32 (decoders.py:80-100, the full P x K search).  The `assign` and `counts` the decode wrote are not
- * read, so the decode's own conf does not matter; it must have grouped (part_out's origins are needed).
- * Every output is indexed [image][threshold]. */
+/* Threshold sweep of the evaluator: for each of T confidence thresholds, and for each of G grouping distances
+ * (gates), what sdnet_match_launch and (with SDNET_SWEEP_OBJECTS) sdnet_match_objects_launch compute on a decode at
+ * that threshold and gate, from ONE decode.  anchor_out / part_out do not depend on the decoder's conf or gate; only
+ * the grouping does, so it is redone per threshold: anchors with score > conf_group[t] keep (x, y), the others sit at
+ * (+1e6, +1e6); parts with score > conf_group[t] keep their origin, the others sit at (-1e6, -1e6); every part goes to
+ * the first anchor at the smallest fp32 distance sqrt(dx*dx + dy*dy) (each step rounded, no FMA), if that distance is
+ * < the gate (decoders.py:80-100, the full P x K search).  The search is done once per threshold; only the final
+ * compare is taken per gate.  The `assign` and `counts` the decode wrote are not read, so the decode's own conf and
+ * gate do not matter; it must have grouped (part_out's origins are needed).
+ * G = 0: one gate, dist_abs_f32, and every output is indexed [image][threshold] (as with ABI version 9).
+ * G >= 1: the gates are dist_abs_grid[0 .. G-1].  The location outputs (anchor_*, part_*) do not depend on the gate
+ * and stay indexed [image][threshold]; the object outputs (csi_*, classif_*, pred_parts) and assign_out are indexed
+ * [image][threshold][gate], row (b*T + t)*G + g. */
+#define SDNET_MAX_GATES 64
 #define SDNET_MAX_THRESHOLDS 256
 #define SDNET_SWEEP_OBJECTS 1u /* SdnetSweepParams.flags: also the object-level (CSI, classification) tables */
 typedef struct SdnetSweepParams {
@@ -270,7 +276,7 @@ typedef struct SdnetSweepParams {
   int32_t T;            /* thresholds, 1 .. SDNET_MAX_THRESHOLDS */
   int32_t max_gt_objects, max_gt_parts; /* row lengths of the ground-truth arrays, <= SDNET_MAX_GT */
   uint32_t flags;       /* SDNET_SWEEP_* */
-  float dist_abs_f32;   /* the decoder's gate: (float)(dist_thresh * min(W, H)) (decoders.py:100) */
+  float dist_abs_f32;   /* the decoder's gate: (float)(dist_thresh * min(W, H)) (decoders.py:100); read when G = 0 */
   double sx, sy;        /* heat-map -> network-input scale, in/out (decoders.py:139) */
   double csi_threshold; /* args.csi_threshold (evaluator.py:414); read with SDNET_SWEEP_OBJECTS */
   const double* conf;          /* (T): the evaluator's thresholds (objects: score > conf; raw parts: not score < conf) */
@@ -290,10 +296,12 @@ typedef struct SdnetSweepParams {
   double* part_acc;            /* (B, T, P) */
   int32_t* csi_stats;          /* (B, T, M, 3)   } SDNET_SWEEP_OBJECTS only: */
   double* csi_acc;             /* (B, T, K)      } as the fields of the same name */
-  int32_t* classif_stats;      /* (B, T, 20, 3)  } in SdnetObjectMatchParams */
-  double* classif_acc;         /* (B, T, K)      } */
+  int32_t* classif_stats;      /* (B, T, 20, 3)  } in SdnetObjectMatchParams; */
+  double* classif_acc;         /* (B, T, K)      } (B, T, G, ...) with G >= 1 */
   int32_t* pred_parts;         /* (B, T, K)      } */
-  int32_t* assign_out;         /* optional (B, T, P): the regrouped assignment (NULL to skip) */
+  int32_t* assign_out;         /* optional (B, T, P), (B, T, G, P) with G >= 1: the regrouped assignment (NULL to skip) */
+  int32_t G;                   /* gates, 0 .. SDNET_MAX_GATES; 0 = one gate, dist_abs_f32 */
+  const float* dist_abs_grid;  /* (G): the gates, each (float)(dist_thresh * min(W, H)) as dist_abs_f32; read when G >= 1 */
 } SdnetSweepParams;
 
 int sdnet_sweep_launch(const SdnetSweepParams* params, void* stream);

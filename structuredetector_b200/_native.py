@@ -13,7 +13,7 @@ import os as _os
 
 # SDNET_DECODE_LIB: load another build of the same library (kernel experiments, tools/xbuild.sh)
 LIB_PATH = Path(_os.environ.get("SDNET_DECODE_LIB") or Path(__file__).resolve().parent / "csrc" / "libsdnet_decode.so").resolve()
-ABI_VERSION = 9
+ABI_VERSION = 10
 DEST_PEER_STORES, DEST_MULTICAST = 0, 1  # SdnetDecodeParams.dest_mode
 
 FLAG_PRE_ACTIVATED = 1
@@ -29,6 +29,7 @@ MAX_CHANNELS = 255
 MAX_DEST = 16
 MAX_GT = 1024  # SDNET_MAX_GT
 MAX_THRESHOLDS = 256  # SDNET_MAX_THRESHOLDS
+MAX_GATES = 64  # SDNET_MAX_GATES
 SWEEP_OBJECTS = 1  # SdnetSweepParams.flags
 
 EXPORTS = (
@@ -151,6 +152,7 @@ class SdnetSweepParams(ctypes.Structure):
         ("csi_stats", ctypes.c_void_p), ("csi_acc", ctypes.c_void_p),
         ("classif_stats", ctypes.c_void_p), ("classif_acc", ctypes.c_void_p), ("pred_parts", ctypes.c_void_p),
         ("assign_out", ctypes.c_void_p),
+        ("G", ctypes.c_int32), ("dist_abs_grid", ctypes.c_void_p),
     ]
 
 

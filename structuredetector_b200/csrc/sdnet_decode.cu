@@ -541,7 +541,8 @@ int sdnet_sweep_launch(const SdnetSweepParams* p, void* stream) {
   const bool objects = (p->flags & SDNET_SWEEP_OBJECTS) != 0;
   if (!p->conf || !p->conf_group || !p->anchor_out || !p->part_out || !p->image_scale || !p->n_gt_objects ||
       !p->n_gt_parts || !p->anchor_stats || !p->part_stats || !p->anchor_acc || !p->part_acc ||
-      (p->max_gt_objects > 0 && !p->gt_objects) || (p->max_gt_parts > 0 && !p->gt_parts))
+      (p->max_gt_objects > 0 && !p->gt_objects) || (p->max_gt_parts > 0 && !p->gt_parts) ||
+      (p->G >= 1 && !p->dist_abs_grid))
     return SDNET_E_NULL;
   if (objects && (!p->cls_group || !p->csi_stats || !p->csi_acc || !p->classif_stats || !p->classif_acc ||
                   !p->pred_parts || (p->max_gt_parts > 0 && !p->gt_part_owner)))
@@ -549,7 +550,7 @@ int sdnet_sweep_launch(const SdnetSweepParams* p, void* stream) {
   if (p->B <= 0 || p->M <= 0 || p->N <= 0 || p->K <= 0 || p->P <= 0 || p->K > SDNET_MAX_TOPK || p->P > SDNET_MAX_TOPK ||
       p->M + p->N > SDNET_MAX_CHANNELS || p->T < 1 || p->T > SDNET_MAX_THRESHOLDS || p->max_gt_objects < 0 ||
       p->max_gt_parts < 0 || p->max_gt_objects > SDNET_MAX_GT || p->max_gt_parts > SDNET_MAX_GT ||
-      (long long)p->B * p->T > 0x7fffffffll)
+      p->G < 0 || p->G > SDNET_MAX_GATES || (long long)p->B * p->T * (p->G > 1 ? p->G : 1) > 0x7fffffffll)
     return SDNET_E_SHAPE;
   const size_t smem = sweep_smem_bytes(*p);
   cudaError_t err = cudaFuncSetAttribute(sdnet_sweep_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);

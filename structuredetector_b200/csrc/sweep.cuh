@@ -8,17 +8,21 @@ namespace {
 // `score > conf` only feeds its grouping and its counts), so a decode at any threshold holds every other
 // threshold's detections; what changes is the grouping, redone here:
 //   1. regroup at conf_group[t]: masked anchors at (+1e6, +1e6), masked part origins at (-1e6, -1e6)
-//      (decoders.py:80-86), every part to the first anchor at the smallest fp32 distance, gated
-//      (decoders.py:88-100).  The plain P x K search in slot order: no near-field restriction and no
-//      square-then-root shortcut as in tail.cuh, so it holds for any coordinate and any gate;
-//   2. location matching at conf[t] (match_pass, as sdnet_match_kernel);
-//   3. with SDNET_SWEEP_OBJECTS, object matching at conf[t] on the regrouped assignment (match_objects, as
-//      sdnet_match_objects_kernel).
-// The regrouped assignment lives at the front of the dynamic shared memory; the three phases share the rest.
+//      (decoders.py:80-86), every part's first anchor at the smallest fp32 distance (decoders.py:88-99).  The plain
+//      P x K search in slot order: no near-field restriction and no square-then-root shortcut as in tail.cuh, so it
+//      holds for any coordinate and any gate.  The search does not depend on the gate: its slot and distance are
+//      kept, and only the final `distance < gate` (decoders.py:100) is taken per gate in phase 3;
+//   2. location matching at conf[t] (match_pass, as sdnet_match_kernel), which never reads the grouping: once per
+//      (image, threshold), whatever the number of gates;
+//   3. per gate g: the assignment at dist_abs_grid[g] (dist_abs_f32 when G = 0) and, with SDNET_SWEEP_OBJECTS, object
+//      matching at conf[t] on it (match_objects, as sdnet_match_objects_kernel) into row (b*T + t)*G + g.
+// The nearest slots, their distances and the gated assignment live at the front of the dynamic shared memory (12 B
+// per part slot); the three phases share the rest.
 // ---------------------------------------------------------------------------------------------
 constexpr float kSweepFar = 1e6f;  // decoders.py:80-86 (kFar in tail.cuh)
 
-// Dynamic shared memory of one sweep CTA: assignment, then the largest of the three phases' scratch.
+// Dynamic shared memory of one sweep CTA: nearest slots, distances, assignment, then the largest of the three
+// phases' scratch.
 inline size_t sweep_smem_bytes(const SdnetSweepParams& p) {
   const size_t K = (size_t)p.K, P = (size_t)p.P;
   const size_t G = (size_t)(p.max_gt_objects > p.max_gt_parts ? p.max_gt_objects : p.max_gt_parts);
@@ -31,7 +35,7 @@ inline size_t sweep_smem_bytes(const SdnetSweepParams& p) {
                              ? match_objects_smem_bytes(p.max_gt_objects, p.max_gt_parts, p.K, p.P, p.M) : 0;
   size_t scratch = regroup > location ? regroup : location;
   if (objects > scratch) scratch = objects;
-  return (4 * P + 15) / 16 * 16 + scratch;
+  return (12 * P + 15) / 16 * 16 + scratch;
 }
 
 __global__ void __launch_bounds__(kMatchThreads) sdnet_sweep_kernel(const SdnetSweepParams p) {
@@ -39,12 +43,15 @@ __global__ void __launch_bounds__(kMatchThreads) sdnet_sweep_kernel(const SdnetS
   const int b = blockIdx.x / p.T, t = blockIdx.x - b * p.T;
   const size_t row = (size_t)b * p.T + t;
   const int K = p.K, P = p.P, tid = threadIdx.x, nt = blockDim.x;
-  int* s_assign = reinterpret_cast<int*>(sweep_smem);
-  unsigned char* scratch = sweep_smem + ((size_t)4 * P + 15) / 16 * 16;
+  const int n_gates = p.G > 0 ? p.G : 1;
+  int* s_arg = reinterpret_cast<int*>(sweep_smem);
+  float* s_best = reinterpret_cast<float*>(s_arg + P);
+  int* s_assign = reinterpret_cast<int*>(s_best + P);
+  unsigned char* scratch = sweep_smem + ((size_t)12 * P + 15) / 16 * 16;
   const float* A = p.anchor_out + (size_t)b * K * 4;
   const float* Q = p.part_out + (size_t)b * P * 6;
 
-  // ---- 1. regroup at conf_group[t]
+  // ---- 1. nearest anchor of every part at conf_group[t]
   {
     const float cg = p.conf_group[t];
     float2* s_apos = reinterpret_cast<float2*>(scratch);
@@ -64,9 +71,8 @@ __global__ void __launch_bounds__(kMatchThreads) sdnet_sweep_kernel(const SdnetS
         const float d = __fsqrt_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)));
         if (d < best) { best = d; arg = a; }
       }
-      const int slot = (arg >= 0 && best < p.dist_abs_f32) ? arg : -1;
-      s_assign[q] = slot;
-      if (p.assign_out) p.assign_out[row * P + q] = slot;
+      s_arg[q] = arg;
+      s_best[q] = best;
     }
     __syncthreads();
   }
@@ -94,9 +100,10 @@ __global__ void __launch_bounds__(kMatchThreads) sdnet_sweep_kernel(const SdnetS
                s_glab, s_winner, s_jmin, s_dist, s_stats);
   }
 
-  // ---- 3. object matching at conf[t] on the regrouped assignment (match_pass ends with a barrier)
-  if (p.flags & SDNET_SWEEP_OBJECTS) {
-    SdnetObjectMatchParams op;
+  // ---- 3. per gate: the gated assignment, then object matching at conf[t] on it (match_pass ends with a barrier)
+  const bool objects = (p.flags & SDNET_SWEEP_OBJECTS) != 0;
+  SdnetObjectMatchParams op;
+  if (objects) {
     op.K = K; op.P = P; op.M = p.M; op.N = p.N; op.B = p.B;
     op.max_gt_objects = p.max_gt_objects; op.max_gt_parts = p.max_gt_parts;
     op.conf = conf; op.sx = p.sx; op.sy = p.sy; op.csi_threshold = p.csi_threshold;
@@ -107,7 +114,21 @@ __global__ void __launch_bounds__(kMatchThreads) sdnet_sweep_kernel(const SdnetS
     op.cls_group = p.cls_group;
     op.csi_stats = p.csi_stats; op.csi_acc = p.csi_acc;
     op.classif_stats = p.classif_stats; op.classif_acc = p.classif_acc; op.pred_parts = p.pred_parts;
-    match_objects(op, b, row, s_assign, scratch);
+  }
+  for (int g = 0; g < n_gates; ++g) {
+    const float gate = p.G > 0 ? p.dist_abs_grid[g] : p.dist_abs_f32;
+    const size_t grow = row * n_gates + g;
+    for (int q = tid; q < P; q += nt) {
+      const int arg = s_arg[q];
+      const int slot = (arg >= 0 && s_best[q] < gate) ? arg : -1;
+      s_assign[q] = slot;
+      if (p.assign_out) p.assign_out[grow * P + q] = slot;
+    }
+    if (objects) {
+      __syncthreads();
+      match_objects(op, b, grow, s_assign, scratch);
+      __syncthreads();  // the next gate overwrites the assignment match_objects reads
+    }
   }
 }
 

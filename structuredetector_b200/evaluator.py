@@ -8,7 +8,8 @@ against their nearest ground truth -- through ``sdnet_match_launch``; ``eval_csi
 (:380-420, 539-581) and ``eval_classif`` (:429-474) -- predicted objects (anchor + grouped parts) against
 ground-truth objects -- through ``sdnet_match_objects_launch``; both straight on the tensors
 ``sdnet_decode_launch`` wrote: no Python object is built for a prediction.  ``ThresholdSweep`` runs both at many
-confidence thresholds from one decode (``sdnet_sweep_launch``): the precision / recall / F1 curve over the threshold.
+confidence thresholds, and optionally grouping distances, from one decode (``sdnet_sweep_launch``): the precision /
+recall / F1 curve over the threshold, or its surface over (threshold, grouping distance).
 """
 from __future__ import annotations
 
@@ -378,8 +379,12 @@ class Evaluator:
         return text
 
 
+# Device bytes one sweep launch may write; accumulate_packed splits a larger batch into consecutive image slices.
+SWEEP_OUTPUT_BUDGET = 1 << 30
+
+
 class ThresholdSweep:
-    """The evaluator at a grid of confidence thresholds, from one decode.
+    """The evaluator at a grid of confidence thresholds, and optionally of grouping distances, from one decode.
 
     ``at(t)`` is a plain ``Evaluator`` holding exactly what ``Evaluator.accumulate_packed(decode at t, ...,
     conf_thresh=t)`` would hold, for every decode and evaluation this sweep has accumulated: the detections a decoder
@@ -390,12 +395,18 @@ class ThresholdSweep:
     ``thresholds``: finite, strictly increasing, at most 256.  ``dtype``: the dtype of the heat maps the detections
     were decoded from -- the grouping compares ``score > t`` in that dtype, as the decoder does.  ``dist_thresh``: the
     decoder's grouping distance (default ``args.decoder_dist_thresh``); ``args`` as for ``Evaluator``.
+
+    ``gates``: a grid of grouping distances instead of the one ``dist_thresh`` -- ``decoder_dist_thresh`` values
+    (fractions of min(W, H)), finite, >= 0, strictly increasing, at most 64.  ``at(t, gate)`` is then what a decode at
+    (t, gate) evaluated at t would hold; ``surface`` and ``best`` read the (threshold x gate) grid.  The nearest-anchor
+    search and the location tables do not depend on the gate: they are computed once per threshold.
     """
 
     TABLES = {"anchor": "anchor_eval", "part": "part_eval", "kps": "kps_eval", "csi": "csi_eval",
               "classification": "classification_eval"}
+    _LOCATION = ("anchor_eval", "part_eval")
 
-    def __init__(self, args, thresholds, *, dtype: torch.dtype = torch.float32, dist_thresh=None):
+    def __init__(self, args, thresholds, *, dtype: torch.dtype = torch.float32, dist_thresh=None, gates=None):
         values = [float(t) for t in thresholds]
         if not values or len(values) > _native.MAX_THRESHOLDS:
             raise ValueError(f"{len(values)} thresholds; a sweep takes 1 to {_native.MAX_THRESHOLDS}")
@@ -405,41 +416,90 @@ class ThresholdSweep:
             raise ValueError("thresholds must be strictly increasing")
         if dtype not in ops._DTYPES:
             raise ValueError(f"dtype {dtype} is not a heat-map dtype of the decoder (float32, float16, bfloat16)")
+        if gates is not None:
+            if dist_thresh is not None:
+                raise ValueError("pass either dist_thresh or gates, not both")
+            gate_values = [float(g) for g in gates]
+            if not gate_values or len(gate_values) > _native.MAX_GATES:
+                raise ValueError(f"{len(gate_values)} gates; a sweep takes 1 to {_native.MAX_GATES}")
+            if not all(math.isfinite(g) and g >= 0 for g in gate_values):
+                raise ValueError("gates must be finite and >= 0")
+            if any(b <= a for a, b in zip(gate_values, gate_values[1:])):
+                raise ValueError("gates must be strictly increasing")
         self.args = args
         self.thresholds = np.array(values, dtype=np.float64)
         self.dtype = dtype
-        self.dist_thresh = float(args.decoder_dist_thresh if dist_thresh is None else dist_thresh)
-        self._evaluators = [Evaluator(args) for _ in values]
+        if gates is None:
+            self.dist_thresh = float(args.decoder_dist_thresh if dist_thresh is None else dist_thresh)
+            self.gates = np.array([self.dist_thresh], dtype=np.float64)
+        else:
+            self.dist_thresh = None
+            self.gates = np.array(gate_values, dtype=np.float64)
+        self._gated = gates is not None  # launch with the gate grid (G >= 1) rather than the one dist_abs_f32 (G = 0)
+        self._grid = [[Evaluator(args) for _ in self.gates] for _ in values]  # [threshold][gate]
         self.lib = _native.load()
         self.last_copy_bytes = 0  # device -> host bytes of the last accumulate_packed
 
     def reset(self):
-        for ev in self._evaluators:
-            ev.reset()
+        for row in self._grid:
+            for ev in row:
+                ev.reset()
 
-    def at(self, t) -> Evaluator:
-        """The ``Evaluator`` of grid point ``t`` (``KeyError`` if ``t`` is not on the grid)."""
+    def _gate_index(self, gate) -> int:
+        if gate is None:
+            if len(self.gates) != 1:
+                raise KeyError(f"this sweep has {len(self.gates)} gates: name one")
+            return 0
+        hit = np.flatnonzero(self.gates == float(gate))
+        if hit.size == 0:
+            raise KeyError(gate)
+        return int(hit[0])
+
+    def at(self, t, gate=None) -> Evaluator:
+        """The ``Evaluator`` of grid point (``t``, ``gate``); ``gate`` may be left out when the sweep has one gate
+        (``KeyError`` otherwise, and for a point not on the grid)."""
         hit = np.flatnonzero(self.thresholds == float(t))
         if hit.size == 0:
             raise KeyError(t)
-        return self._evaluators[int(hit[0])]
+        return self._grid[int(hit[0])][self._gate_index(gate)]
 
     def accumulate_packed(self, packed: ops.PackedDetections, annotations, out_size, eval_csi=False, eval_classif=False):
-        """Add one decoded batch at every threshold of the grid.  Arguments as for ``Evaluator.accumulate_packed``, but
+        """Add one decoded batch at every point of the grid.  Arguments as for ``Evaluator.accumulate_packed``, but
         ``packed`` must come from a decode WITH grouping (``Decoder``, ``CoreMLDecoder``, ``ops.decode_packed(...,
-        group=True)``), because the part origins are regrouped; the threshold it was decoded at does not matter: its
-        ``assign`` and ``counts`` are not read."""
-        ev0 = self._evaluators[0]
+        group=True)``), because the part origins are regrouped; the threshold and gate it was decoded at do not matter:
+        its ``assign`` and ``counts`` are not read."""
+        ev0 = self._grid[0][0]
         B, K = packed.anchor_inds.shape
         P = packed.part_inds.shape[1]
-        T = len(self.thresholds)
+        T, G = len(self.thresholds), len(self.gates)
         if len(annotations) != B:
             raise ValueError(f"{len(annotations)} annotations for a batch of {B} images")
         device = packed.anchor_out.device
         M, N = len(ev0._label_index), len(ev0._part_index)
-        (gt_a, n_a, wa), (gt_p, n_p, wp), scale, owner = ev0._pack_ground_truth(annotations, device)
+        gt = ev0._pack_ground_truth(annotations, device)
         if device.type != "cuda":
             raise RuntimeError(f"the packed detections live on {device}: the sweep runs on a CUDA device only")
+        objects = eval_csi or eval_classif
+        # device bytes one image's outputs take; the batch goes through in slices that stay under the budget
+        per_image = T * (12 * (M + N) + 8 * (K + P))
+        if objects:
+            per_image += T * G * (12 * M + 240 + 20 * K)
+        step = max(1, SWEEP_OUTPUT_BUDGET // per_image)
+        self.last_copy_bytes = 0
+        for b0 in range(0, B, step):
+            self._accumulate_slice(packed, gt, b0, min(B, b0 + step), out_size, eval_csi, eval_classif)
+
+    def _accumulate_slice(self, packed, gt, b0, b1, out_size, eval_csi, eval_classif):
+        """One launch over images b0 .. b1-1 of the batch (``gt`` = the whole batch's packed ground truth), absorbed
+        into every grid point after the images before b0."""
+        ev0 = self._grid[0][0]
+        B, K, P = b1 - b0, packed.anchor_inds.shape[1], packed.part_inds.shape[1]
+        T, G = len(self.thresholds), len(self.gates)
+        device = packed.anchor_out.device
+        M, N = len(ev0._label_index), len(ev0._part_index)
+        (gt_a, n_a, wa), (gt_p, n_p, wp), scale, owner = gt
+        gt_a, n_a, gt_p, n_p, scale, owner = (x[b0:b1] for x in (gt_a, n_a, gt_p, n_p, scale, owner))
+        anchor_out, part_out = packed.anchor_out[b0:b1], packed.part_out[b0:b1]
         objects = eval_csi or eval_classif
         out_w, out_h = out_size
         in_w, in_h = int(self.args.down_ratio * out_w), int(self.args.down_ratio * out_h)  # decoders.py:37-38
@@ -452,26 +512,31 @@ class ThresholdSweep:
         prm.struct_size = ctypes.sizeof(_native.SdnetSweepParams)
         prm.B, prm.M, prm.N, prm.K, prm.P, prm.T = B, M, N, K, P, T
         prm.max_gt_objects, prm.max_gt_parts = wa, wp
-        prm.dist_abs_f32 = ops._f32(self.dist_thresh * min(out_w, out_h))  # as ops.decode_packed
+        if self._gated:  # as ops.decode_packed rounds its gate
+            grid = torch.tensor([ops._f32(g * min(out_w, out_h)) for g in self.gates], dtype=torch.float32, device=device)
+            prm.G, prm.dist_abs_grid = G, grid.data_ptr()
+        else:
+            prm.dist_abs_f32 = ops._f32(self.dist_thresh * min(out_w, out_h))  # as ops.decode_packed
         prm.sx, prm.sy = in_w / out_w, in_h / out_h
         prm.csi_threshold = float(getattr(self.args, "csi_threshold", 0.75))
         prm.conf, prm.conf_group = conf.data_ptr(), conf_group.data_ptr()
-        prm.anchor_out, prm.part_out = packed.anchor_out.data_ptr(), packed.part_out.data_ptr()
+        prm.anchor_out, prm.part_out = anchor_out.data_ptr(), part_out.data_ptr()
         prm.image_scale = scale.data_ptr()
         prm.gt_objects, prm.n_gt_objects = gt_a.data_ptr(), n_a.data_ptr()
         prm.gt_parts, prm.gt_part_owner, prm.n_gt_parts = gt_p.data_ptr(), owner.data_ptr(), n_p.data_ptr()
         prm.anchor_stats, prm.part_stats = a_stats.data_ptr(), p_stats.data_ptr()
         prm.anchor_acc, prm.part_acc = a_acc.data_ptr(), p_acc.data_ptr()
-        a_cls = packed.anchor_out[:, :, 3].to(torch.int32)
-        p_cls = packed.part_out[:, :, 3].to(torch.int32)
-        # (evaluations of each grid point, names, stats (B, T, C, 3), acc (B, T, slots), label of each acc (B, T, slots))
+        a_cls = anchor_out[:, :, 3].to(torch.int32)
+        p_cls = part_out[:, :, 3].to(torch.int32)
+        # (evaluations of each grid point, names, stats (B, R, C, 3), acc (B, R, slots), label of each acc (B, R, slots)):
+        # R = T rows for the location tables, T * G rows (threshold-major) for the object tables
         tables = [("anchor_eval", ev0._label_names, a_stats, a_acc, a_cls[:, None].expand(B, T, K)),
                   ("part_eval", ev0._part_names, p_stats, p_acc, p_cls[:, None].expand(B, T, P))]
         if objects:
             groups = ev0._classification_groups(device)
-            c_stats, k_stats = torch.empty(B, T, M, 3, **i32), torch.empty(B, T, 20, 3, **i32)
-            c_acc, k_acc = torch.empty(B, T, K, **f64), torch.empty(B, T, K, **f64)
-            n_parts = torch.empty(B, T, K, **i32)
+            c_stats, k_stats = torch.empty(B, T * G, M, 3, **i32), torch.empty(B, T * G, 20, 3, **i32)
+            c_acc, k_acc = torch.empty(B, T * G, K, **f64), torch.empty(B, T * G, K, **f64)
+            n_parts = torch.empty(B, T * G, K, **i32)
             prm.flags = _native.SWEEP_OBJECTS
             prm.cls_group = groups.data_ptr()
             prm.csi_stats, prm.csi_acc = c_stats.data_ptr(), c_acc.data_ptr()
@@ -479,54 +544,76 @@ class ThresholdSweep:
         stream = torch.cuda.current_stream(device).cuda_stream
         _native.check(self.lib.sdnet_sweep_launch(ctypes.byref(prm), ctypes.c_void_p(stream)), "sdnet_sweep_launch")
         if eval_csi:
-            tables.append(("csi_eval", ev0._label_names, c_stats, c_acc, a_cls[:, None].expand(B, T, K)))
+            tables.append(("csi_eval", ev0._label_names, c_stats, c_acc, a_cls[:, None].expand(B, T * G, K)))
         if eval_classif:
             g = groups[a_cls.clamp(0, M - 1).long()][:, None]  # as Evaluator.accumulate_packed's classification key
             key = torch.where((n_parts >= 0) & (n_parts <= 9), g * 10 + n_parts, -1)
             tables.append(("classification_eval", dict(enumerate(Evaluator.get_classification_labels())), k_stats, k_acc,
                            torch.where(g >= 0, key, -1)))
-        # Only the true positives' values cross to the host: per table, the non-NaN accumulators in (threshold, image,
-        # slot) order with their labels, and the per-threshold totals.
+        # Only the true positives' values cross to the host: per table, the non-NaN accumulators in (row, image, slot)
+        # order with their labels, and the per-row totals.
         stats, hits, vals, labs = [], [], [], []
         for _, _, st, acc, cls in tables:
-            acc, cls = acc.transpose(0, 1), cls.transpose(0, 1)  # (T, B, slots)
+            acc, cls = acc.transpose(0, 1), cls.transpose(0, 1)  # (R, B, slots)
             hit = ~torch.isnan(acc)
             stats.append(st.sum(dim=0, dtype=torch.int64).flatten())
             hits.append(hit.sum(dim=(1, 2)))
             vals.append(acc[hit])
             labs.append(cls[hit].to(torch.int32))
         host = [torch.cat(x).cpu().numpy() for x in (stats, hits, vals, labs)]
-        self.last_copy_bytes = sum(x.nbytes for x in host)
+        self.last_copy_bytes += sum(x.nbytes for x in host)
         h_stats, h_hits, h_vals, h_labs = host
         s_off = h_off = v_off = 0
         for attr, names, st, _, _ in tables:
-            per_t = st.shape[2] * 3
-            for t, ev in enumerate(self._evaluators):
-                n = int(h_hits[h_off + t])
-                Evaluator._absorb(getattr(ev, attr), names, h_stats[s_off: s_off + per_t].reshape(1, -1, 3),
-                                  h_vals[v_off: v_off + n], h_labs[v_off: v_off + n])
-                s_off += per_t
+            per_row, rows = st.shape[2] * 3, st.shape[1]
+            for r in range(rows):
+                n = int(h_hits[h_off + r])
+                # a location row is threshold r at every gate; an object row is (threshold r // G, gate r % G)
+                targets = self._grid[r] if attr in self._LOCATION else [self._grid[r // G][r % G]]
+                for ev in targets:
+                    Evaluator._absorb(getattr(ev, attr), names, h_stats[s_off: s_off + per_row].reshape(1, -1, 3),
+                                      h_vals[v_off: v_off + n], h_labs[v_off: v_off + n])
+                s_off += per_row
                 v_off += n
-            h_off += T
+            h_off += rows
 
-    def curve(self, table: str, label=None) -> dict:
-        """Per grid point: threshold, tp, npos, ndet, precision, recall, f1_score of ``table`` (anchor, part, kps, csi,
-        classification) for ``label``, or for all its labels together (``Evaluations.reduce``) when ``label`` is None."""
+    def _rows(self, table, label, cells):
         if table not in self.TABLES:
             raise ValueError(f"unknown table {table!r}; one of {sorted(self.TABLES)}")
         rows = []
-        for ev in self._evaluators:
+        for ev in cells:
             evals = getattr(ev, self.TABLES[table])
             e = evals.reduce() if label is None else evals[label]
             rows.append((e.tp, e.npos, e.ndet, e.precision, e.recall, e.f1_score))
         cols = list(zip(*rows))
-        out = {"threshold": self.thresholds.copy()}
+        out = {}
         for i, name in enumerate(("tp", "npos", "ndet")):
             out[name] = np.array(cols[i], dtype=np.int64)
         for i, name in enumerate(("precision", "recall", "f1_score"), start=3):
             out[name] = np.array(cols[i], dtype=np.float64)
         return out
 
-    def best_threshold(self, table: str, label=None) -> float:
-        """The grid threshold with the highest F1 score of ``table`` / ``label`` (the lowest one on a tie)."""
-        return float(self.thresholds[int(np.argmax(self.curve(table, label)["f1_score"]))])
+    def curve(self, table: str, label=None, gate=None) -> dict:
+        """Per grid threshold, at ``gate`` (may be left out when the sweep has one gate): threshold, tp, npos, ndet,
+        precision, recall, f1_score of ``table`` (anchor, part, kps, csi, classification) for ``label``, or for all its
+        labels together (``Evaluations.reduce``) when ``label`` is None."""
+        j = self._gate_index(gate)
+        return {"threshold": self.thresholds.copy(), **self._rows(table, label, [row[j] for row in self._grid])}
+
+    def best_threshold(self, table: str, label=None, gate=None) -> float:
+        """The grid threshold with the highest F1 score of ``table`` / ``label`` at ``gate`` (the lowest one on a tie)."""
+        return float(self.thresholds[int(np.argmax(self.curve(table, label, gate)["f1_score"]))])
+
+    def surface(self, table: str, label=None) -> dict:
+        """``curve`` over the whole grid: threshold (T,), gate (G,), and tp, npos, ndet, precision, recall, f1_score
+        as (T, G) arrays."""
+        T, G = len(self.thresholds), len(self.gates)
+        out = self._rows(table, label, [ev for row in self._grid for ev in row])
+        return {"threshold": self.thresholds.copy(), "gate": self.gates.copy(),
+                **{name: v.reshape(T, G) for name, v in out.items()}}
+
+    def best(self, table: str, label=None) -> tuple:
+        """The (threshold, gate) with the highest F1 score of ``table`` / ``label``; on a tie the lowest threshold, then
+        the lowest gate."""
+        t, g = np.unravel_index(int(np.argmax(self.surface(table, label)["f1_score"])), (len(self.thresholds), len(self.gates)))
+        return float(self.thresholds[t]), float(self.gates[g])
