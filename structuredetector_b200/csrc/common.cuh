@@ -74,6 +74,14 @@ struct PeaksParams {
 template <int DT>
 struct Num;
 
+// For logits x < h: false only where S(x) < S(h) is certain (outside the zones above), so the exact
+// scores need comparing only where it is true.  The first zone is tested for any h, a superset.
+template <int DT>
+__device__ __forceinline__ bool may_tie(float x, float h) {
+  return (x >= h - Num<DT>::kNear) || (h > Num<DT>::kHi && x >= h - Num<DT>::kNear2) ||
+         (h > Num<DT>::kHi2 && x > Num<DT>::kHi2 - 1.0f) || (h < Num<DT>::kLo);
+}
+
 template <>
 struct Num<SDNET_DTYPE_F32> {
   typedef float In;
@@ -166,25 +174,13 @@ __device__ __forceinline__ void mbar_arrive_expect_tx(u32 bar, u32 bytes) {
 // try_wait with a suspend-time hint: the warp sleeps until the phase completes instead of spinning.
 // Measured: a spinning test_wait streams faster when nothing else runs (0.62 vs 0.94 ms with the
 // slow path disabled) but steals issue slots from the working warps in the real kernel (0.724 vs 0.718 ms).
-#ifndef SDNET_X_WAIT_NS
-#define SDNET_X_WAIT_NS 1000
-#endif
 __device__ __forceinline__ void mbar_wait(u32 bar, u32 parity) {
-#if SDNET_X_WAIT_NS > 0
   asm volatile(
       "{\n\t.reg .pred p;\n"
       "WAIT_LOOP:\n\t"
       "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1, %2;\n\t"
       "@!p bra WAIT_LOOP;\n\t}"
-      ::"r"(bar), "r"(parity), "r"((u32)SDNET_X_WAIT_NS) : "memory");
-#else  // no suspend-time hint: the hardware's default time limit
-  asm volatile(
-      "{\n\t.reg .pred p;\n"
-      "WAIT_LOOP:\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-      "@!p bra WAIT_LOOP;\n\t}"
-      ::"r"(bar), "r"(parity) : "memory");
-#endif
+      ::"r"(bar), "r"(parity), "r"(1000u) : "memory");  // suspend-time hint, ns
 }
 __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 

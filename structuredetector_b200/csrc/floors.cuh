@@ -5,21 +5,7 @@
 
 namespace {
 
-#ifndef SDNET_X_BUF
-#define SDNET_X_BUF 64
-#endif
-constexpr int kBuf = SDNET_X_BUF;      // per-warp candidate buffer (records), a multiple of 32
-#ifndef SDNET_X_GRATE
-#define SDNET_X_GRATE 0
-#endif
-#ifndef SDNET_X_LRATE
-#define SDNET_X_LRATE 0
-#endif
-// Floors are recomputed from the histograms only when that can change them: the plane-wide floor needs K
-// recorded candidates in the plane, the warp-local one K in the unit; beyond that, every kGRate / kLRate
-// new records (0 = at every flush).
-constexpr int kGRate = SDNET_X_GRATE, kLRate = SDNET_X_LRATE;
-constexpr int kGDiv = kGRate ? kGRate : 1, kLDiv = kLRate ? kLRate : 1;
+constexpr int kBuf = 64;  // per-warp candidate buffer (records), a multiple of 32
 
 __device__ __forceinline__ int logit_bin(float x) {
   int bin = __float2int_rd((x - kBinLo) * kBinScale);
@@ -193,15 +179,16 @@ __device__ __forceinline__ void flush_candidates(UnitState& st, const u64* buf, 
       }
     }
   }
-  const u32 before = st.emitted;
   st.emitted += n;
   st.nbuf = 0;
   __syncwarp();
+  // Floors are recomputed from the histograms, at every flush, once that can change them: the warp-local
+  // floor needs K recorded candidates in the unit, the plane-wide one K in the plane.
   // xscale is a power of two, so the division is exact
-  if (st.emitted >= (u32)K && (kLRate == 0 || before < (u32)K || before / kLDiv != st.emitted / kLDiv))
+  if (st.emitted >= (u32)K)
     st.floorx = fmaxf(st.floorx, local_floor(hist, minx, lane, K) / xscale);
   // publish / refresh the shared floors (`base` = records in the plane before this flush)
-  if (sf.ghist && base + n >= K && (kGRate == 0 || base < K || base / kGDiv != (base + n) / kGDiv)) {
+  if (sf.ghist && base + n >= K) {
     const int gb = floor_bin_fine<false>(sf.ghist, lane, K);
     if (gb > 0) {
       if (lane == 0) atomicMax(sf.gfloor, gb);

@@ -22,24 +22,12 @@ constexpr int kGroupRows = 4;                                // output rows per 
 constexpr int kTileCols = kPanelW + 8;
 constexpr int kTilePitchB = kTileCols * 4;                   // 544 B per ring row
 constexpr int kTileBytes = kGroupRows * kTilePitchB;         // 2176 B per TMA tile (17 x 128 B)
-#ifndef SDNET_X_WARPS
-#define SDNET_X_WARPS 4
-#endif
-constexpr int kTileWarps = SDNET_X_WARPS;  // warps per CTA; they never talk to each other (no __syncthreads in the kernel)
-#ifndef SDNET_X_CTAS
-#define SDNET_X_CTAS (24 / SDNET_X_WARPS)
-#endif
-constexpr int kTileMinCtas = SDNET_X_CTAS;  // resident CTAs per SM the register allocation aims for (24 warps)
+constexpr int kTileWarps = 4;  // warps per CTA; they never talk to each other (no __syncthreads in the kernel)
+constexpr int kTileMinCtas = 6;  // resident CTAs per SM the register allocation aims for (24 warps)
 constexpr int kMinChunkGroups = 8;  // shortest tier-2 unit (32 rows)
-#ifndef SDNET_X_NG
-#define SDNET_X_NG 3
-#endif
-constexpr int kTileNG = SDNET_X_NG;   // ring slots (tiles) per warp: a group reads two of them, the others are in flight
-#ifndef SDNET_X_FLUSH_AT
-#define SDNET_X_FLUSH_AT 16
-#endif
+constexpr int kTileNG = 3;   // ring slots (tiles) per warp: a group reads two of them, the others are in flight
 constexpr int kWork = 128;   // per-warp work list: one byte per (row of the group, lane) whose 16-byte word holds a pixel above the floor
-constexpr int kFlushAt = SDNET_X_FLUSH_AT;  // buffered candidates that trigger a flush once the plane has a floor
+constexpr int kFlushAt = 16;  // buffered candidates that trigger a flush
 // S = rows per TMA row (see the kernel).  Under S = 2 a tile arrives as two 2-row boxes and a TMA
 // destination must be 128-byte aligned: the second box sits at +1152 and a slot takes 2304 bytes.
 __host__ __device__ constexpr int tile_slot_bytes(int S) { return S == 1 ? kTileBytes : 2304; }
@@ -162,21 +150,6 @@ __device__ __forceinline__ u32 ring_row_off(u32 rr) {
   return (rr >> 2) * tile_slot_bytes(2) + (rr & 1u) * (kOddBoxOff + kOddShiftB) + ((rr >> 1) & 1u) * kTilePitchB;
 }
 
-#ifndef SDNET_X_TRACE
-#define SDNET_X_TRACE 0
-#endif
-#ifndef SDNET_X_WARMPOLL
-#define SDNET_X_WARMPOLL 1  // poll the published floor every group, synchronously, while this warp has none
-#endif
-#ifndef SDNET_X_EARLYFLUSH
-#define SDNET_X_EARLYFLUSH 0  // 1: flush after every group while the plane has no floor (the pre-early-histogram rule)
-#endif
-#ifndef SDNET_X_QUICK
-#define SDNET_X_QUICK 1  // settle_entries: reject flank pixels on their four direct neighbours before the full window
-#endif
-#ifndef SDNET_X_EARLYHIST
-#define SDNET_X_EARLYHIST 1  // count a candidate in the plane-wide histogram when it is found, not when it is flushed
-#endif
 // Settle the work list of one 4-row group.  Entry e = (row in group << 5) | lane names one 16-byte
 // word of centre pixels holding at least one pixel above the floor; kPx consecutive lanes take the
 // pixels of an entry.  (Listing the two halves of a fp16 / bf16 word separately -- twice the ballots, half the
@@ -190,8 +163,6 @@ __device__ __forceinline__ void settle_entries(UnitState& st, const unsigned cha
                                                u32 row_tab, float floorx, u32 idx0, int W, bool pre, u64* buf, u32* hist, int* minx,
                                                const SharedFloors& sf, int* count_ptr, u64* __restrict__ list, int cap,
                                                int K, int lane, float xscale, float satx) {
-  constexpr float kNearTie = Num<DT>::kNear, kHiZone = Num<DT>::kHi, kLoZone = Num<DT>::kLo, kNearTie2 = Num<DT>::kNear2,
-                  kHiZone2 = Num<DT>::kHi2;
   constexpr u32 kRingRows = kTileNG * kGroupRows;
   constexpr int kPx = TileGeom<DT>::kPx, kEsz = TileGeom<DT>::kEsz;
   const int nslots = kPx * nent;
@@ -211,7 +182,6 @@ __device__ __forceinline__ void settle_entries(UnitState& st, const unsigned cha
     }
     const float x = TileMax<DT>::elem(col_addr + R * kEsz + roff[R]);
     bool keep = slot < nslots && x > floorx;
-#if SDNET_X_QUICK
     if (!pre) {
       // Most pixels above the floor are not peaks but the flanks of one (a blob holds ~200 of them): four loads
       // settle those.  With m4 = the largest of the four direct neighbours (<= the window maximum h), x cannot
@@ -220,9 +190,8 @@ __device__ __forceinline__ void settle_entries(UnitState& st, const unsigned cha
       const u32 ctr = col_addr + R * kEsz;
       const float m4 = fmaxf(fmaxf(TileMax<DT>::elem(ctr + roff[R - 1]), TileMax<DT>::elem(ctr + roff[R + 1])),
                              fmaxf(TileMax<DT>::elem(ctr - kEsz + roff[R]), TileMax<DT>::elem(ctr + kEsz + roff[R])));
-      if (x < m4 - kNearTie2 && x <= kHiZone2 - 1.0f && x >= kLoZone) keep = false;
+      if (x < m4 - Num<DT>::kNear2 && x <= Num<DT>::kHi2 - 1.0f && x >= Num<DT>::kLo) keep = false;
     }
-#endif
     if (keep && !pre) {
       // window max in the storage format (no conversions for fp16/bf16), one accumulator per window row
       u32 hr[2 * R + 1];
@@ -239,23 +208,18 @@ __device__ __forceinline__ void settle_entries(UnitState& st, const unsigned cha
 #pragma unroll
       for (int d = 1; d <= 2 * R; ++d) hr[0] = TileMax<DT>::rmax(hr[0], hr[d]);
       const float h = fmaxf(x, TileMax<DT>::rfloat(hr[0]));  // an all-NaN window cannot happen: the centre is in it
-      if (x != h) {
-        const bool amb = (x >= h - kNearTie) || (h > kHiZone && x >= h - kNearTie2) ||
-                         (h > kHiZone2 && x > kHiZone2 - 1.0f) || (h < kLoZone);  // same zones as classify_row
-        keep = amb && Num<DT>::act(x) == Num<DT>::act(h);  // rare
-      }
+      if (x != h) keep = may_tie<DT>(x, h) && Num<DT>::act(x) == Num<DT>::act(h);  // rare
     }
     const u32 m = __ballot_sync(0xffffffffu, keep);
     if (m) {  // warp-uniform
       if (st.nbuf + __popc(m) > kBuf) {
         __syncwarp();
-        flush_candidates<DT, !SDNET_X_EARLYHIST>(st, buf, hist, minx, sf, count_ptr, list, cap, K, lane, pre, xscale, satx);
+        flush_candidates<DT, false>(st, buf, hist, minx, sf, count_ptr, list, cap, K, lane, pre, xscale, satx);
       }
       if (keep) {
         buf[st.nbuf + __popc(m & ((1u << lane) - 1u))] = ((u64)__float_as_uint(x) << 32) | (idx0 + i * (u32)W + colp);
-#if SDNET_X_EARLYHIST
-        atomicAdd(&sf.ghist[fine_bin(fminf(fmaxf(x * xscale, -satx), satx))], 1u);  // the plane's other warps see it at once
-#endif
+        // counted in the plane-wide histogram when found, not when flushed: the plane's other warps see it at once
+        atomicAdd(&sf.ghist[fine_bin(fminf(fmaxf(x * xscale, -satx), satx))], 1u);
       }
       st.nbuf += __popc(m);
     }
@@ -270,10 +234,7 @@ __device__ __forceinline__ void settle_entries(UnitState& st, const unsigned cha
 // adjacent lanes by shuffle, and classifies its 16 pixels exactly like the pixel-centric path.  ~300 instructions for
 // the group, whatever the number of hot pixels.  Returns false (nothing recorded) when the group holds more
 // survivors than the candidate buffer: the caller then takes the pixel-centric path, which flushes as it goes.
-#ifndef SDNET_X_DENSE
-#define SDNET_X_DENSE 16
-#endif
-constexpr int kDenseLanes = SDNET_X_DENSE;  // hot lanes from which the dense path is taken (0 = never)
+constexpr int kDenseLanes = 16;  // hot lanes from which the dense path is taken
 
 
 // The dense maximum filter of one 4-row group (fp32, plain rows): bit 4 i + c of the result says that pixel
@@ -281,7 +242,6 @@ constexpr int kDenseLanes = SDNET_X_DENSE;  // hot lanes from which the dense pa
 template <int R>
 __device__ __forceinline__ u32 dense_keep_mask_f32(int rows_here, u32 ring_s, u32 ring_own, u32 row0, float floorx, bool pre, int lane) {
   constexpr int DT = SDNET_DTYPE_F32;
-  constexpr float kNearTie = Num<DT>::kNear, kHiZone = Num<DT>::kHi, kLoZone = Num<DT>::kLo;
   constexpr u32 kRingRows = kTileNG * kGroupRows;
   // own word and, for the panel's edge lanes, the halo word next to it (the other lanes read word 0 for nothing)
   const u32 halo_a = ring_s + (lane == 31 ? 33u * 16u : 0u);
@@ -330,10 +290,7 @@ __device__ __forceinline__ u32 dense_keep_mask_f32(int rows_here, u32 ring_s, u3
       for (int c = 0; c < 4; ++c) {
         const float x = comp(xc, c), hh = comp(h, c);
         bool keep = x > floorx;
-        if (keep && !pre && x != hh) {
-          const bool amb = (x >= hh - kNearTie) || (hh > kHiZone && x > kHiZone - 1.0f) || (hh < kLoZone);
-          keep = amb && Num<DT>::act(x) == Num<DT>::act(hh);  // rare
-        }
+        if (keep && !pre && x != hh) keep = may_tie<DT>(x, hh) && Num<DT>::act(x) == Num<DT>::act(hh);  // rare
         km |= (keep ? 1u : 0u) << (4 * i + c);
       }
     }
@@ -362,7 +319,7 @@ __device__ __forceinline__ bool settle_dense_f32(UnitState& st, int rows_here, u
   if (total > kBuf) return false;
   if (st.nbuf + total > kBuf) {
     __syncwarp();
-    flush_candidates<DT, !SDNET_X_EARLYHIST>(st, buf, hist, minx, sf, count_ptr, list, cap, K, lane, pre, xscale, satx);
+    flush_candidates<DT, false>(st, buf, hist, minx, sf, count_ptr, list, cap, K, lane, pre, xscale, satx);
   }
   int pos = st.nbuf + incl - cnt;
   const u32 centre0 = row0 + R;
@@ -374,9 +331,7 @@ __device__ __forceinline__ bool settle_dense_f32(UnitState& st, int rows_here, u
     if (rr >= kRingRows) rr -= kRingRows;
     const float x = TileMax<DT>::elem(ring_own + rr * kTilePitchB + 4 * c);
     buf[pos++] = ((u64)__float_as_uint(x) << 32) | (idx0 + i * (u32)W + 4u * (u32)lane + c);
-#if SDNET_X_EARLYHIST
     atomicAdd(&sf.ghist[fine_bin(fminf(fmaxf(x * xscale, -satx), satx))], 1u);
-#endif
   }
   st.nbuf += total;
   return true;
@@ -420,15 +375,6 @@ __device__ __forceinline__ void tile_fix_edges(u32 slot_s, int x0, int W, int la
 // at pitch + x - 4 (a box has to start on a 16-byte boundary, measured: anything else is an illegal
 // instruction) -- and lands in its slot as rows 0, 2 | 1, 3 with the odd rows 8 bytes further right.
 // At the image edges such a box reads across the row boundary; tile_fix_edges repairs that after the wait.
-#if SDNET_X_TRACE  // diagnostics builds only (tools/xbuild.sh -DSDNET_X_TRACE=1): per-warp timeline of the last launch
-__device__ unsigned long long g_tile_trace[8192 * 4];  // [warp]: start, first tile landed, end (globaltimer ns), groups << 32 | units
-__device__ __forceinline__ unsigned long long trace_now() {
-  unsigned long long t;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-  return t;
-}
-#endif
-
 template <int R, int DT, int S>
 __global__ void __launch_bounds__(kTileWarps * 32, kTileMinCtas)
 sdnet_peaks_tile_kernel(const __grid_constant__ PeaksParams p, const __grid_constant__ CUtensorMap tm_anchor,
@@ -473,18 +419,11 @@ sdnet_peaks_tile_kernel(const __grid_constant__ PeaksParams p, const __grid_cons
   auto step_pos = [&](u32& slot, u32& par) {
     if (++slot == (u32)NG) { slot = 0; par ^= 1u; }
   };
-#if SDNET_X_TRACE
-  const unsigned long long tr_start = trace_now();
-  unsigned long long tr_first = 0, tr_groups = 0, tr_units = 0;
-#endif
   for (;;) {
     u32 unit = 0;
     if (lane == 0) unit = atomicAdd(p.sched, 1u);
     unit = __shfl_sync(0xffffffffu, unit, 0);
     if (unit >= (u32)p.units) break;
-#if SDNET_X_TRACE
-    ++tr_units;
-#endif
     // the unit's piece of the line of groups; it is walked one column segment at a time
     u32 pos, pos_end;
     if (unit < (u32)p.tier1_units) {
@@ -559,24 +498,17 @@ sdnet_peaks_tile_kernel(const __grid_constant__ PeaksParams p, const __grid_cons
     constexpr int poll_mask = 3;  // measured at 128-row strips: polling every group 0.179 ms, every 4th 0.136 ms, every 8th 0.146 ms
     u32 idx0 = (u32)(r_begin * W + panel * kPanel);  // flat index of the group's row 0, panel column 0
     wait_tile(cur_slot, cur_par);
-#if SDNET_X_TRACE
-    if (!tr_first) tr_first = trace_now();
-    tr_groups += (unsigned long long)groups_out;
-#endif
     for (int g = 0; g < groups_out; ++g, idx0 += (u32)(kGroupRows * W)) {
       // cur_* = the tile holding the group's first window row, nxt_* = the one after it
       u32 nxt_slot = cur_slot, nxt_par = cur_par;
       step_pos(nxt_slot, nxt_par);
       if (R == 2 || g + 1 < groups) wait_tile(nxt_slot, nxt_par);
-#if SDNET_X_WARMPOLL
       if (gfloor_seen <= 0 && g > 0) {
         // The plane has no floor that this warp knows of: every pixel it looks at goes through the slow path, so a
         // fresh look at the published floor is worth its latency (one L2 round trip) -- every group, applied at once.
         gfloor_seen = __ldcg(gfloor_ptr);
         st.floorx = fmaxf(st.floorx, shared_floor<DT>(gfloor_seen, xscale));
-      } else
-#endif
-      if ((g & poll_mask) == 0) {
+      } else if ((g & poll_mask) == 0) {
         // every 16 rows: apply the plane-wide floor fetched one period ago
         // and start the next fetch.  The load writes straight into the register it will be read
         // from a period later, so its latency is never waited for.
@@ -629,7 +561,7 @@ sdnet_peaks_tile_kernel(const __grid_constant__ PeaksParams p, const __grid_cons
         const int nhot = __popc(hot), rows_here = nrows - g * kGroupRows;
         const float floorx = st.floorx;
         bool settled = false;
-        if (DT == SDNET_DTYPE_F32 && S == 1 && kDenseLanes > 0 && nhot >= kDenseLanes)
+        if (DT == SDNET_DTYPE_F32 && S == 1 && nhot >= kDenseLanes)
           settled = settle_dense_f32<R>(st, rows_here, ring_s, ring_own, row0, floorx, idx0, W, pre, buf, hist, minx, sf, count_ptr,
                                         list, p.cap, K, lane, xscale, satx);
         if (!settled) {
@@ -646,12 +578,11 @@ sdnet_peaks_tile_kernel(const __grid_constant__ PeaksParams p, const __grid_cons
           settle_entries<R, DT, S>(st, work, nent, ring_s, row0, row_tab, floorx, idx0, W, pre, buf, hist, minx, sf, count_ptr, list,
                                    p.cap, K, lane, xscale, satx);
         }
-        // while the plane has no floor yet, publish early and often; later only in batches
-        // (candidates are counted in the plane-wide histogram when they are found, so a flush is no longer what
-        // publishes them: while the plane has no floor, flushing after every group only added its latency)
-        if (st.nbuf >= kFlushAt || (SDNET_X_EARLYFLUSH && st.nbuf > 0 && gfloor_seen <= 0)) {
+        // flush in batches: candidates are counted in the plane-wide histogram when they are found, so a flush is
+        // not what publishes them (flushing after every group while the plane has no floor only added its latency)
+        if (st.nbuf >= kFlushAt) {
           __syncwarp();
-          flush_candidates<DT, !SDNET_X_EARLYHIST>(st, buf, hist, minx, sf, count_ptr, list, p.cap, K, lane, pre, xscale, satx);
+          flush_candidates<DT, false>(st, buf, hist, minx, sf, count_ptr, list, p.cap, K, lane, pre, xscale, satx);
         }
       }
       // every lane's reads of the group's first tile are done (the votes above): refill its slot
@@ -668,19 +599,10 @@ sdnet_peaks_tile_kernel(const __grid_constant__ PeaksParams p, const __grid_cons
     for (int k = groups_out; k < groups; ++k) step_pos(cur_slot, cur_par);  // the halo tile below the last group
     if (st.nbuf) {
       __syncwarp();
-      flush_candidates<DT, !SDNET_X_EARLYHIST>(st, buf, hist, minx, sf, count_ptr, list, p.cap, K, lane, pre, xscale, satx);
+      flush_candidates<DT, false>(st, buf, hist, minx, sf, count_ptr, list, p.cap, K, lane, pre, xscale, satx);
     }
     }  // segments of the unit
   }
-#if SDNET_X_TRACE
-  if (lane == 0) {
-    const u32 w = blockIdx.x * kTileWarps + warp;
-    if (w < 8192) {
-      g_tile_trace[4 * w + 0] = tr_start; g_tile_trace[4 * w + 1] = tr_first; g_tile_trace[4 * w + 2] = trace_now();
-      g_tile_trace[4 * w + 3] = (tr_groups << 32) | tr_units;
-    }
-  }
-#endif
 }
 
 

@@ -21,16 +21,13 @@ namespace {
 constexpr int kStages = 8;             // ring depth (power of two); kStages - 1 - 2R rows stay in flight
 constexpr int kPitch = 136;            // floats per ring row
 constexpr int kPitchB = kPitch * 4;
+// (the last kStages * 8 bytes are unused; dropping them changes the launch's shared memory and wants its own timing)
 constexpr int kPeaksSmemPerWarp = kStages * kPitchB + kBins * 8 + kBuf * 8 + kStages * 8;
 constexpr int kPeaksSmem = kWarps * kPeaksSmemPerWarp;
 
 // Feeds one warp's ring in the fallback kernel: every lane copies its own four columns with
 // 4-byte cp.async (any alignment).  Ring sequence number q of a unit <-> image row row0 + q.
-template <bool kBulk>
-struct RowFeed;
-
-template <>
-struct RowFeed<false> {
+struct RowFeed {
   u32 ring_s, base;
   const char* gown;
   const char* ghalo;
@@ -38,7 +35,7 @@ struct RowFeed<false> {
   u32 s_own, s_halo, own_ok, halo_ok;
   int row0, H, q_last;
 
-  __device__ __forceinline__ void init(u32 ring, u32, int lane) {
+  __device__ __forceinline__ void init(u32 ring, int lane) {
     ring_s = ring; base = 0;
     s_own = ring + (4 + 4 * lane) * 4;
     s_halo = ring + (lane == 31 ? 4 + kPanelW : 2) * 4;
@@ -88,7 +85,7 @@ struct RowFeed<false> {
 // Feed for fp16 / bf16 maps: the ring stays fp32 (so everything downstream is shared with the
 // fp32 path); each lane loads its own four columns (and lanes 0 / 31 the two halo columns) with
 // plain 2-byte loads -- any alignment, any W -- converts, and stores to the ring three steps
-// later, so kDepth rows per warp are in flight in registers.  Same call pattern as RowFeed<false>:
+// later, so kDepth rows per warp are in flight in registers.  Same call pattern as RowFeed:
 // issue(q) makes row q - kDepth resident, which is exactly the row step q - 7 needs.
 template <int DT>
 struct RowFeedCvt {
@@ -103,7 +100,7 @@ struct RowFeedCvt {
   float4 own[kDepth];
   float2 halo[kDepth];
 
-  __device__ __forceinline__ void init(u32 ring, u32, int lane) {
+  __device__ __forceinline__ void init(u32 ring, int lane) {
     ring_s = ring;
     s_own = ring + (4 + 4 * lane) * 4;
     s_halo = ring + (lane == 31 ? 4 + kPanelW : 2) * 4;
@@ -168,7 +165,7 @@ struct RowFeedCvt {
 template <int DT>
 struct FeedFor { typedef RowFeedCvt<DT> type; };
 template <>
-struct FeedFor<SDNET_DTYPE_F32> { typedef RowFeed<false> type; };
+struct FeedFor<SDNET_DTYPE_F32> { typedef RowFeed type; };
 
 // Which of a lane's four pixels survive NMS, given their window maxima h0..h3 (logit space).
 //   x == h            -> certainly survives;
@@ -176,15 +173,11 @@ struct FeedFor<SDNET_DTYPE_F32> { typedef RowFeed<false> type; };
 // Columns outside the image hold -inf and never pass x > floorx.
 template <int R, int DT = SDNET_DTYPE_F32>
 __device__ __forceinline__ u32 classify_row(const float4 ctr, float h0, float h1, float h2, float h3, float floorx) {
-  constexpr float kNearTie = Num<DT>::kNear, kHiZone = Num<DT>::kHi, kLoZone = Num<DT>::kLo;
-  constexpr float kNearTie2 = Num<DT>::kNear2, kHiZone2 = Num<DT>::kHi2;
   u32 cmask = 0, amb = 0;
 #define SDNET_CLASSIFY(x, h, j)                                                                        \
   if ((x) > floorx) {                                                                                  \
     if ((x) == (h)) cmask |= 1u << j;                                                                  \
-    else if (((x) >= (h) - kNearTie) || ((h) > kHiZone && (x) >= (h) - kNearTie2) ||                    \
-             ((h) > kHiZone2 && (x) > kHiZone2 - 1.0f) || ((h) < kLoZone))                              \
-      amb |= 1u << j;                                                                                  \
+    else if (may_tie<DT>((x), (h))) amb |= 1u << j;                                                    \
   }
   SDNET_CLASSIFY(ctr.x, h0, 0)
   SDNET_CLASSIFY(ctr.y, h1, 1)
@@ -246,7 +239,7 @@ __device__ __forceinline__ void append_row(UnitState& st, u32 cmask, const float
   }
 }
 
-template <bool kAligned, int R, int DT>
+template <int R, int DT>
 __global__ void __launch_bounds__(kThreads, DT == SDNET_DTYPE_F32 ? 4 : 3)
 sdnet_peaks_kernel(const __grid_constant__ PeaksParams p) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -257,7 +250,6 @@ sdnet_peaks_kernel(const __grid_constant__ PeaksParams p) {
   u32* hist = reinterpret_cast<u32*>(wbase + kStages * kPitchB);
   int* minx = reinterpret_cast<int*>(hist + kBins);
   u64* buf = reinterpret_cast<u64*>(minx + kBins);
-  const u32 bars_s = smem_u32(buf + kBuf);
   const bool pre = p.pre_activated != 0;
   const float xscale = pre ? kPreScale : 1.0f;
   const float satx = pre ? CUDART_INF_F : kSatX;
@@ -266,7 +258,7 @@ sdnet_peaks_kernel(const __grid_constant__ PeaksParams p) {
   const u32 own_off = (4 + 4 * lane) * 4;                      // this lane's four columns inside a ring row
   const u32 halo_off = (lane == 31 ? 4 + kPanelW : 2) * 4;     // the two columns beyond the panel edge
   typename FeedFor<DT>::type feed;
-  feed.init(ring_s, bars_s, lane);
+  feed.init(ring_s, lane);
 
   for (;;) {
     u32 unit = 0;

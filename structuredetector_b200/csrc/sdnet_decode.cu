@@ -191,12 +191,7 @@ TileKernel tile_kernel_for(int radius, int dtype, int S) {
 
 // Which peaks kernel a decode of these tensors runs (SDNET_PATH_*), encoding the tensor maps on the way.
 int select_peaks_path(const SdnetDecodeParams* p, CUtensorMap* tm_anchor, CUtensorMap* tm_part, int* tile_s_out) {
-  static const int path_override = [] {  // tuning knob, read once: SDNET_PEAKS_PATH = tile | warp
-    const char* e = getenv("SDNET_PEAKS_PATH");
-    if (!e) return 0;
-    return e[0] == 't' ? 1 : (e[0] == 'w' ? 3 : 0);
-  }();
-  if ((p->flags & SDNET_FLAG_WARP_KERNEL) || path_override == 3) return SDNET_PATH_WARP;
+  if (p->flags & SDNET_FLAG_WARP_KERNEL) return SDNET_PATH_WARP;
   int tile_s = tile_rows_per_tma_row(p->anchor_hm, p->dtype, p->H, p->W, p->radius);
   if (tile_s != tile_rows_per_tma_row(p->part_hm, p->dtype, p->H, p->W, p->radius) ||
       (tile_s == 2 && p->anchor_hm.stride_h != p->part_hm.stride_h))
@@ -269,7 +264,7 @@ struct PeaksPlan {
 };
 
 // Cut the line of columns x groups (pp.panels, pp.H set) into units for `resident` warps: see plan_peaks.
-bool plan_tile_line(PeaksParams& pp, long long planes, long long resident, int chunk_override, int* ctas, long long max_ctas) {
+bool plan_tile_line(PeaksParams& pp, long long planes, long long resident, int* ctas, long long max_ctas) {
   const long long G = (pp.H + kGroupRows - 1) / kGroupRows;
   const long long columns = planes * pp.panels;
   if (columns * G >= (1ll << 31)) return false;
@@ -277,7 +272,6 @@ bool plan_tile_line(PeaksParams& pp, long long planes, long long resident, int c
   const long long rest = (columns - tier1) * G;
   long long chunk = (rest + resident - 1) / resident;
   if (chunk < kMinChunkGroups) chunk = kMinChunkGroups;
-  if (chunk_override > 0) chunk = chunk_override;
   if (chunk > G) chunk = G;
   pp.tier1_units = (int)tier1;
   pp.groups_per_col = (int)G;
@@ -312,11 +306,6 @@ cudaError_t plan_peaks(const SdnetDecodeParams* p, PeaksParams& pp, PeaksPlan& p
     cudaError_t err = cudaSuccess;
     pl.ctas_per_sm = tile_ctas_per_sm(pl.tile_kern, p->dtype, pl.tile_s, p->radius, pl.smem, &err);
     if (pl.ctas_per_sm <= 0) return err != cudaSuccess ? err : cudaErrorUnknown;
-    static const int occ_cap = [] {  // tuning knob, read once: SDNET_PEAKS_OCC = resident CTAs per SM one launch may take
-      const char* e = getenv("SDNET_PEAKS_OCC");
-      return e ? atoi(e) : 0;
-    }();
-    if (occ_cap > 0 && occ_cap < pl.ctas_per_sm) pl.ctas_per_sm = occ_cap;
     pp.panels = (p->W + panel_cols - 1) / panel_cols;
     // The work is a line of `columns` x G groups of four rows (a column = one panel of one plane, top to
     // bottom), cut into units handed out in order by an atomic counter.  Long units prune best (a unit
@@ -325,13 +314,8 @@ cudaError_t plan_peaks(const SdnetDecodeParams* p, PeaksParams& pp, PeaksPlan& p
     //   tier 2: what is left of the line cut into equal chunks, one per resident warp (a chunk may run
     //           over the end of a column into the next one), so the last wave ends everywhere at once.
     // With fewer columns than resident warps (small shards) everything is tier 2: one balanced wave.
-    static const int chunk_override = [] {  // tuning knob, read once: SDNET_CHUNK_GROUPS = n
-      const char* e = getenv("SDNET_CHUNK_GROUPS");
-      return e ? atoi(e) : 0;
-    }();
     pp.H = p->H;
-    if (!plan_tile_line(pp, planes, (long long)pl.sms * pl.ctas_per_sm * kTileWarps, chunk_override, &pl.ctas,
-                        (long long)pl.sms * pl.ctas_per_sm))
+    if (!plan_tile_line(pp, planes, (long long)pl.sms * pl.ctas_per_sm * kTileWarps, &pl.ctas, (long long)pl.sms * pl.ctas_per_sm))
       return cudaErrorInvalidValue;
   } else {
     pl.tile_kern = nullptr;
@@ -388,14 +372,14 @@ int launch_decode(const SdnetDecodeParams* p, cudaStream_t stream, cudaEvent_t* 
     dim3 grid((unsigned)pl.ctas), block(kThreads);
     const bool r2 = p->radius == 2;
     if (p->dtype == SDNET_DTYPE_F16) {
-      err = r2 ? launch_peaks(sdnet_peaks_kernel<false, 2, SDNET_DTYPE_F16>, grid, block, stream, pp)
-               : launch_peaks(sdnet_peaks_kernel<false, 1, SDNET_DTYPE_F16>, grid, block, stream, pp);
+      err = r2 ? launch_peaks(sdnet_peaks_kernel<2, SDNET_DTYPE_F16>, grid, block, stream, pp)
+               : launch_peaks(sdnet_peaks_kernel<1, SDNET_DTYPE_F16>, grid, block, stream, pp);
     } else if (p->dtype == SDNET_DTYPE_BF16) {
-      err = r2 ? launch_peaks(sdnet_peaks_kernel<false, 2, SDNET_DTYPE_BF16>, grid, block, stream, pp)
-               : launch_peaks(sdnet_peaks_kernel<false, 1, SDNET_DTYPE_BF16>, grid, block, stream, pp);
+      err = r2 ? launch_peaks(sdnet_peaks_kernel<2, SDNET_DTYPE_BF16>, grid, block, stream, pp)
+               : launch_peaks(sdnet_peaks_kernel<1, SDNET_DTYPE_BF16>, grid, block, stream, pp);
     } else {
-      err = r2 ? launch_peaks(sdnet_peaks_kernel<false, 2, SDNET_DTYPE_F32>, grid, block, stream, pp)
-               : launch_peaks(sdnet_peaks_kernel<false, 1, SDNET_DTYPE_F32>, grid, block, stream, pp);
+      err = r2 ? launch_peaks(sdnet_peaks_kernel<2, SDNET_DTYPE_F32>, grid, block, stream, pp)
+               : launch_peaks(sdnet_peaks_kernel<1, SDNET_DTYPE_F32>, grid, block, stream, pp);
     }
     if (err != cudaSuccess) return (int)err;
   }
@@ -567,13 +551,6 @@ int sdnet_decode_peaks_path(const SdnetDecodeParams* params) {
   return select_peaks_path(params, &a, &b, &tile_s);
 }
 
-#if SDNET_X_TRACE
-// diagnostics builds only: copy out the per-warp timeline of the last fp32 tile-kernel launch (4 u64 per warp)
-int sdnet_debug_trace(unsigned long long* out, int n_warps) {
-  return (int)cudaMemcpyFromSymbol(out, g_tile_trace, sizeof(unsigned long long) * 4 * (size_t)n_warps);
-}
-#endif
-
 int sdnet_decode_schedule(const SdnetDecodeParams* params, SdnetSchedule* out) {
   const int rc = validate(params);
   if (rc != 0) return rc;
@@ -654,10 +631,9 @@ int sdnet_suppress_into_launch(const SdnetTensor4* in, int dtype, int B, int C, 
   if (in->stride_w != 1) return SDNET_E_STRIDE;
   if (dtype != SDNET_DTYPE_F32 && dtype != SDNET_DTYPE_F16 && dtype != SDNET_DTYPE_BF16) return SDNET_E_DTYPE;
   if (radius != 1 && radius != 2) return SDNET_E_RADIUS;
-  static const bool no_tile = [] { const char* e = getenv("SDNET_SUPPRESS_PATH"); return e && e[0] == 'w'; }();  // tuning knob
   // fp32 maps that TMA can describe (and a 16-byte-aligned output): the tile kernel
   CUtensorMap tm;
-  if (!no_tile && dtype == SDNET_DTYPE_F32 &&
+  if (dtype == SDNET_DTYPE_F32 &&
       (((uintptr_t)out_t->data | (uintptr_t)(out_t->stride_b * 4) | (uintptr_t)(out_t->stride_c * 4) | (uintptr_t)(out_t->stride_h * 4)) & 15) == 0 && (long long)B * C * ((W + kPanelW - 1) / kPanelW) * ((H + 3) / 4) < (1ll << 31) &&
       tile_rows_per_tma_row(*in, dtype, H, W, radius) == 1 && make_tile_map(&tm, *in, dtype, B, C, H, W, 1)) {
     PeaksParams pp = {};
@@ -674,7 +650,7 @@ int sdnet_suppress_into_launch(const SdnetTensor4* in, int dtype, int B, int C, 
     if (per_sm < 1) per_sm = 1;
     const int sms = device_sm_count();
     int ctas = 0;
-    plan_tile_line(pp, (long long)B * C, (long long)sms * per_sm * kTileWarps, 0, &ctas, sms * per_sm);
+    plan_tile_line(pp, (long long)B * C, (long long)sms * per_sm * kTileWarps, &ctas, sms * per_sm);
     kern<<<dim3((unsigned)ctas), dim3(kTileWarps * 32), kSupTileSmem, static_cast<cudaStream_t>(stream)>>>(pp, tm, outv);
     return (int)cudaGetLastError();
   }

@@ -30,10 +30,8 @@ __device__ __forceinline__ float4 sup_load4(const void* base, long long row_off,
 
 template <int DT>
 __device__ __forceinline__ float sup_score(float x, float h) {
-  constexpr float kNearTie = Num<DT>::kNear, kHiZone = Num<DT>::kHi, kLoZone = Num<DT>::kLo, kNearTie2 = Num<DT>::kNear2,
-                  kHiZone2 = Num<DT>::kHi2;
   if (x == h) return Num<DT>::act(x);
-  if ((x >= h - kNearTie) || (h > kHiZone && x >= h - kNearTie2) || (h > kHiZone2 && x > kHiZone2 - 1.0f) || (h < kLoZone)) {
+  if (may_tie<DT>(x, h)) {
     const float sx = Num<DT>::act(x);
     if (sx == Num<DT>::act(h)) return sx;
   }

@@ -11,6 +11,4 @@ for (h, w, k) in ((40, 132, 30), (37, 53, 20), (24, 1028, 40)):
         for kw in ({}, {"warp_kernel": True}, {"exact_select": True}, {"radius": 1}):
             pk = ops.decode_packed(outs, k, k, 0.4, 0.1, **kw)
         torch.cuda.synchronize()
-import os
-os.environ["SDNET_PEAKS_PATH"] = "tile"
 print("ok", int(pk.counts.sum()))

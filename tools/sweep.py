@@ -1,8 +1,8 @@
 """Time several builds of the decode library side by side in ONE process (kernel experiments).
 
-    python tools/sweep.py [--images 1024,128] [--modes noise,blobs] [--dtype f32] [--reps 20] name[=ENV=VAL,...] ...
+    python tools/sweep.py [--images 1024,128] [--modes noise,blobs] [--dtype f32] [--reps 20] name ...
 
-``name`` = ``base`` (the product library) or a build made by ``tools/xbuild.sh <name> -D...``
+``name`` = ``base`` (the product library) or a build made by ``tools/xbuild.sh <name>``
 (``structuredetector_b200/csrc/exp/lib_<name>.so``).  For every (build, images, mode): the per-kernel
 device times of ``sdnet_decode_launch_timed`` (mean of --reps), the peaks kernel's fraction of the
 measured copy peak, candidates per plane, and whether the packed result equals the base build's
@@ -42,30 +42,11 @@ def main():
     M, N, H, W, K, P = cfg.labels, cfg.parts, cfg.height, cfg.width, cfg.max_objects, cfg.max_parts
     conf = float(torch.tensor(cfg.conf_threshold, dtype=tdtype))
     dist = float(torch.tensor(cfg.dist_thresh * min(W, H), dtype=torch.float32))
-    import os
-    import shutil
-    import tempfile
 
     libs = {}
-    tmpdir = tempfile.mkdtemp()
-    for spec in args.names:  # name[@ENV=VAL[,ENV=VAL...]]: the library's read-once tuning knobs come from the environment
-        name, _, envs = spec.partition("@")
+    for name in args.names:
         path = _native.LIB_PATH if name == "base" else ROOT / "structuredetector_b200" / "csrc" / "exp" / f"lib_{name}.so"
-        env = dict(kv.split("=") for kv in envs.split(",")) if envs else {}
-        if env:  # a private copy, so that dlopen gives this spec its own statics
-            copy = Path(tmpdir) / f"lib_{spec.replace('@', '_').replace('=', '_').replace(',', '_')}.so"
-            shutil.copy(path, copy)
-            path = copy
-        os.environ.update(env)
-        lib = _native.load_from(path)
-        # one tiny decode now: the knobs are read at the library's first launch
-        tiny = torch.zeros(1, 7, 32, 32, device=dev)
-        to = split_outputs(tiny, 2, 1)
-        ops.DecodePlan(dev, 1, 2, 1, 32, 32, 10, 10, lib=lib).run(to["anchor_hm"], to["part_hm"], to["offsets"], to["embeddings"], 0.4, 3.2)
-        torch.cuda.synchronize()
-        for k in env:
-            del os.environ[k]
-        libs[spec] = lib
+        libs[name] = _native.load_from(path)
     results = []
     for mode in args.modes.split(","):
         uniq = make_raw(cfg, mode, batch=32).to(dev)

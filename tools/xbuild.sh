@@ -1,7 +1,7 @@
 #!/bin/bash
-# Build a macro variant of the decode library for kernel experiments:
-#   bash tools/xbuild.sh <name> -DSDNET_X_WAIT=1 ...   ->  structuredetector_b200/csrc/exp/lib_<name>.so
-# and run with SDNET_DECODE_LIB=structuredetector_b200/csrc/exp/lib_<name>.so
+# Build the working tree's decode library under another name for kernel experiments (A/B runs against base):
+#   bash tools/xbuild.sh <name> [extra nvcc flags, e.g. -Xptxas -v]   ->  structuredetector_b200/csrc/exp/lib_<name>.so
+# and run with SDNET_DECODE_LIB=structuredetector_b200/csrc/exp/lib_<name>.so, or time it with tools/sweep.py base <name>
 name=$1; shift
 mkdir -p structuredetector_b200/csrc/exp
 nvcc -gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 -prec-div=true -prec-sqrt=true -ftz=false \
