@@ -38,10 +38,17 @@ def test_saturated_plateaus_survive(cuda_device):
     assert torch.equal(got, _reference_maps(hm)) and int((got > 0).sum()) == 20 * 24
 
 
-@pytest.mark.parametrize("name,mode", [("cfg1", "blobs"), ("cfg1", "ladder"), ("cfg3", "blobs")])
-def test_raw_decoder_feeds_coreml_decoder(cuda_device, name, mode):
+@pytest.mark.parametrize("name,mode,batch,dtype", [
+    pytest.param("cfg1", "blobs", 2, torch.float32, id="cfg1-blobs"),
+    pytest.param("cfg1", "ladder", 2, torch.float32, id="cfg1-ladder"),
+    pytest.param("cfg3", "blobs", 2, torch.float32, id="cfg3-blobs"),
+    # the benchmarked geometry: 960 tile-kernel columns (fp32), 8 strips x 5 panels per plane (fp16)
+    pytest.param("cfg5", "blobs", 64, torch.float32, id="cfg5-blobs-64-float32"),
+    pytest.param("cfg5", "blobs", 64, torch.float16, id="cfg5-blobs-64-float16"),
+])
+def test_raw_decoder_feeds_coreml_decoder(cuda_device, name, mode, batch, dtype):
     cfg = CONFIGS[name]
-    raw = make_raw(cfg, mode, batch=2).to(cuda_device)
+    raw = make_raw(cfg, mode, batch=batch).to(dtype).to(cuda_device)
     args = make_args(cfg)
     baked = RawDecoder(cfg.labels + cfg.parts)(raw)
     assert baked.shape == raw.shape and torch.equal(baked[:, cfg.labels + cfg.parts:], raw[:, cfg.labels + cfg.parts:])
