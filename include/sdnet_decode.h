@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define SDNET_ABI_VERSION 10
+#define SDNET_ABI_VERSION 11
 
 /* element types of the four input tensors */
 #define SDNET_DTYPE_F32 0
@@ -54,6 +54,7 @@ extern "C" {
 #define SDNET_E_WORKSPACE -5 /* workspace missing, misaligned (256 B) or smaller than sdnet_decode_workspace_bytes */
 #define SDNET_E_RADIUS -6    /* NMS window radius other than 2 (5x5, utils.py:442) or 1 (3x3) */
 #define SDNET_E_STRUCT -7    /* struct_size does not match this library's SdnetDecodeParams */
+#define SDNET_E_TABLE -8     /* a per-class threshold table (conf_class_f32, conf_class) is not aligned to its element type */
 
 #define SDNET_MAX_TOPK 1024
 #define SDNET_MAX_CHANNELS 255
@@ -112,6 +113,12 @@ typedef struct SdnetDecodeParams {
   uint32_t* done_flag;
   uint32_t done_value;
   uint32_t reserved1;
+  /* Per-class thresholds (optional, device memory): M + N floats, the M anchor classes first, then the N part kinds,
+   * each rounded to the heat maps' dtype as conf_f32 is.  A slot of class c is valid when score > conf_class_f32[c]
+   * (anchors) or score > conf_class_f32[M + c] (parts), instead of score > conf_f32; counts, the grouping's masks
+   * and nothing else depend on it.  NULL: every slot compares against conf_f32 (a zeroed field means what it meant
+   * under ABI version 10).  The table is read by the tail kernel; keep it alive until the decode has run. */
+  const float* conf_class_f32;
 } SdnetDecodeParams;
 
 /* Library / ABI identification. */
@@ -217,6 +224,11 @@ typedef struct SdnetMatchParams {
   int32_t* part_stats;         /* (B, N, 3) */
   double* anchor_acc;          /* (B, K): min_dist / min(img_size) of the true positives, NaN elsewhere (slot = score order) */
   double* part_acc;            /* (B, P) */
+  /* Per-class thresholds (optional, device memory): M + N doubles, the M anchor classes first, then the N part kinds.
+   * An anchor slot of class c < M is a detection when score > conf_class[c], a part slot of kind c < N when
+   * !(score < conf_class[M + c]).  The index is guarded, not the table sized: a slot whose class is >= M (kind >= N)
+   * -- a decode may emit any class up to SDNET_MAX_CHANNELS - 1 -- compares against conf.  NULL: conf for every slot. */
+  const double* conf_class;
 } SdnetMatchParams;
 
 int sdnet_match_launch(const SdnetMatchParams* params, void* stream);
@@ -250,6 +262,10 @@ typedef struct SdnetObjectMatchParams {
   int32_t* classif_stats;      /* (B, 20, 3): ndet, npos, tp for "bean_0".."bean_9", "maize_0".."maize_9" */
   double* classif_acc;         /* (B, K): distance / min(img_size) of the true positives, NaN elsewhere */
   int32_t* pred_parts;         /* (B, K): number of parts of each emitted object, -1 for slots not emitted */
+  /* Per-class thresholds (optional, device memory): as SdnetMatchParams.conf_class (M + N doubles; only the first M,
+   * the anchor classes, are read here): an object is emitted when its anchor has score > conf_class[class], with
+   * conf for a class >= M.  NULL: conf for every object. */
+  const double* conf_class;
 } SdnetObjectMatchParams;
 
 int sdnet_match_objects_launch(const SdnetObjectMatchParams* params, void* stream);

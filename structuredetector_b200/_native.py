@@ -13,7 +13,7 @@ import os as _os
 
 # SDNET_DECODE_LIB: load another build of the same library (kernel experiments, tools/xbuild.sh)
 LIB_PATH = Path(_os.environ.get("SDNET_DECODE_LIB") or Path(__file__).resolve().parent / "csrc" / "libsdnet_decode.so").resolve()
-ABI_VERSION = 10
+ABI_VERSION = 11
 DEST_PEER_STORES, DEST_MULTICAST = 0, 1  # SdnetDecodeParams.dest_mode
 
 FLAG_PRE_ACTIVATED = 1
@@ -96,6 +96,7 @@ class SdnetDecodeParams(ctypes.Structure):
         ("done_flag", ctypes.c_void_p),
         ("done_value", ctypes.c_uint32),
         ("reserved1", ctypes.c_uint32),
+        ("conf_class_f32", ctypes.c_void_p),
     ]
 
 
@@ -116,6 +117,7 @@ class SdnetMatchParams(ctypes.Structure):
         ("gt_parts", ctypes.c_void_p), ("n_gt_parts", ctypes.c_void_p),
         ("anchor_stats", ctypes.c_void_p), ("part_stats", ctypes.c_void_p),
         ("anchor_acc", ctypes.c_void_p), ("part_acc", ctypes.c_void_p),
+        ("conf_class", ctypes.c_void_p),
     ]
 
 
@@ -132,6 +134,7 @@ class SdnetObjectMatchParams(ctypes.Structure):
         ("cls_group", ctypes.c_void_p),
         ("csi_stats", ctypes.c_void_p), ("csi_acc", ctypes.c_void_p),
         ("classif_stats", ctypes.c_void_p), ("classif_acc", ctypes.c_void_p), ("pred_parts", ctypes.c_void_p),
+        ("conf_class", ctypes.c_void_p),
     ]
 
 

@@ -10,7 +10,8 @@
  * offsets (no __init__ call, no attribute protocol): ~0.1 us per object instead of ~0.4 us.  The arithmetic
  * is the reference's: coordinates are float32 values widened to double and multiplied by in/out in double
  * (utils.py:19-26 via decoders.py:139), `score > conf` for objects and `not score < conf` for raw parts in
- * double (decoders.py:116,153).
+ * double (decoders.py:116,153).  `conf` is one threshold, or a sequence of thresholds indexed by the slot's class
+ * (anchor classes for assemble / json_text, part kinds for keypoints).
  *
  * Host-only C (gcc); built by structuredetector_b200/build.py next to the CUDA library.
  */
@@ -72,6 +73,46 @@ typedef struct {
   Py_buffer anchor, part, assign;
 } Views;
 
+/* The threshold of a slot: one number for every class, or one per class index.  A class index the table does not
+ * cover compares against -inf, so the slot is always kept and name_at reports the missing name. */
+typedef struct {
+  double scalar;
+  double* table; /* NULL: scalar for every class */
+  Py_ssize_t n;
+} Conf;
+
+static int conf_parse(PyObject* obj, Conf* c) {
+  c->table = NULL;
+  c->n = 0;
+  c->scalar = 0.0;
+  if (!PySequence_Check(obj)) {
+    c->scalar = PyFloat_AsDouble(obj);
+    return (c->scalar == -1.0 && PyErr_Occurred()) ? -1 : 0;
+  }
+  PyObject* seq = PySequence_Fast(obj, "conf must be a number or a sequence of per-class thresholds");
+  if (!seq) return -1;
+  c->n = PySequence_Fast_GET_SIZE(seq);
+  c->table = (double*)PyMem_Malloc((size_t)(c->n > 0 ? c->n : 1) * sizeof(double));
+  if (!c->table) { Py_DECREF(seq); PyErr_NoMemory(); return -1; }
+  for (Py_ssize_t i = 0; i < c->n; ++i) {
+    c->table[i] = PyFloat_AsDouble(PySequence_Fast_GET_ITEM(seq, i));
+    if (c->table[i] == -1.0 && PyErr_Occurred()) { Py_DECREF(seq); PyMem_Free(c->table); c->table = NULL; return -1; }
+  }
+  Py_DECREF(seq);
+  return 0;
+}
+
+static void conf_release(Conf* c) {
+  if (c->table) PyMem_Free(c->table);
+  c->table = NULL;
+}
+
+static inline double conf_of(const Conf* c, float cls) {
+  if (!c->table) return c->scalar;
+  const long idx = (long)cls;
+  return (idx >= 0 && idx < c->n) ? c->table[idx] : -1.0 / 0.0;
+}
+
 static void views_release(Views* v) {
   if (v->anchor.obj) PyBuffer_Release(&v->anchor);
   if (v->part.obj) PyBuffer_Release(&v->part);
@@ -92,18 +133,20 @@ static PyObject* name_at(PyObject* names, long idx) {
 }
 
 /* assemble(anchor_out, part_out, assign, B, K, P, conf, sx, sy, labels, kinds, anchor_name, Keypoint, Object, ImageAnnotation)
- *   -> list[ImageAnnotation]       (decoders.py:103-139) */
+ *   -> list[ImageAnnotation]       (decoders.py:103-139); conf: a number or one threshold per anchor class */
 static PyObject* assemble(PyObject* self, PyObject* args) {
-  PyObject *a_obj, *p_obj, *s_obj, *labels, *kinds, *anchor_name, *kp_type, *obj_type, *ann_type;
+  PyObject *a_obj, *p_obj, *s_obj, *c_obj, *labels, *kinds, *anchor_name, *kp_type, *obj_type, *ann_type;
   Py_ssize_t B, K, P;
-  double conf, sx, sy;
-  if (!PyArg_ParseTuple(args, "OOOnnndddO!O!UOOO", &a_obj, &p_obj, &s_obj, &B, &K, &P, &conf, &sx, &sy, &PyList_Type, &labels,
+  double sx, sy;
+  if (!PyArg_ParseTuple(args, "OOOnnnOddO!O!UOOO", &a_obj, &p_obj, &s_obj, &B, &K, &P, &c_obj, &sx, &sy, &PyList_Type, &labels,
                         &PyList_Type, &kinds, &anchor_name, &kp_type, &obj_type, &ann_type))
     return NULL;
   static const char* const kp_names[] = {"kind", "x", "y", "score"};
   static const char* const ob_names[] = {"name", "anchor", "parts", "box"};
   SlotClass kc, oc;
   if (slot_class_init(&kc, kp_type, kp_names, 4) < 0 || slot_class_init(&oc, obj_type, ob_names, 4) < 0) return NULL;
+  Conf conf;
+  if (conf_parse(c_obj, &conf) < 0) return NULL;
   Views v = {{0}, {0}, {0}};
   PyObject* result = NULL;
   PyObject** buckets = NULL;
@@ -132,16 +175,16 @@ static PyObject* assemble(PyObject* self, PyObject* args) {
     Py_ssize_t n_objects = 0;
     for (Py_ssize_t k = 0; k < K; ++k) {
       fill[k] = fill[K + k] = 0;
-      n_objects += (double)a[k * 4 + 2] > conf; /* decoders.py:116: score <= conf_thresh -> skip */
+      n_objects += (double)a[k * 4 + 2] > conf_of(&conf, a[k * 4 + 3]); /* decoders.py:116: score <= conf_thresh -> skip */
     }
     for (Py_ssize_t i = 0; i < P; ++i) {
       const int32_t slot = s[i];
       /* grouped onto an anchor that is not emitted (score == float32(conf) > conf): dropped, as in the reference */
-      if (slot >= 0 && slot < K && (double)a[slot * 4 + 2] > conf) ++fill[slot];
+      if (slot >= 0 && slot < K && (double)a[slot * 4 + 2] > conf_of(&conf, a[slot * 4 + 3])) ++fill[slot];
     }
     for (Py_ssize_t i = 0; i < P && !failed; ++i) {
       const int32_t slot = s[i];
-      if (slot < 0 || slot >= K || !((double)a[slot * 4 + 2] > conf)) continue;
+      if (slot < 0 || slot >= K || !((double)a[slot * 4 + 2] > conf_of(&conf, a[slot * 4 + 3]))) continue;
       PyObject* kind = name_at(kinds, (long)p[i * 6 + 3]);
       PyObject* kp = kind ? new_keypoint(&kc, kind, (double)p[i * 6] * sx, (double)p[i * 6 + 1] * sy, (double)p[i * 6 + 2]) : NULL;
       if (!kp) { failed = 1; break; }
@@ -156,7 +199,7 @@ static PyObject* assemble(PyObject* self, PyObject* args) {
     if (!objects) failed = 1;
     Py_ssize_t n_out = 0;
     for (Py_ssize_t k = 0; k < K && !failed; ++k) {
-      if (!((double)a[k * 4 + 2] > conf)) continue;
+      if (!((double)a[k * 4 + 2] > conf_of(&conf, a[k * 4 + 3]))) continue;
       PyObject* label = name_at(labels, (long)a[k * 4 + 3]);
       PyObject* anchor = label ? new_keypoint(&kc, anchor_name, (double)a[k * 4] * sx, (double)a[k * 4 + 1] * sy, (double)a[k * 4 + 2]) : NULL;
       PyObject* parts = buckets[k] ? buckets[k] : (anchor ? PyList_New(0) : NULL);
@@ -190,22 +233,25 @@ done:
   if (buckets) PyMem_Free(buckets);
   if (fill) PyMem_Free(fill);
   views_release(&v);
+  conf_release(&conf);
   return result;
 }
 
 /* keypoints(rows, B, n, width, conf, sx, sy, names, Keypoint) -> list[list[Keypoint]]
- * Every slot of a (B, n, width) float32 array (x, y, score, class, ...) whose score is not below conf, in slot
- * order: raw_parts of Decoder (decoders.py:142-159; double arithmetic). */
+ * Every slot of a (B, n, width) float32 array (x, y, score, class, ...) whose score is not below conf (a number or one
+ * threshold per class), in slot order: raw_parts of Decoder (decoders.py:142-159; double arithmetic). */
 static PyObject* keypoints(PyObject* self, PyObject* args) {
-  PyObject *r_obj, *names, *kp_type;
+  PyObject *r_obj, *c_obj, *names, *kp_type;
   Py_ssize_t B, n, width;
-  double conf, sx, sy;
-  if (!PyArg_ParseTuple(args, "OnnndddO!O", &r_obj, &B, &n, &width, &conf, &sx, &sy, &PyList_Type, &names, &kp_type)) return NULL;
+  double sx, sy;
+  if (!PyArg_ParseTuple(args, "OnnnOddO!O", &r_obj, &B, &n, &width, &c_obj, &sx, &sy, &PyList_Type, &names, &kp_type)) return NULL;
   static const char* const kp_names[] = {"kind", "x", "y", "score"};
   SlotClass kc;
   if (slot_class_init(&kc, kp_type, kp_names, 4) < 0) return NULL;
+  Conf conf;
+  if (conf_parse(c_obj, &conf) < 0) return NULL;
   Py_buffer rows;
-  if (PyObject_GetBuffer(r_obj, &rows, PyBUF_SIMPLE) < 0) return NULL;
+  if (PyObject_GetBuffer(r_obj, &rows, PyBUF_SIMPLE) < 0) { conf_release(&conf); return NULL; }
   PyObject* result = NULL;
   if (B < 0 || n <= 0 || width < 4 || rows.len < B * n * width * 4) {
     PyErr_SetString(PyExc_ValueError, "packed buffer is smaller than (B, n, width)");
@@ -220,7 +266,7 @@ static PyObject* keypoints(PyObject* self, PyObject* args) {
     PyList_SET_ITEM(result, b, out);
     for (Py_ssize_t i = 0; i < n; ++i) {
       const float* r = R + (b * n + i) * width;
-      if ((double)r[2] < conf) continue; /* decoders.py:153 */
+      if ((double)r[2] < conf_of(&conf, r[3])) continue; /* decoders.py:153 */
       PyObject* kind = name_at(names, (long)r[3]);
       PyObject* kp = kind ? new_keypoint(&kc, kind, (double)r[0] * sx, (double)r[1] * sy, (double)r[2]) : NULL;
       if (!kp || PyList_Append(out, kp) < 0) { Py_XDECREF(kp); Py_CLEAR(result); goto done; }
@@ -229,6 +275,7 @@ static PyObject* keypoints(PyObject* self, PyObject* args) {
   }
 done:
   PyBuffer_Release(&rows);
+  conf_release(&conf);
   return result;
 }
 
@@ -288,16 +335,18 @@ static int put_keypoint(Buf* b, PyObject* kind_json, double x, double y, double 
 }
 
 static PyObject* json_text(PyObject* self, PyObject* args) {
-  PyObject *a_obj, *p_obj, *s_obj, *resize, *labels, *kinds, *anchor_json, *paths, *sizes;
+  PyObject *a_obj, *p_obj, *s_obj, *c_obj, *resize, *labels, *kinds, *anchor_json, *paths, *sizes;
   Py_ssize_t B, K, P;
-  double conf, sx, sy;
-  if (!PyArg_ParseTuple(args, "OOOnnndddO!O!O!UO!O!", &a_obj, &p_obj, &s_obj, &B, &K, &P, &conf, &sx, &sy, &PyList_Type, &resize,
+  double sx, sy;
+  if (!PyArg_ParseTuple(args, "OOOnnnOddO!O!O!UO!O!", &a_obj, &p_obj, &s_obj, &B, &K, &P, &c_obj, &sx, &sy, &PyList_Type, &resize,
                         &PyList_Type, &labels, &PyList_Type, &kinds, &anchor_json, &PyList_Type, &paths, &PyList_Type, &sizes))
     return NULL;
   if (PyList_GET_SIZE(resize) != B || PyList_GET_SIZE(paths) != B || PyList_GET_SIZE(sizes) != B) {
     PyErr_SetString(PyExc_ValueError, "resize, paths and sizes need one entry per image");
     return NULL;
   }
+  Conf conf;
+  if (conf_parse(c_obj, &conf) < 0) return NULL;
   Views v = {{0}, {0}, {0}};
   PyObject* result = NULL;
   Buf buf = {NULL, 0, 0};
@@ -330,7 +379,7 @@ static PyObject* json_text(PyObject* self, PyObject* args) {
               PUT(&buf, ",\n  \"objects\": [") < 0;
     Py_ssize_t n_out = 0;
     for (Py_ssize_t k = 0; k < K && !bad; ++k) {
-      if (!((double)a[k * 4 + 2] > conf)) continue;
+      if (!((double)a[k * 4 + 2] > conf_of(&conf, a[k * 4 + 3]))) continue;
       PyObject* label = name_at(labels, (long)a[k * 4 + 3]);
       if (!label) { bad = 1; break; }
       bad = (n_out && PUT(&buf, ",") < 0) || PUT(&buf, "\n    {\n      \"label\": ") < 0 || buf_put_obj(&buf, label) < 0 ||
@@ -357,6 +406,7 @@ static PyObject* json_text(PyObject* self, PyObject* args) {
 done:
   if (buf.data) PyMem_Free(buf.data);
   views_release(&v);
+  conf_release(&conf);
   return result;
 }
 

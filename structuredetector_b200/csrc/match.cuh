@@ -13,8 +13,15 @@ namespace {
 // ---------------------------------------------------------------------------------------------
 constexpr int kMatchThreads = 256;
 
+// conf_class: n_classes per-class thresholds or nullptr; a slot whose class is outside [0, n_classes) compares against
+// conf (SdnetMatchParams.conf_class).
+__device__ __forceinline__ double class_conf(const double* __restrict__ conf_class, int n_classes, double conf, int cls) {
+  return (conf_class && cls >= 0 && cls < n_classes) ? conf_class[cls] : conf;
+}
+
 __device__ void match_pass(const float* __restrict__ out, int row_len, int slots, int n_classes, bool strict_gt,
-                           double conf, double sx, double sy, const double* __restrict__ scale,
+                           double conf, const double* __restrict__ conf_class, double sx, double sy,
+                           const double* __restrict__ scale,
                            const double* __restrict__ gt, int n_gt, int* __restrict__ stats_out,
                            double* __restrict__ acc_out, double* s_gx, double* s_gy, int* s_glab, int* s_winner,
                            int* s_jmin, double* s_dist, int* s_stats) {
@@ -32,8 +39,9 @@ __device__ void match_pass(const float* __restrict__ out, int row_len, int slots
   for (int i = threadIdx.x; i < slots; i += blockDim.x) {
     const float* row = out + (size_t)i * row_len;
     const double score = (double)row[2];
-    const bool det = strict_gt ? (score > conf) : !(score < conf);
     const int lab = (int)row[3];
+    const double c = class_conf(conf_class, n_classes, conf, lab);
+    const bool det = strict_gt ? (score > c) : !(score < c);
     int jmin = -1;
     double best = 1.7976931348623157e308;  // sys.float_info.max
     if (det) {
@@ -66,11 +74,12 @@ __global__ void __launch_bounds__(kMatchThreads) sdnet_match_kernel(const SdnetM
   __shared__ int s_glab[SDNET_MAX_GT], s_winner[SDNET_MAX_GT], s_jmin[SDNET_MAX_TOPK], s_stats[3 * SDNET_MAX_CHANNELS];
   const int b = blockIdx.x;
   const double* scale = p.image_scale + 4 * (size_t)b;
-  match_pass(p.anchor_out + (size_t)b * p.K * 4, 4, p.K, p.M, true, p.conf, p.sx, p.sy, scale,
+  match_pass(p.anchor_out + (size_t)b * p.K * 4, 4, p.K, p.M, true, p.conf, p.conf_class, p.sx, p.sy, scale,
              p.gt_anchors + (size_t)b * p.max_gt_anchors * 3, min(p.n_gt_anchors[b], p.max_gt_anchors),
              p.anchor_stats + (size_t)b * p.M * 3, p.anchor_acc + (size_t)b * p.K, s_gx, s_gy, s_glab, s_winner, s_jmin,
              s_dist, s_stats);
-  match_pass(p.part_out + (size_t)b * p.P * 6, 6, p.P, p.N, false, p.conf, p.sx, p.sy, scale,
+  match_pass(p.part_out + (size_t)b * p.P * 6, 6, p.P, p.N, false, p.conf, p.conf_class ? p.conf_class + p.M : nullptr,
+             p.sx, p.sy, scale,
              p.gt_parts + (size_t)b * p.max_gt_parts * 3, min(p.n_gt_parts[b], p.max_gt_parts),
              p.part_stats + (size_t)b * p.N * 3, p.part_acc + (size_t)b * p.P, s_gx, s_gy, s_glab, s_winner, s_jmin, s_dist,
              s_stats);
@@ -150,6 +159,8 @@ __device__ __forceinline__ void match_objects(const SdnetObjectMatchParams& p, i
   const double* G = p.gt_objects + (size_t)b * Go * 3;
   const double* Hh = p.gt_parts + (size_t)b * Gp * 3;
   const int* owner = p.gt_part_owner + (size_t)b * Gp;
+  // decoders.py:116 with the anchor's own threshold
+  auto emitted = [&](int k) { return (double)A[4 * k + 2] > class_conf(p.conf_class, p.M, p.conf, (int)A[4 * k + 3]); };
 
   // ---- stage everything in the evaluator's frame (annotation.resized / prediction.resized: evaluator.py:381-383)
   for (int j = tid; j < n_go; j += nt) {
@@ -171,7 +182,7 @@ __device__ __forceinline__ void match_objects(const SdnetObjectMatchParams& p, i
   for (int h = tid; h < n_gp; h += nt) atomicAdd(&s.gstart[owner[h] + 1], 1);
   for (int q = tid; q < P; q += nt) {
     const int k = asg[q];
-    if (k >= 0 && k < K && (double)A[4 * k + 2] > p.conf) atomicAdd(&s.npp[k], 1);
+    if (k >= 0 && k < K && emitted(k)) atomicAdd(&s.npp[k], 1);
   }
   __syncthreads();
   if (tid == 0) {  // prefix sums (at most ~1000 entries each)
@@ -183,7 +194,7 @@ __device__ __forceinline__ void match_objects(const SdnetObjectMatchParams& p, i
     for (int k = 0; k < K; ++k) s.npp[k] = 0;
     for (int q = 0; q < P; ++q) {
       const int k = asg[q];
-      if (k >= 0 && k < K && (double)A[4 * k + 2] > p.conf) s.plist[s.pstart[k] + s.npp[k]++] = q;
+      if (k >= 0 && k < K && emitted(k)) s.plist[s.pstart[k] + s.npp[k]++] = q;
     }
   }
   __syncthreads();
@@ -206,7 +217,7 @@ __device__ __forceinline__ void match_objects(const SdnetObjectMatchParams& p, i
     for (int k = tid; k < K; k += nt) {
       int jb = -1;
       double best = pass == 0 ? 1.7976931348623157e308 : 0.0;
-      const bool det = (double)A[4 * k + 2] > p.conf;
+      const bool det = emitted(k);
       const int key = det ? key_of((int)A[4 * k + 3], s.npp[k]) : -1;
       if (key >= 0) {
         atomicAdd(&s.stats[3 * key + 0], 1);  // ndet
@@ -239,7 +250,7 @@ __device__ __forceinline__ void match_objects(const SdnetObjectMatchParams& p, i
     int* stats_out = pass == 0 ? p.classif_stats + row * 60 : p.csi_stats + row * p.M * 3;
     for (int i = tid; i < 3 * n_lab; i += nt) stats_out[i] = s.stats[i];
     if (pass == 0)
-      for (int k = tid; k < K; k += nt) p.pred_parts[row * K + k] = (double)A[4 * k + 2] > p.conf ? s.npp[k] : -1;
+      for (int k = tid; k < K; k += nt) p.pred_parts[row * K + k] = emitted(k) ? s.npp[k] : -1;
     __syncthreads();
   }
 }

@@ -109,6 +109,7 @@ int validate(const SdnetDecodeParams* p) {
   const bool no_group = (p->flags & SDNET_FLAG_NO_GROUPING) != 0;
   if (!p->anchor_hm.data || !p->part_hm.data || !p->offsets.data || (!no_group && !p->embeddings.data)) return SDNET_E_NULL;
   if (!p->anchor_out || !p->part_out || !p->anchor_inds || !p->part_inds || !p->assign || !p->counts) return SDNET_E_NULL;
+  if ((uintptr_t)p->conf_class_f32 % alignof(float)) return SDNET_E_TABLE;
   if (p->anchor_hm.stride_w != 1 || p->part_hm.stride_w != 1 || p->offsets.stride_w != 1 ||
       (p->embeddings.data && p->embeddings.stride_w != 1))
     return SDNET_E_STRIDE;
@@ -418,6 +419,7 @@ int launch_decode(const SdnetDecodeParams* p, cudaStream_t stream, cudaEvent_t* 
   tp.pre_activated = pp.pre_activated;
   tp.no_grouping = (p->flags & SDNET_FLAG_NO_GROUPING) ? 1 : 0;
   tp.conf = p->conf_f32;
+  tp.conf_class = p->conf_class_f32;
   tp.dist_abs = p->dist_abs_f32;
   tp.lists = pp.lists;
   tp.counts = pp.counts;
@@ -466,6 +468,7 @@ const char* sdnet_error_string(int code) {
     case SDNET_E_WORKSPACE: return "workspace missing, misaligned or too small";
     case SDNET_E_RADIUS: return "unsupported NMS radius";
     case SDNET_E_STRUCT: return "SdnetDecodeParams.struct_size mismatch";
+    case SDNET_E_TABLE: return "per-class threshold table not aligned to its element type";
     default: return code > 0 ? cudaGetErrorString((cudaError_t)code) : "unknown error";
   }
 }
@@ -497,6 +500,7 @@ int sdnet_match_launch(const SdnetMatchParams* p, void* stream) {
       p->M + p->N > SDNET_MAX_CHANNELS || p->max_gt_anchors < 0 || p->max_gt_parts < 0 || p->max_gt_anchors > SDNET_MAX_GT ||
       p->max_gt_parts > SDNET_MAX_GT)
     return SDNET_E_SHAPE;
+  if ((uintptr_t)p->conf_class % alignof(double)) return SDNET_E_TABLE;
   sdnet_match_kernel<<<dim3((unsigned)p->B), dim3(kMatchThreads), 0, static_cast<cudaStream_t>(stream)>>>(*p);
   return (int)cudaGetLastError();
 }
@@ -512,6 +516,7 @@ int sdnet_match_objects_launch(const SdnetObjectMatchParams* p, void* stream) {
       p->M + p->N > SDNET_MAX_CHANNELS || p->max_gt_objects < 0 || p->max_gt_parts < 0 || p->max_gt_objects > SDNET_MAX_GT ||
       p->max_gt_parts > SDNET_MAX_GT)
     return SDNET_E_SHAPE;
+  if ((uintptr_t)p->conf_class % alignof(double)) return SDNET_E_TABLE;
   const size_t smem = match_objects_smem_bytes(p->max_gt_objects, p->max_gt_parts, p->K, p->P, p->M);
   cudaError_t err = cudaFuncSetAttribute(sdnet_match_objects_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (err != cudaSuccess) return (int)err;

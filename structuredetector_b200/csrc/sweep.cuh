@@ -92,10 +92,10 @@ __global__ void __launch_bounds__(kMatchThreads) sdnet_sweep_kernel(const SdnetS
     int* s_winner = i; i += G;
     int* s_jmin = i; i += S;
     int* s_stats = i;
-    match_pass(A, 4, K, p.M, true, conf, p.sx, p.sy, scale, p.gt_objects + (size_t)b * p.max_gt_objects * 3,
+    match_pass(A, 4, K, p.M, true, conf, nullptr, p.sx, p.sy, scale, p.gt_objects + (size_t)b * p.max_gt_objects * 3,
                min(p.n_gt_objects[b], p.max_gt_objects), p.anchor_stats + row * p.M * 3, p.anchor_acc + row * K, s_gx,
                s_gy, s_glab, s_winner, s_jmin, s_dist, s_stats);
-    match_pass(Q, 6, P, p.N, false, conf, p.sx, p.sy, scale, p.gt_parts + (size_t)b * p.max_gt_parts * 3,
+    match_pass(Q, 6, P, p.N, false, conf, nullptr, p.sx, p.sy, scale, p.gt_parts + (size_t)b * p.max_gt_parts * 3,
                min(p.n_gt_parts[b], p.max_gt_parts), p.part_stats + row * p.N * 3, p.part_acc + row * P, s_gx, s_gy,
                s_glab, s_winner, s_jmin, s_dist, s_stats);
   }
@@ -112,6 +112,7 @@ __global__ void __launch_bounds__(kMatchThreads) sdnet_sweep_kernel(const SdnetS
     op.gt_objects = p.gt_objects; op.n_gt_objects = p.n_gt_objects;
     op.gt_parts = p.gt_parts; op.gt_part_owner = p.gt_part_owner; op.n_gt_parts = p.n_gt_parts;
     op.cls_group = p.cls_group;
+    op.conf_class = nullptr;
     op.csi_stats = p.csi_stats; op.csi_acc = p.csi_acc;
     op.classif_stats = p.classif_stats; op.classif_acc = p.classif_acc; op.pred_parts = p.pred_parts;
   }

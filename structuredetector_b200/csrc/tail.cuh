@@ -12,6 +12,7 @@ struct TailParams {
   int cap;
   int pre_activated, no_grouping;
   float conf, dist_abs;
+  const float* conf_class;  // [M + N] per-class thresholds (anchor classes, then part kinds), or nullptr: conf for all
   const u64* lists;
   const int* counts;
   float* anchor_out;
@@ -369,6 +370,7 @@ __global__ void __launch_bounds__(2 * kTeamThreads, 3) sdnet_tail_kernel(const _
   __shared__ int s_misc[2][8];
   __shared__ float s_ax[SDNET_MAX_TOPK], s_ay[SDNET_MAX_TOPK];
   __shared__ int s_cnt[2];
+  __shared__ int s_end[2];  // last valid anchor / part slot + 1
   __shared__ int s_far;  // a valid anchor or part origin lies outside +-kNearField: grouping must look at the masked slots too
   const int b = blockIdx.x;
   Team tm;
@@ -376,7 +378,7 @@ __global__ void __launch_bounds__(2 * kTeamThreads, 3) sdnet_tail_kernel(const _
   tm.tid = threadIdx.x % kTeamThreads;
   const int W = p.W;
   const bool pre = p.pre_activated != 0;
-  if (threadIdx.x < 2) s_cnt[threadIdx.x] = 0;
+  if (threadIdx.x < 2) s_cnt[threadIdx.x] = s_end[threadIdx.x] = 0;
   if (threadIdx.x == 2) s_far = 0;
   pdl_wait();  // candidate lists (peaks kernel, possibly rewritten by the exact select) are final
   __syncthreads();
@@ -390,7 +392,7 @@ __global__ void __launch_bounds__(2 * kTeamThreads, 3) sdnet_tail_kernel(const _
     // ---- anchors
     const int have = select_group<DT>(tm, p, b, 0, p.M, p.K, sel, s_hist[0], s_misc[0]);
     if (have < p.K) zero_fill(tm, p, b, 0, have, p.K, sel, s_hist[0]);
-    int n_valid = 0;
+    int n_valid = 0, end = 0;
     for (int s = tm.tid; s < p.K; s += kTeamThreads) {
       const u64 v = sel[s];
       const int cls = 255 - (int)((v >> 24) & 0xffu);
@@ -401,14 +403,18 @@ __global__ void __launch_bounds__(2 * kTeamThreads, 3) sdnet_tail_kernel(const _
       const float y = __fadd_rn((float)yy, Num<DT>::to_float(__ldg(offy + (long long)yy * osh + xx)));
       store_out(p, reinterpret_cast<float4*>(p.anchor_out) + (size_t)b * p.K + s, make_float4(x, y, score, (float)cls));
       store_out(p, p.anchor_inds + (size_t)b * p.K + s, (long long)idx);
-      const bool valid = score > p.conf;
+      const bool valid = score > (p.conf_class ? __ldg(p.conf_class + cls) : p.conf);
       // masked anchors sit at (+1e6, +1e6): decoders.py:85-86
       s_ax[s] = valid ? x : kFar;
       s_ay[s] = valid ? y : kFar;
       n_valid += valid ? 1 : 0;
+      end = valid ? s + 1 : end;
       if (valid && !(fabsf(x) < kNearField && fabsf(y) < kNearField)) s_far = 1;
     }
-    if (n_valid) atomicAdd(&s_cnt[0], n_valid);
+    if (n_valid) {
+      atomicAdd(&s_cnt[0], n_valid);
+      atomicMax(&s_end[0], end);
+    }
   } else {
     // ---- parts
     const int have = select_group<DT>(tm, p, b, p.M, p.N, p.P, sel, s_hist[1], s_misc[1]);
@@ -416,7 +422,7 @@ __global__ void __launch_bounds__(2 * kTeamThreads, 3) sdnet_tail_kernel(const _
     const In* embx = p.embeddings.data ? static_cast<const In*>(p.embeddings.data) + (long long)b * p.embeddings.sb : nullptr;
     const In* emby = embx ? embx + p.embeddings.sc : nullptr;
     const long long esh = p.embeddings.sh;
-    int n_valid = 0;
+    int n_valid = 0, end = 0;
     for (int s = tm.tid; s < p.P; s += kTeamThreads) {
       const u64 v = sel[s];
       const int cls = 255 - (int)((v >> 24) & 0xffu);
@@ -437,14 +443,18 @@ __global__ void __launch_bounds__(2 * kTeamThreads, 3) sdnet_tail_kernel(const _
       store_out(p, po + 2, make_float2(ox, oy));
       store_out(p, p.part_inds + (size_t)b * p.P + s, (long long)idx);
       if (p.part_emb) store_out(p, reinterpret_cast<float2*>(p.part_emb) + (size_t)b * p.P + s, make_float2(ex, ey));
-      const bool valid = score > p.conf;
+      const bool valid = score > (p.conf_class ? __ldg(p.conf_class + p.M + cls) : p.conf);
       n_valid += valid ? 1 : 0;
+      end = valid ? s + 1 : end;
       if (valid && !(fabsf(ox) < kNearField && fabsf(oy) < kNearField)) s_far = 1;
       // masked parts sit at (-1e6, -1e6): decoders.py:80-81.  The slot's composite is no longer
       // needed: keep the part's origin there for the grouping pass.
       reinterpret_cast<float2*>(sel)[s] = make_float2(valid ? ox : -kFar, valid ? oy : -kFar);
     }
-    if (n_valid) atomicAdd(&s_cnt[1], n_valid);
+    if (n_valid) {
+      atomicAdd(&s_cnt[1], n_valid);
+      atomicMax(&s_end[1], end);
+    }
   }
   __syncthreads();
 
@@ -455,13 +465,14 @@ __global__ void __launch_bounds__(2 * kTeamThreads, 3) sdnet_tail_kernel(const _
   // the same root and the reference's min() then keeps the FIRST anchor.  Hence two sweeps without a
   // root in the loop: m2, then the first anchor whose square lies within 1e-6 of m2 (a root can only
   // tie if its square is within 2^-22 relative) AND whose root equals root(m2).
-  // Slots are in score order, so the valid anchors / parts are the first s_cnt[0] / s_cnt[1] slots.  Masked slots sit
-  // 1e6 away (decoders.py:80-86); as long as every valid coordinate is within kNearField = 1e5 and the gate is below
-  // 1e5, no pair with a masked member can pass the gate or tie with one that does, so only valid x valid pairs are
-  // searched (13 x 36 instead of 100 x 100 on the realistic maps).  Otherwise: the full P x K search.
+  // Masked slots sit 1e6 away (decoders.py:80-86); as long as every valid coordinate is within kNearField = 1e5 and the
+  // gate is below 1e5, no pair with a masked member can pass the gate or tie with one that does, so only the slots up
+  // to the last valid anchor / part are searched (13 x 36 instead of 100 x 100 on the realistic maps).  With one
+  // threshold those are exactly the valid slots (slots are in score order); with per-class thresholds masked slots can
+  // sit among them, at the 1e6 guard, where they cannot win.  Otherwise: the full P x K search.
   const float2* origin = reinterpret_cast<const float2*>(s_sel[1]);
   const bool full = s_far != 0 || !(p.dist_abs < kNearField);
-  const int Ka = full ? p.K : s_cnt[0], Pp = full ? p.P : s_cnt[1];
+  const int Ka = full ? p.K : s_end[0], Pp = full ? p.P : s_end[1];
   int g = 32;
   while (g > 1 && Pp * g > (int)blockDim.x) g >>= 1;
   const int sub = threadIdx.x & (g - 1), per_pass = blockDim.x / g;

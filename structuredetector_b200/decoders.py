@@ -71,18 +71,31 @@ class _DecoderBase:
 
 
 class Decoder(_DecoderBase):
-    """``decoder(outputs, conf_thresh=None, dist_thresh=None, return_metadata=False)``."""
+    """``decoder(outputs, conf_thresh=None, dist_thresh=None, return_metadata=False)``.
+
+    ``conf_thresh`` may also be a mapping from class or part kind name (``args._r_labels`` / ``args._r_parts``) to
+    threshold, e.g. ``ThresholdSweep.best_thresholds()``: every compare against the threshold then uses the entry of
+    the slot's own class, and a name the mapping leaves out takes ``args.conf_threshold``."""
+
+    def _conf(self, outputs, conf_thresh):
+        """The threshold as the decode takes it: a number, or M + N per-class thresholds."""
+        if conf_thresh is None:
+            return float(self.args.conf_threshold)
+        M, N = outputs["anchor_hm"].shape[1], outputs["part_hm"].shape[1]
+        names = lambda mapping, n: [mapping.get(i) for i in range(n)]
+        return ops.class_thresholds(conf_thresh, names(self.label_map, M), names(self.part_map, N), self.args.conf_threshold)
 
     def __call__(self, outputs, conf_thresh=None, dist_thresh=None, return_metadata=False):
-        conf_thresh = self.args.conf_threshold if conf_thresh is None else conf_thresh
+        conf_thresh = self._conf(outputs, conf_thresh)
         dist_thresh = self.args.decoder_dist_thresh if dist_thresh is None else dist_thresh
         out_size, in_size = self._sizes(outputs)
 
         packed = ops.decode_packed(outputs, self.max_objects, self.max_parts, conf_thresh, dist_thresh,
                                    pre_activated=self._pre_activated)
         host = self._to_host(packed)
+        host_conf = self._host_conf(conf_thresh, outputs["anchor_hm"].shape[1])
         with _gc_paused():
-            annotations = self._assemble(host, conf_thresh, out_size, in_size)
+            annotations = self._assemble(host, host_conf, out_size, in_size)
         if not return_metadata:
             return annotations
 
@@ -95,12 +108,15 @@ class Decoder(_DecoderBase):
         # returning them (decoders.py:79,84 then 166-173): kept, oddity included
         in_dtype = outputs["anchor_hm"].dtype
         conf32 = torch.tensor(conf_thresh, dtype=in_dtype, device=a.device).float()  # compared in the scores' dtype
-        mask = lambda s: torch.where(s > conf32, s, torch.full_like(s, -1.0))
+        a_conf = p_conf = conf32
+        if conf32.dim() == 1:  # each slot against its own class's threshold: anchor classes first, then part kinds
+            a_conf, p_conf = conf32[a[..., 3].long()], conf32[outputs["anchor_hm"].shape[1] + p[..., 3].long()]
+        mask = lambda s, conf: torch.where(s > conf, s, torch.full_like(s, -1.0))
         meta["embeddings"] = packed.part_emb if in_dtype == torch.float32 else packed.part_emb.to(in_dtype)
-        meta["topk_anchor"] = (mask(a[..., 2]), packed.anchor_inds, a[..., 3], a[..., 1], a[..., 0])
-        meta["topk_kp"] = (mask(p[..., 2]), packed.part_inds, p[..., 3], p[..., 1], p[..., 0])
+        meta["topk_anchor"] = (mask(a[..., 2], a_conf), packed.anchor_inds, a[..., 3], a[..., 1], a[..., 0])
+        meta["topk_kp"] = (mask(p[..., 2], p_conf), packed.part_inds, p[..., 3], p[..., 1], p[..., 0])
         with _gc_paused():
-            meta["raw_parts"] = self._raw_parts(host, conf_thresh, out_size, in_size)
+            meta["raw_parts"] = self._raw_parts(host, host_conf, out_size, in_size)
         meta["raw_embeddings"] = outputs["embeddings"]
         meta["raw_offsets"] = outputs["offsets"]
         return meta
@@ -113,13 +129,15 @@ class Decoder(_DecoderBase):
 
         With ``img_sizes`` (one ``(w, h)`` per image) and ``net_size = (args.width, args.height)`` the documents are
         those of the reference's ``detect`` loop (cli/detect.py:41-52): the annotation resized from the network input
-        to the original image, ``img_size`` and ``image_path`` set.  ``image_paths`` default to ``batch_<i>``."""
-        conf_thresh = self.args.conf_threshold if conf_thresh is None else conf_thresh
+        to the original image, ``img_size`` and ``image_path`` set.  ``image_paths`` default to ``batch_<i>``.
+        ``conf_thresh``: as for ``__call__``, a number or a name mapping."""
+        conf_thresh = self._conf(outputs, conf_thresh)
         dist_thresh = self.args.decoder_dist_thresh if dist_thresh is None else dist_thresh
         out_size, in_size = self._sizes(outputs)
         packed = ops.decode_packed(outputs, self.max_objects, self.max_parts, conf_thresh, dist_thresh,
                                    pre_activated=self._pre_activated)
-        return self._json_from_host(self._to_host(packed), conf_thresh, out_size, in_size, image_paths, img_sizes, net_size)
+        return self._json_from_host(self._to_host(packed), self._host_conf(conf_thresh, outputs["anchor_hm"].shape[1]), out_size,
+                                    in_size, image_paths, img_sizes, net_size)
 
     def _json_from_host(self, host, conf_thresh, out_size, in_size, image_paths=None, img_sizes=None, net_size=None):
         B, K = host.anchor_out.shape[:2]
@@ -134,7 +152,7 @@ class Decoder(_DecoderBase):
         enc = lambda names: [None if name is None else json.dumps(name) for name in names]
         return _fastobj.json_text(
             host.anchor_out.contiguous().numpy(), host.part_out.contiguous().numpy(), host.assign.contiguous().numpy(), B, K,
-            host.part_out.shape[1], float(conf_thresh), in_size[0] / out_size[0], in_size[1] / out_size[1], resize,
+            host.part_out.shape[1], self._side(conf_thresh, 0), in_size[0] / out_size[0], in_size[1] / out_size[1], resize,
             enc(self._names(self.label_map)), enc(self._names(self.part_map)), json.dumps(self.anchor_name),
             [json.dumps(str(path.expanduser().resolve())) for path in paths],
             [json.dumps(None if size is None else list(size), indent=2).replace("\n", "\n  ") for size in sizes])
@@ -154,13 +172,24 @@ class Decoder(_DecoderBase):
     def _assemble(self, host: ops.PackedDetections, conf_thresh, out_size, in_size):
         """Python objects from the packed rows, built by the C loop in ``csrc/fastobj.c``: float32 coordinates
         widened to double and multiplied by ``in/out`` in double (the reference multiplies ``.item()`` doubles),
-        ``score > conf`` in double, parts bucketed by anchor slot in part-slot order."""
+        ``score > conf`` in double, parts bucketed by anchor slot in part-slot order.  ``conf_thresh``: a number, or
+        (thresholds of the anchor classes, thresholds of the part kinds)."""
         sx, sy = in_size[0] / out_size[0], in_size[1] / out_size[1]
         a, p, assign = host.anchor_out, host.part_out, host.assign
         B, K = a.shape[:2]
         return _fastobj.assemble(a.contiguous().numpy(), p.contiguous().numpy(), assign.contiguous().numpy(), B, K,
-                                 p.shape[1], float(conf_thresh), sx, sy, self._names(self.label_map),
+                                 p.shape[1], self._side(conf_thresh, 0), sx, sy, self._names(self.label_map),
                                  self._names(self.part_map), self.anchor_name, Keypoint, Object, ImageAnnotation)
+
+    @staticmethod
+    def _host_conf(conf_thresh, M):
+        """What the host loops compare scores with: the number, or (anchor classes' thresholds, part kinds')."""
+        return (conf_thresh[:M], conf_thresh[M:]) if isinstance(conf_thresh, list) else float(conf_thresh)
+
+    @staticmethod
+    def _side(conf_thresh, side):
+        """The anchors' (side 0) or the parts' (side 1) threshold argument of the host loops."""
+        return conf_thresh[side] if isinstance(conf_thresh, tuple) else float(conf_thresh)
 
     @staticmethod
     def _names(mapping):
@@ -176,7 +205,7 @@ class Decoder(_DecoderBase):
     def _raw_parts(self, host: ops.PackedDetections, conf_thresh, out_size, in_size):
         sx, sy = in_size[0] / out_size[0], in_size[1] / out_size[1]
         p = host.part_out
-        return _fastobj.keypoints(p.contiguous().numpy(), p.shape[0], p.shape[1], p.shape[2], float(conf_thresh), sx, sy,
+        return _fastobj.keypoints(p.contiguous().numpy(), p.shape[0], p.shape[1], p.shape[2], self._side(conf_thresh, 1), sx, sy,
                                   self._names(self.part_map), Keypoint)
 
 

@@ -273,8 +273,14 @@ class Evaluator:
         ``annotations`` = the batch's ground truth (``ImageAnnotation`` with ``img_size``, coordinates in the
         network-input frame, as the reference's dataset yields them), ``out_size`` = (W, H) of the heat maps.
         Equivalent to ``accumulate(prediction, annotation, raw_parts, eval_csi, eval_classif)`` of the reference per
-        image (evaluator.py:226-242; ``evaluate`` passes True, True: cli/evaluate.py:43-45)."""
-        conf = self.args.conf_threshold if conf_thresh is None else conf_thresh
+        image (evaluator.py:226-242; ``evaluate`` passes True, True: cli/evaluate.py:43-45).
+
+        ``conf_thresh`` may be a mapping from label or part name to threshold, as ``Decoder`` takes it (the one the
+        batch was decoded with): detections are then counted against their own label's threshold, and a name the
+        mapping leaves out takes ``args.conf_threshold``."""
+        default = self.args.conf_threshold
+        conf = ops.class_thresholds(default if conf_thresh is None else conf_thresh, self._index_names(self._label_names),
+                                    self._index_names(self._part_names), default)
         B, K = packed.anchor_inds.shape
         P = packed.part_inds.shape[1]
         assert len(annotations) == B
@@ -285,6 +291,9 @@ class Evaluator:
         p_stats = torch.empty(B, N, 3, dtype=torch.int32, device=device)
         a_acc = torch.empty(B, K, dtype=torch.float64, device=device)
         p_acc = torch.empty(B, P, dtype=torch.float64, device=device)
+        # per-class thresholds: M + N doubles (labels, then parts); `conf` covers classes the table has no entry for
+        conf_class = torch.tensor(conf, dtype=torch.float64, device=device) if isinstance(conf, list) else None
+        conf = float(default) if conf_class is not None else conf
         out_w, out_h = out_size
         in_w, in_h = int(self.args.down_ratio * out_w), int(self.args.down_ratio * out_h)  # decoders.py:37-38
         prm = _native.SdnetMatchParams()
@@ -298,6 +307,7 @@ class Evaluator:
         prm.gt_parts, prm.n_gt_parts = gt_p.data_ptr(), n_p.data_ptr()
         prm.anchor_stats, prm.part_stats = a_stats.data_ptr(), p_stats.data_ptr()
         prm.anchor_acc, prm.part_acc = a_acc.data_ptr(), p_acc.data_ptr()
+        prm.conf_class = conf_class.data_ptr() if conf_class is not None else None
         stream = torch.cuda.current_stream(device).cuda_stream
         _native.check(self.lib.sdnet_match_launch(ctypes.byref(prm), ctypes.c_void_p(stream)), "sdnet_match_launch")
         a_cls = packed.anchor_out[:, :, 3].to(torch.int32)
@@ -327,6 +337,7 @@ class Evaluator:
         op.cls_group = groups.data_ptr()
         op.csi_stats, op.csi_acc = c_stats.data_ptr(), c_acc.data_ptr()
         op.classif_stats, op.classif_acc, op.pred_parts = k_stats.data_ptr(), k_acc.data_ptr(), n_parts.data_ptr()
+        op.conf_class = prm.conf_class
         _native.check(self.lib.sdnet_match_objects_launch(ctypes.byref(op), ctypes.c_void_p(stream)), "sdnet_match_objects_launch")
         c_stats, k_stats, c_acc, k_acc, n_parts = (t.cpu().numpy() for t in (c_stats, k_stats, c_acc, k_acc, n_parts))
         if eval_csi:
@@ -336,6 +347,11 @@ class Evaluator:
             key = np.where((n_parts >= 0) & (n_parts <= 9), group_np[np.clip(host[4], 0, M - 1)] * 10 + n_parts, -1)
             key = np.where(group_np[np.clip(host[4], 0, M - 1)] >= 0, key, -1)
             self._absorb(self.classification_eval, dict(enumerate(Evaluator.get_classification_labels())), k_stats, k_acc, key)
+
+    @staticmethod
+    def _index_names(names):
+        """Name of every index 0 .. max, None where an index has no name."""
+        return [names.get(i) for i in range(max(names, default=-1) + 1)]
 
     def _classification_groups(self, device):
         """cls_group of the object matchers: 0 / 1 for the classes named "bean" / "maize", -1 for the others."""
@@ -603,6 +619,16 @@ class ThresholdSweep:
     def best_threshold(self, table: str, label=None, gate=None) -> float:
         """The grid threshold with the highest F1 score of ``table`` / ``label`` at ``gate`` (the lowest one on a tie)."""
         return float(self.thresholds[int(np.argmax(self.curve(table, label, gate)["f1_score"]))])
+
+    def best_thresholds(self, gate=None) -> dict:
+        """``{name: threshold}``: every label's ``best_threshold`` of the ``anchor`` table and every part kind's of the
+        ``part`` table, at ``gate``.  Pass it as ``conf_thresh`` to ``Decoder`` and ``Evaluator.accumulate_packed``:
+        a decode with these thresholds has, label by label, exactly the location tables of ``at(best)`` for that label,
+        because a label's detections are matched against that label's ground truth only."""
+        ev = self._grid[0][0]
+        best = {name: self.best_threshold("anchor", name, gate) for name in ev.labels}
+        best.update({name: self.best_threshold("part", name, gate) for name in ev.kp_labels})
+        return best
 
     def surface(self, table: str, label=None) -> dict:
         """``curve`` over the whole grid: threshold (T,), gate (G,), and tp, npos, ndet, precision, recall, f1_score

@@ -12,6 +12,8 @@ src/sdnet/utils/utils.py:342-361,422-467.
 from __future__ import annotations
 
 import ctypes
+import math
+from collections.abc import Mapping
 from dataclasses import dataclass
 
 import torch
@@ -23,7 +25,7 @@ from ._native import (FLAG_EXACT_SELECT, FLAG_NO_GROUPING, FLAG_PRE_ACTIVATED, F
                       SdnetSchedule, SdnetTensor4)
 
 __all__ = ["decode_packed", "activate_maps", "suppress_maps", "suppress_into", "DecodePlan", "DecodePipeline",
-           "PackedDetections", "gpu_launches_per_decode"]
+           "PackedDetections", "gpu_launches_per_decode", "class_thresholds"]
 
 # kernels launched by one sdnet_decode_launch: peaks, exact-select, tail (+ one memset node)
 _KERNELS_PER_DECODE = 3
@@ -162,19 +164,34 @@ class DecodePlan:
             elif not (host_ok and t.is_pinned()):
                 raise RuntimeError(f"{name} lives on {t.device}: the B200 decode path has no CPU fallback")
 
+    def _check_conf_class(self, conf_class):
+        """The tail kernel reads M + N fp32 thresholds from the table's device pointer: refuse anything else."""
+        _, M, N = self.shape[:3]
+        if conf_class.dtype != torch.float32 or conf_class.dim() != 1 or conf_class.numel() != M + N:
+            raise ValueError(f"conf_class: expected a 1-D float32 tensor of M + N = {M + N} thresholds, got "
+                             f"{conf_class.dtype} of shape {tuple(conf_class.shape)}")
+        if not conf_class.is_cuda or conf_class.device != self.device or not conf_class.is_contiguous():
+            raise ValueError(f"conf_class must be a contiguous tensor on {self.device}, not on {conf_class.device}")
+
     def _bind_inputs(self, anchor_hm, part_hm, offsets, embeddings, conf_f32, dist_abs_f32, radius, flags,
-                     host_ok: bool = False):
+                     host_ok: bool = False, conf_class=None):
         self._check_inputs(anchor_hm, part_hm, offsets, embeddings, host_ok)
+        if conf_class is not None:
+            self._check_conf_class(conf_class)
         p = self.params
         p.anchor_hm, p.part_hm, p.offsets = _view4(anchor_hm), _view4(part_hm), _view4(offsets)
         p.embeddings = _view4(embeddings) if embeddings is not None else SdnetTensor4(None, 0, 0, 0, 1)
         p.conf_f32, p.dist_abs_f32 = conf_f32, dist_abs_f32
+        p.conf_class_f32 = conf_class.data_ptr() if conf_class is not None else None
         p.radius, p.flags = radius, flags
 
     def run(self, anchor_hm, part_hm, offsets, embeddings, conf_f32, dist_abs_f32, radius=2, flags=0,
-            stream=None) -> PackedDetections:
-        """Enqueue one decode on ``stream`` (a torch stream or raw handle; default: torch's current stream). Asynchronous."""
-        self._bind_inputs(anchor_hm, part_hm, offsets, embeddings, conf_f32, dist_abs_f32, radius, flags)
+            stream=None, conf_class=None) -> PackedDetections:
+        """Enqueue one decode on ``stream`` (a torch stream or raw handle; default: torch's current stream). Asynchronous.
+        ``conf_class``: optional per-class thresholds, a float32 tensor of M + N entries on the plan's device (anchor
+        classes, then part kinds; each rounded to the heat maps' dtype) used instead of ``conf_f32``."""
+        self._bind_inputs(anchor_hm, part_hm, offsets, embeddings, conf_f32, dist_abs_f32, radius, flags,
+                          conf_class=conf_class)
         if stream is None:
             stream = torch.cuda.current_stream(self.device)
         stream = getattr(stream, "cuda_stream", stream)  # a torch.cuda.Stream or a raw cudaStream_t
@@ -201,18 +218,22 @@ class DecodePlan:
         d["path"] = PEAKS_PATHS[d["path"]]
         return d
 
-    def run_timed(self, anchor_hm, part_hm, offsets, embeddings, conf_f32, dist_abs_f32, radius=2, flags=0):
+    def run_timed(self, anchor_hm, part_hm, offsets, embeddings, conf_f32, dist_abs_f32, radius=2, flags=0,
+                  conf_class=None):
         """Synchronous profiling run: returns (peaks_ms, exact_select_ms, tail_ms) device times."""
-        self._bind_inputs(anchor_hm, part_hm, offsets, embeddings, conf_f32, dist_abs_f32, radius, flags)
+        self._bind_inputs(anchor_hm, part_hm, offsets, embeddings, conf_f32, dist_abs_f32, radius, flags,
+                          conf_class=conf_class)
         ms = (ctypes.c_float * 3)()
         stream = torch.cuda.current_stream(self.device).cuda_stream
         self._launch(self.lib.sdnet_decode_launch_timed, ctypes.c_void_p(stream), ms)
         return tuple(float(x) for x in ms)
 
     def run_host(self, anchor_hm, part_hm, offsets, embeddings, conf_f32, dist_abs_f32, staging: torch.Tensor,
-                 radius=2, flags=0, stream=None) -> PackedDetections:
-        """Same, with the four inputs in pinned HOST memory (``sdnet_decode_host_launch``)."""
-        self._bind_inputs(anchor_hm, part_hm, offsets, embeddings, conf_f32, dist_abs_f32, radius, flags, host_ok=True)
+                 radius=2, flags=0, stream=None, conf_class=None) -> PackedDetections:
+        """Same, with the four inputs in pinned HOST memory (``sdnet_decode_host_launch``); ``conf_class`` stays a
+        device tensor."""
+        self._bind_inputs(anchor_hm, part_hm, offsets, embeddings, conf_f32, dist_abs_f32, radius, flags, host_ok=True,
+                          conf_class=conf_class)
         if stream is None:
             stream = torch.cuda.current_stream(self.device)
         stream = getattr(stream, "cuda_stream", stream)
@@ -252,15 +273,18 @@ class DecodePipeline:
         for st in self.streams:
             st.wait_event(event)
 
-    def submit(self, anchor_hm, part_hm, offsets, embeddings, conf_f32, dist_abs_f32, radius=2, flags=0):
+    def submit(self, anchor_hm, part_hm, offsets, embeddings, conf_f32, dist_abs_f32, radius=2, flags=0,
+               conf_class=None):
+        """``conf_class``: as ``DecodePlan.run``; only plans that take it (``DecodePlan``) accept a table."""
         k = self._next
         self._next = (k + 1) % len(self.plans)
         self.streams[k].wait_stream(torch.cuda.current_stream(self.device))
-        for t in (anchor_hm, part_hm, offsets, embeddings):
+        for t in (anchor_hm, part_hm, offsets, embeddings, conf_class):
             if t is not None and t.is_cuda:
                 t.record_stream(self.streams[k])
+        extra = {} if conf_class is None else {"conf_class": conf_class}
         out = self.plans[k].run(anchor_hm, part_hm, offsets, embeddings, conf_f32, dist_abs_f32, radius, flags,
-                                stream=self.streams[k])
+                                stream=self.streams[k], **extra)
         self.events[k].record(self.streams[k])
         return out, self.events[k]
 
@@ -278,6 +302,40 @@ def _f32(value: float, dtype: torch.dtype = torch.float32) -> float:
     """Round a Python double to `dtype` the way torch does when a tensor of that dtype is compared
     with a scalar (the result is exactly representable in fp32 for every supported dtype)."""
     return float(torch.tensor(value, dtype=dtype))
+
+
+def class_thresholds(conf_thresh, class_names, kind_names, default) -> float | list[float]:
+    """A decoder or evaluator threshold as the kernels take it: a number stays a number; a mapping from class or part
+    kind name to threshold becomes one threshold per anchor class, then one per part kind.  ``class_names`` /
+    ``kind_names``: the name of each class / kind index (``None`` for an index without a name); a name the mapping
+    leaves out takes ``default``.  A name that is both a class and a kind sets both.  Raises ``ValueError`` for a name
+    that is neither and for a threshold that is not finite."""
+    if not isinstance(conf_thresh, Mapping):
+        return float(conf_thresh)
+    known = set(class_names) | set(kind_names)
+    unknown = [name for name in conf_thresh if name is None or name not in known]
+    if unknown:
+        raise ValueError(f"conf_thresh names {unknown!r}, which are neither classes {[n for n in class_names if n is not None]} "
+                         f"nor part kinds {[n for n in kind_names if n is not None]}")
+    table = {name: float(value) for name, value in conf_thresh.items()}
+    bad = {name: value for name, value in table.items() if not math.isfinite(value)}
+    if bad:
+        raise ValueError(f"conf_thresh values must be finite: {bad!r}")
+    default = float(default)
+    return [table.get(name, default) if name is not None else default for name in (*class_names, *kind_names)]
+
+
+def _conf_arg(conf_thresh, M: int, N: int, dtype: torch.dtype, device) -> tuple[float, torch.Tensor | None]:
+    """(conf_f32, conf_class) of a decode: one threshold, or M + N per-class thresholds (anchor classes, then part
+    kinds) as a device table, each rounded to the heat maps' dtype like the scalar."""
+    if not isinstance(conf_thresh, (list, tuple)) and getattr(conf_thresh, "ndim", 0) == 0:
+        return _f32(float(conf_thresh), dtype), None
+    values = [float(v) for v in (conf_thresh.tolist() if hasattr(conf_thresh, "tolist") else conf_thresh)]
+    if len(values) != M + N:
+        raise ValueError(f"per-class conf_thresh has {len(values)} entries; the heat maps have M + N = {M + N} classes")
+    if not all(math.isfinite(v) for v in values):
+        raise ValueError("per-class conf_thresh values must be finite")
+    return 0.0, torch.tensor([_f32(v, dtype) for v in values], dtype=torch.float32).to(device)
 
 
 # ------------------------------------------------------------------------------------ custom ops
@@ -301,7 +359,7 @@ def _op_plan(device, B, M, N, H, W, K, P, dtype) -> DecodePlan:
 @torch.library.custom_op("sdnet_b200::decode", mutates_args=(), device_types="cuda")
 def _decode_op(anchor_hm: torch.Tensor, part_hm: torch.Tensor, offsets: torch.Tensor, embeddings: torch.Tensor,
                max_objects: int, max_parts: int, conf_f32: float, dist_abs_f32: float, radius: int,
-               flags: int) -> torch.Tensor:
+               flags: int, conf_class: torch.Tensor | None = None) -> torch.Tensor:
     B, M, H, W = anchor_hm.shape
     N = part_hm.shape[1]
     with torch.cuda.device(anchor_hm.device):
@@ -309,12 +367,13 @@ def _decode_op(anchor_hm: torch.Tensor, part_hm: torch.Tensor, offsets: torch.Te
         # the op returns a fresh tensor (no aliasing between calls); the workspace is the cached part
         blob = torch.empty(plan.out.blob.numel(), dtype=torch.uint8, device=anchor_hm.device)
         plan._bind_outputs(_carve(blob, B, max_objects, max_parts, M + N))
-        plan.run(anchor_hm, part_hm, offsets, embeddings, conf_f32, dist_abs_f32, radius, flags)
+        plan.run(anchor_hm, part_hm, offsets, embeddings, conf_f32, dist_abs_f32, radius, flags, conf_class=conf_class)
     return blob
 
 
 @_decode_op.register_fake
-def _(anchor_hm, part_hm, offsets, embeddings, max_objects, max_parts, conf_f32, dist_abs_f32, radius, flags):
+def _(anchor_hm, part_hm, offsets, embeddings, max_objects, max_parts, conf_f32, dist_abs_f32, radius, flags,
+      conf_class=None):
     B, M = anchor_hm.shape[:2]
     N = part_hm.shape[1]
     return anchor_hm.new_empty(packed_nbytes(B, max_objects, max_parts, M + N), dtype=torch.uint8)
@@ -371,10 +430,14 @@ def _unit_w_stride(t: torch.Tensor) -> torch.Tensor:
     return t if t.stride(3) == 1 else t.contiguous()
 
 
-def decode_packed(outputs: dict, max_objects: int, max_parts: int, conf_thresh: float, dist_thresh: float, *,
+def decode_packed(outputs: dict, max_objects: int, max_parts: int, conf_thresh, dist_thresh: float, *,
                   pre_activated: bool = False, group: bool = True, radius: int = 2,
                   exact_select: bool = False, warp_kernel: bool = False) -> PackedDetections:
-    """Run the CUDA decode on the four network-output views and return packed device tensors."""
+    """Run the CUDA decode on the four network-output views and return packed device tensors.
+
+    ``conf_thresh``: one threshold, or a sequence of M + N per-class thresholds -- one per anchor class (heat-map
+    channel), then one per part kind -- each slot compared against the entry of its own class (``class_thresholds``
+    builds one from a name mapping).  Only ``counts`` and the grouping depend on it."""
     a_hm, p_hm, off = outputs["anchor_hm"], outputs["part_hm"], outputs["offsets"]
     emb = outputs["embeddings"] if group or "embeddings" in outputs else None
     on_host = not a_hm.is_cuda  # pinned host tensors take the host-buffer entry point (everything else on a CPU raises)
@@ -388,18 +451,20 @@ def decode_packed(outputs: dict, max_objects: int, max_parts: int, conf_thresh: 
         emb = off  # never read under NO_GROUPING without part_emb consumers; keeps the op signature tensor-only
     flags = (FLAG_PRE_ACTIVATED if pre_activated else 0) | (0 if group else FLAG_NO_GROUPING) | (
         FLAG_EXACT_SELECT if exact_select else 0) | (FLAG_WARP_KERNEL if warp_kernel else 0)
-    if on_host:
-        return _decode_from_host(a_hm, p_hm, off, emb, int(max_objects), int(max_parts),
-                                 _f32(conf_thresh, a_hm.dtype), _f32(float(dist_thresh) * min(W, H)), int(radius), int(flags))
-    a_hm, p_hm, off, emb = map(_unit_w_stride, (a_hm, p_hm, off, emb))
     # `scores > conf` compares in the scores' dtype (fp16 scores against fp16(conf)); the distance gate
     # always compares fp32 distances
-    blob = _decode_op(a_hm, p_hm, off, emb, int(max_objects), int(max_parts), _f32(conf_thresh, a_hm.dtype),
-                      _f32(float(dist_thresh) * min(W, H)), int(radius), int(flags))
+    device = a_hm.device if not on_host else torch.device("cuda", torch.cuda.current_device())
+    conf_f32, conf_class = _conf_arg(conf_thresh, M, N, a_hm.dtype, device)
+    if on_host:
+        return _decode_from_host(a_hm, p_hm, off, emb, int(max_objects), int(max_parts),
+                                 conf_f32, _f32(float(dist_thresh) * min(W, H)), int(radius), int(flags), conf_class)
+    a_hm, p_hm, off, emb = map(_unit_w_stride, (a_hm, p_hm, off, emb))
+    blob = _decode_op(a_hm, p_hm, off, emb, int(max_objects), int(max_parts), conf_f32,
+                      _f32(float(dist_thresh) * min(W, H)), int(radius), int(flags), conf_class)
     return _carve(blob, B, int(max_objects), int(max_parts), M + N)
 
 
-def _decode_from_host(a_hm, p_hm, off, emb, K, P, conf_f32, dist_abs_f32, radius, flags) -> PackedDetections:
+def _decode_from_host(a_hm, p_hm, off, emb, K, P, conf_f32, dist_abs_f32, radius, flags, conf_class=None) -> PackedDetections:
     """Pinned HOST tensors -> packed detections on the current CUDA device (``sdnet_decode_host_launch``:
     the heat planes are uploaded into a cached staging buffer, offsets/embeddings are read in place)."""
     B, M, H, W = a_hm.shape
@@ -412,7 +477,7 @@ def _decode_from_host(a_hm, p_hm, off, emb, K, P, conf_f32, dist_abs_f32, radius
     blob = torch.empty(plan.out.blob.numel(), dtype=torch.uint8, device=device)
     out = _carve(blob, B, K, P, M + N)
     plan._bind_outputs(out)
-    plan.run_host(a_hm, p_hm, off, emb, conf_f32, dist_abs_f32, plan.staging, radius, flags)
+    plan.run_host(a_hm, p_hm, off, emb, conf_f32, dist_abs_f32, plan.staging, radius, flags, conf_class=conf_class)
     return out
 
 
