@@ -43,6 +43,8 @@ extern "C" {
                                           decode of the same shape (every decode leaves the workspace header zeroed behind
                                           it), so the per-call cudaMemsetAsync of the header is skipped: one stream
                                           operation less per decode.  Never set it for a fresh or reused-elsewhere buffer. */
+#define SDNET_FLAG_NO_FLOOR_HINT 32u /* start every plane with no pruning floor, instead of at the floor hint that the
+                                        batch's finished planes of the same channel supply (same results either way) */
 
 /* argument errors */
 #define SDNET_E_NULL -1      /* a required pointer is NULL */

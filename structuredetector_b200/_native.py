@@ -21,6 +21,7 @@ FLAG_NO_GROUPING = 2
 FLAG_EXACT_SELECT = 4
 FLAG_WARP_KERNEL = 8
 FLAG_WORKSPACE_CLEAN = 16
+FLAG_NO_FLOOR_HINT = 32
 DTYPE_F32 = 0
 DTYPE_F16 = 1
 DTYPE_BF16 = 2

@@ -25,6 +25,11 @@ constexpr float kBinScale = 4.0f;      // bins of 0.25 logit
 constexpr int kFineBins = 512;         // shared (CTA-wide / plane-wide) histograms: bins of 1/16 logit
 constexpr float kFineScale = 16.0f;    // (256 x 0.125: blobs 3 % slower; 1024 x 1/32: flushes 25 % slower)
 constexpr int kFinePerLane = kFineBins / 32;
+// Floor hint (peaks_tile.cuh): planes of a channel that must have finished before their lowest floor, less a margin, is
+// applied to the channel's other planes.  Measured at 1024 cfg5 images, one B200 (1000 W), no plane through the exact
+// select in 25 decodes with a margin of 1, 2 or 4 bins; 2 costs 3-10 % more candidates than 1, 4 another 5-20 %.
+constexpr int kHintMinPlanes = 8;
+constexpr int kHintMarginBins = 2;     // fine bins: 1/8 logit
 constexpr float kSatX = 14.0f;         // |x| >= 14 is inside the clamp on both sides: S(x) == S(+-14)
 constexpr float kPreScale = 8.0f;      // pre-activated maps: histogram runs on 8*value
 constexpr float kClampLo = 1e-6f;
@@ -57,6 +62,14 @@ struct PeaksParams {
   int tier1_units, groups_per_col, chunk_groups;
   u32 total_groups;
   int odd_x;               // tile kernel, row-pair maps: tensor-map x coordinate of an odd row's column 0
+};
+
+// The tile kernel's floor hint (peaks_tile.cuh), an argument of its own so that PeaksParams -- which the suppress kernel
+// takes too -- keeps its layout.  chint[c][0] = kFineBins - the lowest gfloor reported by a finished plane of channel c,
+// chint[c][1] = planes that reported (zeroed = no hint); hint_used[plane] = highest hint bin applied to it (0 = none).
+struct HintParams {
+  u32* chint;
+  int* hint_used;
 };
 
 // Numerics of the score function per input dtype DT (SDNET_DTYPE_*).

@@ -4,8 +4,8 @@
 namespace {
 
 // ---------------------------------------------------------------------------------------------
-// exact-select kernel: bounded-memory fallback for planes whose candidate list overflowed
-// (or for every plane under SDNET_FLAG_EXACT_SELECT).  One CTA per plane: a 3-level radix
+// exact-select kernel: bounded-memory fallback for planes whose candidate list overflowed, or whose
+// floor hint pruned too much (below), or for every plane under SDNET_FLAG_EXACT_SELECT.  One CTA per plane: a 3-level radix
 // select (11/11/10 bits) over the NMS'd scores recomputed straight from the heat map, then an
 // index-ordered emission pass that keeps every score above the K-th and the lowest-index
 // members of the K-th score's tie run.  Rewrites the plane's list with <= K records.
@@ -23,10 +23,32 @@ struct ExactParams {
   View4 anchor, part;
   int B, M, N, H, W, K, P;
   int radius, cap, force, pre_activated;
+  int check_hints;       // the peaks kernel may have applied floor hints (hint_used)
   u64* lists;
   int* counts;
   int* flags;
+  const int* gfloor;     // the peaks kernel's plane floors and histograms (PeaksParams) and applied hints (HintParams)
+  const u32* ghist;
+  const int* hint_used;
 };
+
+// Does the floor hint applied to a plane need the plane redone?  A hint bin h pruned every pixel x with
+// x <= shared_floor(h) (floors.cuh): x < edge(h) - kNear(edge(h)), so S(x) < S(edge(h)) strictly (pre-activated maps:
+// x <= edge(h) / kPreScale, the bound the plane-wide floor applies too).  ghist counts kept survivors only, each in a
+// bin whose lower edge is never above its clamped logit, so every candidate counted in bins >= hint_used scores at
+// least S(edge(hint_used)) >= S(edge(h)) for every hint h the plane's warps applied (h <= hint_used; S is monotone).  With >= K of them the pruned pixels cannot
+// reach the plane's top K -- exactly the certificate gfloor rests on -- so a plane whose gfloor is already >= hint_used
+// passes on that one word, and only the rest sum their histogram.
+__device__ __forceinline__ bool hint_pruned_too_much(const u32* ghist, int hint_bin, int K, int* s_sum) {
+  if (threadIdx.x == 0) *s_sum = 0;
+  __syncthreads();
+  u32 s = 0;
+  for (int bin = hint_bin + (int)threadIdx.x; bin < kFineBins; bin += blockDim.x) s += __ldcg(ghist + bin);
+  s = __reduce_add_sync(0xffffffffu, s);
+  if ((threadIdx.x & 31) == 0 && s) atomicAdd(s_sum, (int)s);
+  __syncthreads();
+  return *s_sum < K;
+}
 
 template <int DT>
 __device__ __forceinline__ u32 exact_key(const void* plane, long long sh, int H, int W, int R, int y, int x, bool pre) {
@@ -99,28 +121,36 @@ __global__ void __launch_bounds__(kExactThreads, kExactCtasPerSm) sdnet_exact_se
   __shared__ int s_out[2];
   __shared__ int s_warp[kExactThreads / 32][2];
   __shared__ int s_base[2];
+  __shared__ int s_sum;
   const int C = p.M + p.N;
   const int planes = p.B * C;
   pdl_launch_dependents();
   pdl_wait();  // the peaks kernel's lists and counts are complete and visible
   if (!p.force) {
-    // common case: nothing overflowed.  One coalesced look at this CTA's planes, then leave.
+    // common case: nothing overflowed and every floor hint is covered by its plane's floor.  One coalesced look at
+    // this CTA's planes, then leave.
     int mine = 0;
     for (int q = blockIdx.x + threadIdx.x * gridDim.x; q < planes; q += blockDim.x * gridDim.x)
-      mine |= p.counts[q] > p.cap;
+      mine |= p.counts[q] > p.cap || (p.check_hints && p.hint_used[q] > p.gfloor[q]);
     if (!__syncthreads_or(mine)) return;
   }
   for (int plane_id = blockIdx.x; plane_id < planes; plane_id += gridDim.x) {
   const int emitted = p.counts[plane_id];
-  if (!p.force && emitted <= p.cap) continue;  // block-uniform
-  __syncthreads();
   const int b = plane_id / C, c = plane_id % C;
   const bool is_anchor = c < p.M;
+  const int K = is_anchor ? p.K : p.P;
+  if (!p.force && emitted <= p.cap) {  // block-uniform
+    if (!p.check_hints) continue;
+    const int hint_bin = p.hint_used[plane_id];
+    if (hint_bin <= p.gfloor[plane_id]) continue;
+    __syncthreads();  // s_sum
+    if (!hint_pruned_too_much(p.ghist + (size_t)plane_id * kFineBins, hint_bin, K, &s_sum)) continue;
+  }
+  __syncthreads();
   const View4& vw = is_anchor ? p.anchor : p.part;
   const void* plane = static_cast<const typename Num<DT>::In*>(vw.data) + (long long)b * vw.sb +
                       (long long)(is_anchor ? c : c - p.M) * vw.sc;
   const long long sh = vw.sh;
-  const int K = is_anchor ? p.K : p.P;
   const int H = p.H, W = p.W, HW = H * W, R = p.radius;
   const bool pre = p.pre_activated != 0;
   const int tid = threadIdx.x;

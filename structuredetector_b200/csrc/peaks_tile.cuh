@@ -375,10 +375,13 @@ __device__ __forceinline__ void tile_fix_edges(u32 slot_s, int x0, int W, int la
 // at pitch + x - 4 (a box has to start on a 16-byte boundary, measured: anything else is an illegal
 // instruction) -- and lands in its slot as rows 0, 2 | 1, 3 with the odd rows 8 bytes further right.
 // At the image edges such a box reads across the row boundary; tile_fix_edges repairs that after the wait.
-template <int R, int DT, int S>
+// kHint: the launch has floor hints (HintParams; sdnet_decode.cu picks the instantiation).  Without, the hint code is
+// compiled out: the flag it needs for the polling below costs a register, and a launch with no hints to give should not
+// pay for it.
+template <int R, int DT, int S, bool kHint>
 __global__ void __launch_bounds__(kTileWarps * 32, kTileMinCtas)
 sdnet_peaks_tile_kernel(const __grid_constant__ PeaksParams p, const __grid_constant__ CUtensorMap tm_anchor,
-                        const __grid_constant__ CUtensorMap tm_part) {
+                        const __grid_constant__ CUtensorMap tm_part, const __grid_constant__ HintParams hp) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   constexpr int NG = kTileNG;
   constexpr u32 kRingRows = NG * kGroupRows;
@@ -495,6 +498,23 @@ sdnet_peaks_tile_kernel(const __grid_constant__ PeaksParams p, const __grid_cons
     }
     y_next += kGroupRows * NG;
     int gfloor_seen = 0;
+    bool hinted = false;
+    if (kHint) {
+      // Start at the channel's floor hint: kHintMarginBins below the lowest floor that kHintMinPlanes or more finished
+      // planes of this channel reached.  It is a guess for this plane, applied like a plane-wide floor; the exact-select
+      // kernel checks it afterwards against the plane's histogram (hint_used) and redoes the plane when it pruned too much.
+      const uint2 h = __ldcg(reinterpret_cast<const uint2*>(hp.chint) + c);
+      if (h.y >= (u32)kHintMinPlanes && h.x != 0u) {
+        const int hb = kFineBins - (int)h.x - kHintMarginBins;
+        const float hf = shared_floor<DT>(hb, xscale);
+        if (hf > st.floorx) {  // warp-uniform
+          st.floorx = hf;
+          gfloor_seen = hb;
+          hinted = true;  // a floor to work with: poll the plane's own at the usual period, not every group
+          if (lane == 0) atomicMax(hp.hint_used + plane_id, hb);
+        }
+      }
+    }
     constexpr int poll_mask = 3;  // measured at 128-row strips: polling every group 0.179 ms, every 4th 0.136 ms, every 8th 0.146 ms
     u32 idx0 = (u32)(r_begin * W + panel * kPanel);  // flat index of the group's row 0, panel column 0
     wait_tile(cur_slot, cur_par);
@@ -503,7 +523,7 @@ sdnet_peaks_tile_kernel(const __grid_constant__ PeaksParams p, const __grid_cons
       u32 nxt_slot = cur_slot, nxt_par = cur_par;
       step_pos(nxt_slot, nxt_par);
       if (R == 2 || g + 1 < groups) wait_tile(nxt_slot, nxt_par);
-      if (gfloor_seen <= 0 && g > 0) {
+      if (gfloor_seen <= 0 && g > 0 && !hinted) {
         // The plane has no floor that this warp knows of: every pixel it looks at goes through the slow path, so a
         // fresh look at the published floor is worth its latency (one L2 round trip) -- every group, applied at once.
         gfloor_seen = __ldcg(gfloor_ptr);
@@ -600,6 +620,21 @@ sdnet_peaks_tile_kernel(const __grid_constant__ PeaksParams p, const __grid_cons
     if (st.nbuf) {
       __syncwarp();
       flush_candidates<DT, false>(st, buf, hist, minx, sf, count_ptr, list, p.cap, K, lane, pre, xscale, satx);
+    }
+    if (kHint && lane == 0 && pos <= (u32)p.tier1_units * (u32)p.groups_per_col &&
+        (pos / (u32)p.groups_per_col - 1u) % (u32)p.panels == 0) {
+      // a tier-1 unit (a whole column) done: its plane's floor so far -- certified by >= K recorded survivors, so a lower
+      // bound of the plane's final one -- joins the channel's hint.  One report per plane: its first panel's column.
+      // A plane without a floor yet says nothing: a hinted plane records few candidates and may not have K of them
+      // when this column ends.  (Everything here is recomputed from what the loop keeps anyway: registers are what
+      // limits the occupancy.)
+      const int gf = __ldcg(gfloor_ptr);
+      if (gf > 0) {
+        u32* hint = hp.chint + 2 * ((int)(gfloor_ptr - p.gfloor) % C);
+        atomicMax(hint, (u32)(kFineBins - gf));
+        __threadfence();  // the minimum before the count: a reader that sees the count sees a minimum
+        atomicAdd(hint + 1, 1u);
+      }
     }
     }  // segments of the unit
   }

@@ -49,7 +49,7 @@ namespace {
 // host side
 // ---------------------------------------------------------------------------------------------
 struct Workspace {
-  size_t off_counts, off_flags, off_sched, off_gfloor, off_ghist, off_lists, total;
+  size_t off_counts, off_flags, off_sched, off_gfloor, off_hint_used, off_chint, off_ghist, off_lists, total;
   int cap;
 };
 
@@ -72,6 +72,8 @@ Workspace plan_workspace(int B, int M, int N, int H, int W, int K, int P) {
   ws.off_flags = off;  off = align_up(off + planes * sizeof(int), 256);
   ws.off_sched = off;  off = align_up(off + 64, 256);
   ws.off_gfloor = off; off = align_up(off + planes * sizeof(int), 256);
+  ws.off_hint_used = off; off = align_up(off + planes * sizeof(int), 256);
+  ws.off_chint = off;  off = align_up(off + 2 * (size_t)(M + N) * sizeof(u32), 256);
   ws.off_ghist = off;  off = align_up(off + planes * kFineBins * sizeof(u32), 256);
   ws.off_lists = off;  off = align_up(off + planes * (size_t)ws.cap * sizeof(u64), 256);
   ws.total = off;
@@ -179,15 +181,16 @@ bool make_tile_map(CUtensorMap* map, const SdnetTensor4& t, int dtype, int B, in
 }
 
 // the tile kernel instantiation for (radius, dtype, rows per TMA row)
-typedef void (*TileKernel)(const PeaksParams, const CUtensorMap, const CUtensorMap);
+typedef void (*TileKernel)(const PeaksParams, const CUtensorMap, const CUtensorMap, const HintParams);
+template <bool H>
 TileKernel tile_kernel_for(int radius, int dtype, int S) {
-  if (dtype == SDNET_DTYPE_F32) return radius == 2 ? sdnet_peaks_tile_kernel<2, SDNET_DTYPE_F32, 1> : sdnet_peaks_tile_kernel<1, SDNET_DTYPE_F32, 1>;
+  if (dtype == SDNET_DTYPE_F32) return radius == 2 ? sdnet_peaks_tile_kernel<2, SDNET_DTYPE_F32, 1, H> : sdnet_peaks_tile_kernel<1, SDNET_DTYPE_F32, 1, H>;
   if (dtype == SDNET_DTYPE_F16) {
-    if (S == 2) return sdnet_peaks_tile_kernel<2, SDNET_DTYPE_F16, 2>;
-    return radius == 2 ? sdnet_peaks_tile_kernel<2, SDNET_DTYPE_F16, 1> : sdnet_peaks_tile_kernel<1, SDNET_DTYPE_F16, 1>;
+    if (S == 2) return sdnet_peaks_tile_kernel<2, SDNET_DTYPE_F16, 2, H>;
+    return radius == 2 ? sdnet_peaks_tile_kernel<2, SDNET_DTYPE_F16, 1, H> : sdnet_peaks_tile_kernel<1, SDNET_DTYPE_F16, 1, H>;
   }
-  if (S == 2) return sdnet_peaks_tile_kernel<2, SDNET_DTYPE_BF16, 2>;
-  return radius == 2 ? sdnet_peaks_tile_kernel<2, SDNET_DTYPE_BF16, 1> : sdnet_peaks_tile_kernel<1, SDNET_DTYPE_BF16, 1>;
+  if (S == 2) return sdnet_peaks_tile_kernel<2, SDNET_DTYPE_BF16, 2, H>;
+  return radius == 2 ? sdnet_peaks_tile_kernel<2, SDNET_DTYPE_BF16, 1, H> : sdnet_peaks_tile_kernel<1, SDNET_DTYPE_BF16, 1, H>;
 }
 
 // Which peaks kernel a decode of these tensors runs (SDNET_PATH_*), encoding the tensor maps on the way.
@@ -233,16 +236,16 @@ void launch_pdl(Kern kern, dim3 grid, dim3 block, cudaStream_t stream, const Par
 
 // Resident CTAs per SM of a tile-kernel instantiation, asked once per (device, instantiation); sets the
 // kernel's shared-memory attributes on the way.  0 = the attributes could not be set (`*err` says why).
-int tile_ctas_per_sm(TileKernel kern, int dtype, int tile_s, int radius, int smem, cudaError_t* err) {
+int tile_ctas_per_sm(TileKernel kern, int dtype, int tile_s, int radius, bool hint, int smem, cudaError_t* err) {
   constexpr int kMaxDev = 64;
   static std::mutex mu;
-  static int cache[kMaxDev][3][3][3] = {};  // [device][dtype][rows per TMA row][radius]; 0 = not asked yet
+  static int cache[kMaxDev][3][3][3][2] = {};  // [device][dtype][rows per TMA row][radius][hints]; 0 = not asked yet
   int dev = 0;
   *err = cudaGetDevice(&dev);
   if (*err != cudaSuccess) return 0;
   if (dev < 0 || dev >= kMaxDev) dev = kMaxDev - 1;
   std::lock_guard<std::mutex> lock(mu);
-  int& per_sm = cache[dev][dtype][tile_s][radius];
+  int& per_sm = cache[dev][dtype][tile_s][radius][hint ? 1 : 0];
   if (per_sm > 0) return per_sm;
   *err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
   if (*err != cudaSuccess) return 0;
@@ -261,6 +264,7 @@ struct PeaksPlan {
   int path, tile_s;
   TileKernel tile_kern;
   int smem, ctas, ctas_per_sm, sms;
+  bool hint;  // the tile kernel runs with floor hints
   CUtensorMap tm_anchor, tm_part;
 };
 
@@ -290,6 +294,7 @@ cudaError_t plan_peaks(const SdnetDecodeParams* p, PeaksParams& pp, PeaksPlan& p
   const long long planes = (long long)p->B * C;
   pl.sms = device_sm_count();
   pl.tile_s = 0;
+  pl.hint = false;
   pl.path = select_peaks_path(p, &pl.tm_anchor, &pl.tm_part, &pl.tile_s);
   const bool use_tile = pl.path == SDNET_PATH_TILE || pl.path == SDNET_PATH_TILE_ROW_PAIRS;
   const bool is_f32 = p->dtype == SDNET_DTYPE_F32;
@@ -301,11 +306,11 @@ cudaError_t plan_peaks(const SdnetDecodeParams* p, PeaksParams& pp, PeaksPlan& p
   pp.strips = 1;
   pp.rows_per_strip = p->H;
   if (use_tile) {
-    pl.tile_kern = tile_kernel_for(p->radius, p->dtype, pl.tile_s);
+    pl.tile_kern = tile_kernel_for<false>(p->radius, p->dtype, pl.tile_s);
     const int panel_cols = is_f32 ? TileGeom<SDNET_DTYPE_F32>::kPanel : TileGeom<SDNET_DTYPE_F16>::kPanel;
     pl.smem = tile_smem(pl.tile_s);
     cudaError_t err = cudaSuccess;
-    pl.ctas_per_sm = tile_ctas_per_sm(pl.tile_kern, p->dtype, pl.tile_s, p->radius, pl.smem, &err);
+    pl.ctas_per_sm = tile_ctas_per_sm(pl.tile_kern, p->dtype, pl.tile_s, p->radius, false, pl.smem, &err);
     if (pl.ctas_per_sm <= 0) return err != cudaSuccess ? err : cudaErrorUnknown;
     pp.panels = (p->W + panel_cols - 1) / panel_cols;
     // The work is a line of `columns` x G groups of four rows (a column = one panel of one plane, top to
@@ -318,6 +323,15 @@ cudaError_t plan_peaks(const SdnetDecodeParams* p, PeaksParams& pp, PeaksPlan& p
     pp.H = p->H;
     if (!plan_tile_line(pp, planes, (long long)pl.sms * pl.ctas_per_sm * kTileWarps, &pl.ctas, (long long)pl.sms * pl.ctas_per_sm))
       return cudaErrorInvalidValue;
+    // Floor hints come from finished whole columns (tier-1 units): a launch without any, e.g. a shard that fits one
+    // wave of the resident warps, has none to give and runs the instantiation without the hint code
+    if (!(p->flags & SDNET_FLAG_NO_FLOOR_HINT) && pp.tier1_units > 0) {
+      pl.hint = true;
+      pl.tile_kern = tile_kernel_for<true>(p->radius, p->dtype, pl.tile_s);
+      // sets its attributes; same registers and shared memory, so the same CTAs per SM
+      if (tile_ctas_per_sm(pl.tile_kern, p->dtype, pl.tile_s, p->radius, true, pl.smem, &err) != pl.ctas_per_sm)
+        return err != cudaSuccess ? err : cudaErrorUnknown;
+    }
   } else {
     pl.tile_kern = nullptr;
     pl.smem = kPeaksSmem;
@@ -361,6 +375,9 @@ int launch_decode(const SdnetDecodeParams* p, cudaStream_t stream, cudaEvent_t* 
   PeaksPlan pl;
   cudaError_t err = plan_peaks(p, pp, pl);
   if (err != cudaSuccess) return (int)err;
+  HintParams hp;
+  hp.chint = reinterpret_cast<u32*>(base + ws.off_chint);
+  hp.hint_used = reinterpret_cast<int*>(base + ws.off_hint_used);
   if (!(p->flags & SDNET_FLAG_WORKSPACE_CLEAN)) {  // else: the previous decode's tail kernel left the header zeroed
     err = cudaMemsetAsync(base, 0, ws.off_lists, stream);
     if (err != cudaSuccess) return (int)err;
@@ -368,7 +385,7 @@ int launch_decode(const SdnetDecodeParams* p, cudaStream_t stream, cudaEvent_t* 
   if (marks) cudaEventRecord(marks[0], stream);
 
   if (pl.tile_kern) {
-    pl.tile_kern<<<dim3((unsigned)pl.ctas), dim3(kTileWarps * 32), pl.smem, stream>>>(pp, pl.tm_anchor, pl.tm_part);
+    pl.tile_kern<<<dim3((unsigned)pl.ctas), dim3(kTileWarps * 32), pl.smem, stream>>>(pp, pl.tm_anchor, pl.tm_part, hp);
   } else {
     dim3 grid((unsigned)pl.ctas), block(kThreads);
     const bool r2 = p->radius == 2;
@@ -397,6 +414,8 @@ int launch_decode(const SdnetDecodeParams* p, cudaStream_t stream, cudaEvent_t* 
     ep.pre_activated = pp.pre_activated;
     ep.lists = pp.lists; ep.counts = pp.counts;
     ep.flags = reinterpret_cast<int*>(base + ws.off_flags);
+    ep.check_hints = pl.hint;
+    ep.gfloor = pp.gfloor; ep.ghist = pp.ghist; ep.hint_used = hp.hint_used;
     // (with several decodes in flight this pass-through launch costs 0.5 % of the step at 1024 images and 1-4 % at 128
     // even with thin CTAs -- measured by skipping it; moving it behind the tail, with a fix-up tail launch after it, gets
     // back 1.5 % at 128 and was not worth a fourth launch)
@@ -442,6 +461,8 @@ int launch_decode(const SdnetDecodeParams* p, cudaStream_t stream, cudaEvent_t* 
   tp.ws_flags = reinterpret_cast<int*>(base + ws.off_flags);
   tp.ws_gfloor = pp.gfloor;
   tp.ws_ghist = pp.ghist;
+  tp.ws_hint_used = hp.hint_used;
+  tp.ws_chint = hp.chint;
   tp.ws_sched = pp.sched;
   for (int j = 0; j < SDNET_MAX_DEST; ++j) tp.dest_delta[j] = j < p->n_dest ? p->dest_delta[j] : 0;
   if (p->dtype == SDNET_DTYPE_F16) launch_pdl(sdnet_tail_kernel<SDNET_DTYPE_F16>, dim3((unsigned)p->B), dim3(2 * kTeamThreads), stream, tp);

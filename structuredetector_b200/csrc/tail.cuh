@@ -35,6 +35,8 @@ struct TailParams {
   int* ws_flags;
   int* ws_gfloor;
   u32* ws_ghist;
+  int* ws_hint_used;
+  u32* ws_chint;
   u32* ws_sched;
   long long dest_delta[SDNET_MAX_DEST];
 };
@@ -509,8 +511,9 @@ __global__ void __launch_bounds__(2 * kTeamThreads, 3) sdnet_tail_kernel(const _
       store_out(p, p.diag + ((size_t)b * C + c) * 2 + 1, p.exact_flags[(size_t)b * C + c]);
     }
   }
-  // Leave the workspace header as a fresh memset would: this image's planes (counts, flags, floors, histograms -- all
-  // consumed above) and, once, the unit counter (the peaks kernel is long complete: pdl_wait).
+  // Leave the workspace header as a fresh memset would: this image's planes (counts, flags, floors, histograms, applied
+  // hints -- all consumed above) and, once, the channels' floor hints and the unit counter (the peaks kernel is long
+  // complete: pdl_wait).
   __syncthreads();
   {
     const int C = p.M + p.N;
@@ -518,7 +521,10 @@ __global__ void __launch_bounds__(2 * kTeamThreads, 3) sdnet_tail_kernel(const _
       p.ws_counts[(size_t)b * C + c] = 0;
       p.ws_flags[(size_t)b * C + c] = 0;
       p.ws_gfloor[(size_t)b * C + c] = 0;
+      p.ws_hint_used[(size_t)b * C + c] = 0;
     }
+    if (b == 0)
+      for (int i = threadIdx.x; i < 2 * C; i += blockDim.x) p.ws_chint[i] = 0;
     uint4* gh = reinterpret_cast<uint4*>(p.ws_ghist + (size_t)b * C * kFineBins);
     for (int i = threadIdx.x; i < C * kFineBins / 4; i += blockDim.x) gh[i] = make_uint4(0, 0, 0, 0);
     if (b == 0 && threadIdx.x == 0) p.ws_sched[0] = 0;
